@@ -8,6 +8,8 @@ pass A, pass B, partial-sum reduction, dot products, projection.
     python bench.py --gpus 1 --steps 50 --warmup 5
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference            # CPU arm (oracle port, all host cores)
+    python bench.py --gpus 1 --steps 50 --warmup 5 --dump-outputs DIR   # + what the last timed step computed
+                                                # (1 GPU only; DESIGN.md "Measurement")
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every key.
 """
@@ -26,6 +28,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree, which may be read-only
 
 METRIC = "Gfacet-evals/s (energy+grad)"
 UNIT = "Gfacet-evals/s"
@@ -36,6 +39,8 @@ B_PASS_A = 44.0
 B_PASS_B = 68.0
 B_STEP = B_PASS_A + B_PASS_B  # 112 B, the headline figure
 B_STRICT = 72.0
+# --dump-outputs keeps at most this many vertex rows of each per-vertex array: 2 x 24 MiB of float64 in all
+DUMP_ROWS = 1 << 20
 
 
 def _peaks():
@@ -238,6 +243,23 @@ def workload_config(args, n_gpus):
     }
 
 
+def dump_outputs(dm, out_dir):
+    """Writes what the last evaluation hands its caller: the 16 scalars (energies, area, volume, dot products, KKT
+    multiplier and coefficient; include/ms_b200.h MS_SC_*), the projected gradient and dV/dx, all float64.  A mesh
+    with more than DUMP_ROWS vertices keeps the same seeded sample of rows (ascending) in both arrays."""
+    from membrane_solver_b200 import _lib as L
+
+    os.makedirs(out_dir, exist_ok=True)
+    scalars = dm.read_scalars().scalars
+    grad, volgrad = dm.download(L.ARR_GRAD), dm.download(L.ARR_VOLGRAD)
+    rows = slice(None)
+    if grad.shape[0] > DUMP_ROWS:
+        rows = np.sort(np.random.default_rng(0).choice(grad.shape[0], DUMP_ROWS, replace=False))
+    np.save(os.path.join(out_dir, "scalars.npy"), scalars)
+    np.save(os.path.join(out_dir, "grad.npy"), grad[rows])
+    np.save(os.path.join(out_dir, "volgrad.npy"), volgrad[rows])
+
+
 def run_b200(args):
     from membrane_solver_b200 import _lib as L
     from membrane_solver_b200.context import DeviceMesh
@@ -286,6 +308,8 @@ def run_b200(args):
         dm.eval_async(opts)
     ms_total = dm.timer_stop()
     sampler.active.clear()
+    if args.dump_outputs:  # before the legs below overwrite the results
+        dump_outputs(dm, args.dump_outputs)
     ms_step = ms_total / args.steps
     value = nf / (ms_step * 1e-3) / 1e9
 
@@ -433,7 +457,13 @@ def main():
                     help="total facets of the strong-scaling leg (BASELINE.json north_star: 100 M); 0 = skip")
     ap.add_argument("--no-full-mesh", action="store_true", help="reference arm: skip the one full-size evaluation")
     ap.add_argument("--no-parity", action="store_true", help="N>1: skip the comparison with one GPU on the same mesh")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="1 GPU: write the scalars, gradient and dV/dx of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs needs --impl b200 --gpus 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_b200(args)

@@ -1,12 +1,11 @@
 """Generate golden input/output vectors by running the REAL reference.
 
-Run in the build container only (``/root/reference`` does not exist on the GPU
-box):
+Needs a checkout of the original membrane_solver:
 
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/generate_golden.py
+    MEMBRANE_REFERENCE_ROOT=<checkout> PYTHONDONTWRITEBYTECODE=1 python tests/golden/generate_golden.py
 
-It imports the unmodified reference from ``/root/reference`` (read-only; NumPy
-path, because no Fortran compiler exists here), evaluates the hot-path modules
+It imports the unmodified reference from that checkout (read-only; NumPy path, without
+its Fortran kernels), evaluates the hot-path modules
 on the reference's own mesh files, and stores dense inputs + outputs as small
 ``.npz`` files next to this script.  The fixtures travel; the reference does not.
 
@@ -25,7 +24,9 @@ import sys
 
 import numpy as np
 
-REF = os.environ.get("MEMBRANE_REFERENCE_ROOT", "/root/reference")
+REF = os.environ.get("MEMBRANE_REFERENCE_ROOT")
+if not REF:
+    sys.exit("set MEMBRANE_REFERENCE_ROOT to a checkout of the original membrane_solver")
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.dont_write_bytecode = True
 sys.path.insert(0, REF)

@@ -6,7 +6,8 @@ as the UNMODIFIED reference produced them, with its per-module energies and its 
 stored state is re-evaluated through the plugin layer (``EnergyModuleManager`` / ``EvaluationManager`` twins) -- on
 the host emulator in the CPU tier, on the device through the C ABI in the GPU tier -- at 1e-12, and the end points
 must be the survey's known answers.  The replay of the instruction lists THROUGH the plugins (reference command
-language, refinement, equiangulation, steppers) is ``test_dropin_reference.py`` (build container only)."""
+language, refinement, equiangulation, steppers) is ``test_dropin_reference.py``, which needs a checkout of the
+original project (``MEMBRANE_REFERENCE_ROOT``)."""
 
 import json
 

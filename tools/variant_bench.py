@@ -1,5 +1,5 @@
-import numpy as np, sys, time
-sys.path.insert(0, '/root/repo')
+import numpy as np, os, sys, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from membrane_solver_b200 import _lib as L
 from membrane_solver_b200.context import DeviceMesh
 from membrane_solver_b200.synthetic import icosphere
