@@ -370,6 +370,17 @@ MS_API int ms_ctx_direction_from_gradient(ms_ctx* ctx, double scale);
 /* dst += alpha * src for two (nv,3) arrays, optionally leaving fixed rows untouched: the position update
  * of the hard volume projection x -= lambda dV/dx (modules/constraints/volume.py:116-149) */
 MS_API int ms_ctx_axpy(ms_ctx* ctx, int dst, int src, double alpha, int32_t skip_fixed);
+/* Evolver-style vertex averaging of MS_ARR_POSITIONS, `rounds` times (the `V[n]` command; runtime/vertex_average.py:28-120,
+ * geometry/vertex_average.py::vertex_average_arrays).  Every edge is weighted by the summed area of the facets that list
+ * it, areas taken from the positions before each round; a vertex that is not fixed (ms_ctx_set_topology /
+ * ms_ctx_set_fixed_mask), has more than one edge and more than one usable edge (weight > 0) and a weight sum
+ * sum w^2 >= 1e-15 moves by 1/4 sum w^2 (x_u - x_v) / sum w^2.  group: nv pin groups in the caller's vertex order,
+ * -1 = none; a grouped vertex uses only edges to vertices of its own group (NULL: no pin groups).  Asynchronous on the
+ * context stream (with a group array the call waits for its upload); no atomics, so repeated calls give identical
+ * bits.  MS_ARR_TRIAL is the double buffer of the rounds: its contents are overwritten; every other array is left
+ * alone.  Single-context meshes only: a partition context (n_owned < nv), rounds < 0, or a context without topology or
+ * positions returns an error; rounds == 0 does nothing. */
+MS_API int ms_ctx_vertex_average(ms_ctx* ctx, const int32_t* group, int32_t rounds);
 /* per-vertex Polak-Ribiere direction (runtime/steppers/conjugate_gradient.py:63-119); restart != 0 or no
  * committed history: direction = -gradient.  ms_ctx_cg_commit stores gradient and direction of an
  * accepted step as the history of the next one. */

@@ -481,6 +481,18 @@ class DeviceMesh:
     def axpy(self, dst: int, src: int, alpha: float, skip_fixed: bool = True) -> None:
         L.check(self._lib.ms_ctx_axpy(self._h, int(dst), int(src), float(alpha), int(bool(skip_fixed))))
 
+    def vertex_average(self, rounds: int = 1, group=None) -> None:
+        """Evolver-style vertex averaging of the resident positions, ``rounds`` times (``ms_ctx_vertex_average``):
+        the device twin of ``geometry.vertex_average.vertex_average_arrays`` with the context's fixed mask as the
+        immovable rows.  ``group``: (nv,) pin groups in the caller's vertex order, -1 = none.  Overwrites the trial
+        positions."""
+        g = None
+        if group is not None:
+            g = np.ascontiguousarray(group, dtype=np.int32)
+            if g.shape != (self.nv,):
+                raise ValueError(f"group must have shape ({self.nv},)")
+        L.check(self._lib.ms_ctx_vertex_average(self._h, L.iptr(g), int(rounds)))
+
     def cg_direction(self, restart: bool) -> None:
         L.check(self._lib.ms_ctx_cg_direction(self._h, int(bool(restart))))
 

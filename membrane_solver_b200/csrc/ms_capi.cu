@@ -75,6 +75,7 @@ struct ms_ctx {
   int device = 0;
   cudaStream_t stream = nullptr;
   bool have_topology = false;
+  bool has_positions = false;  // MS_ARR_POSITIONS has been written since the topology was set
   int32_t nv = 0, nf = 0;
   int32_t n_owned = 0;  // vertex rows owned by this context's patches (== nv unless partitioned)
   ms::PackParams pack_params;
@@ -125,13 +126,14 @@ struct ms_ctx {
   std::vector<int32_t> perm;            // new -> old; empty = identity
   DevBuf<int32_t> d_perm;
   DevBuf<double> d_stage;               // staging for permuted uploads / downloads (5*nv doubles)
-  // bending-tilt coupling: triangle rows + corner CSR on the device (built on first use)
+  // triangle rows + corner CSR on the device (built on first use), bending-tilt buffers
   std::vector<int32_t> h_tri;
-  bool bt_ready = false, tri_ready = false;
+  bool bt_ready = false, tri_ready = false, csr_ready = false;
   DevBuf<double> d_cg_prev_g, d_cg_prev_d;  // conjugate-gradient memory (previous gradient / direction)
   DevBuf<unsigned long long> d_ls_bits;  // line-search reductions: [min edge^2, max |d|^2] as bit patterns, [flag]
   DevBuf<int32_t> d_tri, d_csr_ptr, d_csr_idx;
   DevBuf<double> d_bt_corner, d_bt_base, d_bt_facet_e, d_bt_e;
+  DevBuf<int32_t> d_va_group;  // pin groups of ms_ctx_vertex_average (internal order)
   int64_t n_send_rows = 0;
   // leaflet tilt modules (ms_leaflet.cuh): per-leaflet selections, parameters and tilt fields
   struct Leaflet {
@@ -357,16 +359,24 @@ int ensure_tri(ms_ctx* c) {
   return 0;
 }
 
+// triangle rows and the vertex -> corner CSR (corner id 3 f + k, facet-major) on the device, once per topology
+int ensure_corner_csr(ms_ctx* c) {
+  if (c->csr_ready) return 0;
+  std::vector<int32_t> ptr, idx;
+  ms::build_corner_csr(c->nv, c->nf, c->h_tri.data(), ptr, idx);
+  if (int rc = ensure_tri(c)) return rc;
+  if (int rc = c->d_csr_ptr.ensure(ptr.size())) return rc;
+  if (int rc = c->d_csr_idx.ensure(idx.size() + 1)) return rc;
+  CU(cudaMemcpy(c->d_csr_ptr.p, ptr.data(), ptr.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  if (!idx.empty()) CU(cudaMemcpy(c->d_csr_idx.p, idx.data(), idx.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  c->csr_ready = true;
+  return 0;
+}
+
 int bt_prepare(ms_ctx* c, ms::BtMesh& m) {
   const size_t nv = size_t(c->nv), nf = size_t(c->nf);
+  if (int rc = ensure_corner_csr(c)) return rc;
   if (!c->bt_ready) {
-    std::vector<int32_t> ptr, idx;
-    ms::build_corner_csr(c->nv, c->nf, c->h_tri.data(), ptr, idx);
-    if (int rc = ensure_tri(c)) return rc;
-    if (int rc = c->d_csr_ptr.ensure(ptr.size())) return rc;
-    if (int rc = c->d_csr_idx.ensure(idx.size() + 1)) return rc;
-    CU(cudaMemcpy(c->d_csr_ptr.p, ptr.data(), ptr.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-    if (!idx.empty()) CU(cudaMemcpy(c->d_csr_idx.p, idx.data(), idx.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
     if (int rc = c->d_bt_corner.ensure(12 * nf + 1)) return rc;
     if (int rc = c->d_bt_base.ensure(nv + 1)) return rc;
     if (int rc = c->d_bt_facet_e.ensure(nf + 1)) return rc;
@@ -625,6 +635,8 @@ int ms_ctx_set_topology_partition(ms_ctx* c, int32_t nv, int32_t n_owned, int32_
   c->h_tri.assign(tri, tri + 3 * size_t(nf));
   c->bt_ready = false;
   c->tri_ready = false;
+  c->csr_ready = false;
+  c->has_positions = false;
   c->pipe_ready = false;
   for (auto& lf : c->leaflet) {  // per-leaflet arrays are sized for the previous vertex count
     lf.set = lf.has_fixed = lf.has_minv = false;
@@ -862,6 +874,7 @@ int ms_ctx_upload(ms_ctx* c, int which, const double* host, int64_t offset, int6
   double* d = array_ptr(c, which, &len);
   if (!d && len > 0) return fail(-1, "array is not allocated");
   if (offset < 0 || count < 0 || offset + count > len) return fail(-1, "upload range out of bounds");
+  if (which == MS_ARR_POSITIONS) c->has_positions = true;
   if (!c->perm.empty() && per_vertex_array(which) && count) {
     // the caller's rows are in its own vertex order: land in the staging buffer, gather into internal order
     if (offset != 0 || count != len) return fail(-1, "partial uploads are not available on an internally reordered mesh");
@@ -897,6 +910,7 @@ void* ms_ctx_device_ptr(ms_ctx* c, int which) {
   if (use_device(c)) return nullptr;
   if (ensure_array(c, which)) return nullptr;
   if (which == MS_ARR_GRAD && flush_projection(c)) return nullptr;  // the caller sees the projected gradient
+  if (which == MS_ARR_POSITIONS) c->has_positions = true;             // the caller may write through it
   int64_t len = 0;
   return array_ptr(c, which, &len);
 }
@@ -1259,8 +1273,7 @@ int ms_ctx_set_leaflet_fixed(ms_ctx* c, int32_t leaflet, const uint8_t* fixed_ro
 int ms_ctx_update_vertex_normals(ms_ctx* c) {
   if (int rc = check_ctx(c, true)) return rc;
   if (c->n_owned != c->nv) return fail(-5, "not available on a partitioned context");
-  ms::BtMesh bm;
-  if (int rc = bt_prepare(c, bm)) return rc;
+  if (int rc = ensure_corner_csr(c)) return rc;
   if (int rc = c->d_vnormals.ensure(3 * size_t(c->nv) + 1)) return rc;
   CU(ms::launch_vertex_normals(c->nv, c->d_tri.p, c->d_csr_ptr.p, c->d_csr_idx.p, c->d_pos.p, c->d_vnormals.p, c->stream));
   c->vnormals_ready = true;
@@ -1990,6 +2003,7 @@ static int eval_pipelined(ms_ctx* c, const ms_eval_opts* o, const double* pos_ho
   const bool ran_a = needs_bending(o) || !o->want_grad;
   c->ran_pass_a = ran_a;
   double* dst = o->use_trial ? c->d_trial.p : c->d_pos.p;
+  if (!o->use_trial) c->has_positions = true;
   const int kPipeChunks = pipe_chunks();
   while (c->pipe_events.size() < size_t(kPipeChunks) + 1) {
     cudaEvent_t e = nullptr;
@@ -2129,6 +2143,44 @@ int ms_ctx_accept_trial(ms_ctx* c) {
   if (int rc = check_ctx(c, true)) return rc;
   if (!c->d_trial.p) return fail(-4, "no trial positions exist");
   CU(cudaMemcpyAsync(c->d_pos.p, c->d_trial.p, 3 * size_t(c->nv) * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+  c->has_positions = true;
+  return 0;
+}
+
+int ms_ctx_vertex_average(ms_ctx* c, const int32_t* group, int32_t rounds) {
+  if (int rc = check_ctx(c, true)) return rc;
+  if (c->n_owned != c->nv) return fail(-5, "vertex averaging is not available on a partitioned context");
+  if (rounds < 0) return fail(-1, "rounds must be >= 0");
+  if (!c->has_positions) return fail(-4, "no positions have been set (MS_ARR_POSITIONS)");
+  if (rounds == 0 || c->nv == 0) return 0;
+  if (int rc = ensure_corner_csr(c)) return rc;
+  if (int rc = ensure_array(c, MS_ARR_TRIAL)) return rc;
+  const size_t nv = size_t(c->nv);
+  if (group) {
+    std::vector<int32_t> tmp;
+    if (!c->perm.empty()) {
+      tmp = permuted(group, c->perm);
+      group = tmp.data();
+    }
+    if (int rc = c->d_va_group.ensure(nv)) return rc;
+    CU(cudaMemcpyAsync(c->d_va_group.p, group, nv * sizeof(int32_t), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));  // tmp (or the caller's array) may go away after the return
+  }
+  ms::VaMesh m;
+  m.nv = c->nv;
+  m.tri = c->d_tri.p;
+  m.csr_ptr = c->d_csr_ptr.p;
+  m.csr_idx = c->d_csr_idx.p;
+  m.group = group ? c->d_va_group.p : nullptr;
+  m.fixed = c->has_fixed ? c->d_fixed.p : nullptr;
+  // Jacobi rounds alternate between the positions and the trial buffer; an odd count ends with one copy back
+  double* buf[2] = {c->d_pos.p, c->d_trial.p};
+  for (int32_t r = 0; r < rounds; ++r) {
+    m.pos = buf[r & 1];
+    CU(ms::launch_vertex_average(m, buf[(r + 1) & 1], c->stream));
+  }
+  if (rounds & 1)
+    CU(cudaMemcpyAsync(c->d_pos.p, c->d_trial.p, 3 * nv * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
   return 0;
 }
 

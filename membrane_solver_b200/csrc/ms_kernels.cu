@@ -1410,6 +1410,13 @@ __global__ void __launch_bounds__(128) k_vertex_normals(int32_t nv, const int32_
   st3(normals, v, n);
 }
 
+// Evolver-style vertex averaging (ms_vertex_average.cuh): one thread per vertex over its corner list
+__global__ void __launch_bounds__(128) k_vertex_average(const VaMesh m, double* __restrict__ out) {
+  const int v = blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= m.nv) return;
+  st3(out, v, va_vertex(m, v));
+}
+
 // t -= (t.n) n  (runtime/projections/tilt.py:8-14)
 __global__ void __launch_bounds__(256) k_project_tangent(int64_t nv, const double* __restrict__ normals, double* t) {
   const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -2077,6 +2084,11 @@ cudaError_t launch_leaflet_fused_pair(const LeafletMesh& m0, const LeafletMesh& 
 cudaError_t launch_vertex_normals(int32_t nv, const int32_t* tri, const int32_t* csr_ptr, const int32_t* csr_idx,
                                   const double* pos, double* normals, cudaStream_t st) {
   if (nv > 0) k_vertex_normals<<<blocks_for(nv, 128), 128, 0, st>>>(nv, tri, csr_ptr, csr_idx, pos, normals);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_vertex_average(const VaMesh& m, double* out, cudaStream_t st) {
+  if (m.nv > 0) k_vertex_average<<<blocks_for(m.nv, 128), 128, 0, st>>>(m, out);
   return cudaGetLastError();
 }
 

@@ -10,6 +10,7 @@
 #include "ms_leaflet.cuh"
 #include "ms_math.cuh"
 #include "ms_pack.h"
+#include "ms_vertex_average.cuh"
 
 namespace ms {
 
@@ -313,5 +314,8 @@ cudaError_t launch_tilt_cg_direction(int64_t nv, const double* g, const double* 
                                      cudaStream_t st);
 cudaError_t launch_masked_norm2(int64_t nv, double* g, const uint8_t* fixed, double* rowsq, double* out,
                                 double* sum_scratch, cudaStream_t st);
+
+// --- vertex averaging (the `V` command): one thread per vertex, m.pos -> out (a different buffer) ---
+cudaError_t launch_vertex_average(const VaMesh& m, double* out, cudaStream_t st);
 
 }  // namespace ms

@@ -97,6 +97,18 @@ class DeviceMinimizer:
             lam = delta / (float(res.scalars[L.SC_GC_GC]) + 1e-12)
             dm.axpy(target, L.ARR_VOLGRAD, -lam, skip_fixed=True)
 
+    # -- the V[n] command (commands/mesh_ops.py:45-53) --------------------------------------------------
+    def vertex_average(self, n: int = 1) -> None:
+        """``n`` rounds of vertex averaging on the device (``DeviceMesh.vertex_average``; fixed rows stay), then,
+        with ``enforce_volume``, the hard volume projection of the ``mesh_operation`` context (12 iterations).  The
+        positions jump, so the conjugate-gradient history is discarded: the next ``cg`` step restarts from the
+        steepest-descent direction, as after a failed step."""
+        self.dm.vertex_average(int(n))
+        if self.enforce_volume:
+            self._enforce(trial=False, max_iter=12)
+        self._cg_have_history = False
+        self._cg_iter = 0
+
     # -- one line search (line_search.py:267-430) --------------------------------------------------
     def _line_search(self, step_size: float):
         dm = self.dm
