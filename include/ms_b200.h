@@ -92,7 +92,9 @@ typedef struct ms_eval_opts {
                               evaluation (patches without / with ghost rows in their halo) */
   int32_t diagnostics;     /* also write K_VECS / A_VOR / A_EFF / E_VERTEX */
   int32_t want_tilt_grad;  /* with want_grad == 0: still produce MS_ARR_TILT_GRAD (tilt-only evaluation,
-                              evaluation_manager.py:693-698) */
+                              evaluation_manager.py:693-698).  With MS_MOD_TILT this runs pass B, which overwrites
+                              MS_ARR_GRAD and MS_ARR_VOLGRAD with the raw gradients of the modules and drops a
+                              pending projection: evaluate with want_grad again before using the gradient */
 } ms_eval_opts;
 
 typedef struct ms_pack_info {
@@ -172,9 +174,14 @@ MS_API int ms_ctx_set_bending_params(ms_ctx* ctx, const double* kappa, const dou
 MS_API int ms_ctx_set_tilt_rigidity(ms_ctx* ctx, double k_tilt);
 MS_API int ms_ctx_set_positions(ms_ctx* ctx, const double* pos_host);
 MS_API int ms_ctx_set_tilts(ms_ctx* ctx, const double* tilts_host);
-/* generic host<->device copies of a named array (count doubles from element offset) */
+/* generic host<->device copies of a named array (count doubles from element offset).  Uploading MS_ARR_GRAD
+ * replaces the gradient and drops a pending projection (ms_ctx_eval_async); uploading MS_ARR_VOLGRAD first applies a
+ * pending projection with the gC the evaluation produced, so the gradient stays the one of that evaluation. */
 MS_API int ms_ctx_upload(ms_ctx* ctx, int which, const double* host, int64_t offset, int64_t count);
 MS_API int ms_ctx_get_array(ms_ctx* ctx, int which, double* host, int64_t offset, int64_t count);
+/* Device pointer of a named array (internal row order).  For MS_ARR_GRAD and MS_ARR_VOLGRAD a pending projection is
+ * applied first: the caller reads the projected gradient and may write gC without changing it.  ms_ctx_axpy with
+ * dst == MS_ARR_VOLGRAD does the same. */
 MS_API void* ms_ctx_device_ptr(ms_ctx* ctx, int which);
 MS_API int64_t ms_ctx_array_len(const ms_ctx* ctx, int which);
 MS_API int ms_ctx_set_stream(ms_ctx* ctx, void* cuda_stream);
@@ -390,7 +397,9 @@ MS_API int ms_ctx_cg_commit(ms_ctx* ctx);
  *          <gradient, direction>, <gradient, gradient> } */
 MS_API int ms_ctx_line_search_stats(ms_ctx* ctx, double* out4);
 /* ok = 1 unless a facet normal turns by more than limit_radians between the positions and the trial
- * positions or a facet collapses (runtime/topology.py:13-48) */
+ * positions or a facet collapses (runtime/topology.py:13-48).  Only facets with |n0| > 1e-12 at the positions are
+ * judged; such a facet fails when |n1| < 1e-12, when cos(angle) < cos(limit_radians), or when a trial coordinate
+ * of it is NaN.  limit_radians must lie in [0, pi] (else -1). */
 MS_API int ms_ctx_normal_change_ok(ms_ctx* ctx, double limit_radians, int32_t* ok);
 /* deterministic <g,g>, <g,gC>, <gC,gC> into the scalar vector */
 MS_API int ms_ctx_dots(ms_ctx* ctx);

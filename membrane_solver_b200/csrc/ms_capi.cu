@@ -868,6 +868,9 @@ int ms_ctx_set_tilt_rigidity(ms_ctx* c, double k_tilt) {
 int ms_ctx_upload(ms_ctx* c, int which, const double* host, int64_t offset, int64_t count) {
   if (int rc = check_ctx(c, true)) return rc;
   if (which == MS_ARR_GRAD) c->proj.active = false;
+  // gC takes part in a pending projection: apply it with the OLD gC first
+  if (which == MS_ARR_VOLGRAD)
+    if (int rc = flush_projection(c)) return rc;
   if (!host && count > 0) return fail(-1, "null host pointer");
   if (int rc = ensure_array(c, which)) return rc;
   int64_t len = 0;
@@ -909,7 +912,8 @@ void* ms_ctx_device_ptr(ms_ctx* c, int which) {
   if (!c || !c->have_topology) return nullptr;
   if (use_device(c)) return nullptr;
   if (ensure_array(c, which)) return nullptr;
-  if (which == MS_ARR_GRAD && flush_projection(c)) return nullptr;  // the caller sees the projected gradient
+  // the caller sees the projected gradient, and may write gC only after the projection that uses it
+  if ((which == MS_ARR_GRAD || which == MS_ARR_VOLGRAD) && flush_projection(c)) return nullptr;
   if (which == MS_ARR_POSITIONS) c->has_positions = true;             // the caller may write through it
   int64_t len = 0;
   return array_ptr(c, which, &len);
@@ -2209,7 +2213,7 @@ int ms_ctx_direction_from_gradient(ms_ctx* c, double scale) {
 
 int ms_ctx_axpy(ms_ctx* c, int dst, int src, double alpha, int32_t skip_fixed) {
   if (int rc = check_ctx(c, true)) return rc;
-  if (dst == MS_ARR_GRAD || src == MS_ARR_GRAD)
+  if (dst == MS_ARR_GRAD || src == MS_ARR_GRAD || dst == MS_ARR_VOLGRAD)
     if (int rc = flush_projection(c)) return rc;
   int64_t ld = 0, ls = 0;
   double* d = array_ptr(c, dst, &ld);
@@ -2285,6 +2289,8 @@ int ms_ctx_line_search_stats(ms_ctx* c, double* out4) {
 int ms_ctx_normal_change_ok(ms_ctx* c, double limit_radians, int32_t* ok) {
   if (int rc = check_ctx(c, true)) return rc;
   if (!ok) return fail(-1, "null argument");
+  // beyond pi the cosine rule no longer orders the angles (cos(2 pi) == cos(0))
+  if (!(limit_radians >= 0.0 && limit_radians <= 3.141592653589793)) return fail(-1, "limit_radians must lie in [0, pi]");
   if (!c->d_trial.p) return fail(-4, "no trial positions exist");
   if (int rc = ensure_tri(c)) return rc;
   if (int rc = c->d_ls_bits.ensure(4)) return rc;

@@ -1685,8 +1685,10 @@ __global__ void __launch_bounds__(256) k_normal_change(const int32_t* __restrict
   const double m1 = sqrt(dot(n1, n1));
   bool bad = m1 < 1.0e-12;
   if (!bad) {
+    // clamp without fmin / fmax, which would turn a NaN (a non-finite trial vertex) into a passing -1
     double d = dot(n0, n1) / (m0 * m1);
-    d = fmin(1.0, fmax(-1.0, d));
+    if (d > 1.0) d = 1.0;
+    if (d < -1.0) d = -1.0;
     bad = !(d >= cos_limit);
   }
   if (bad) atomicOr(flag, 1);
@@ -1713,8 +1715,9 @@ __global__ void __launch_bounds__(256) k_cg_direction(const double* __restrict__
   d[3 * v] = dx; d[3 * v + 1] = dy; d[3 * v + 2] = dz;
 }
 
-// y[v,:] += alpha * x[v,:] on the rows that are not fixed (constraint projection of the positions)
-__global__ void __launch_bounds__(256) k_axpy_rows(const double* __restrict__ x, double alpha,
+// y[v,:] += alpha * x[v,:] on the rows that are not fixed (constraint projection of the positions).  x may be y
+// (ms_ctx_axpy with dst == src), so it is not __restrict__; each thread reads and writes only its own element.
+__global__ void __launch_bounds__(256) k_axpy_rows(const double* x, double alpha,
                                                    const uint8_t* __restrict__ fixed, int64_t nv, double* y) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= 3 * nv) return;

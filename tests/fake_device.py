@@ -20,6 +20,8 @@ class FakeDeviceMesh:
         self.k_tilt = 0.0
         self.tilts = None
         self.arrays = {}
+        self.scalars = np.zeros(L.SC_COUNT)
+        self._pg = self._pd = None
         self.topology_uploads = 0
         self.evals = 0
         FakeDeviceMesh.instances.append(self)
@@ -31,6 +33,14 @@ class FakeDeviceMesh:
         self.nf = self.tri.shape[0]
         self.is_boundary, self.body_mask, self.fixed = is_boundary, body_mask, fixed_mask
         self.topology_uploads += 1
+        # like the device: zeroed gradients, no trial positions, direction or conjugate-gradient history
+        self.arrays.update({L.ARR_GRAD: np.zeros((self.nv, 3)), L.ARR_VOLGRAD: np.zeros((self.nv, 3))})
+        self.arrays.pop(L.ARR_TRIAL, None)
+        self.arrays.pop(L.ARR_DIRECTION, None)
+        self._pg = self._pd = None
+
+    def permutation(self):
+        return np.arange(self.nv, dtype=np.int32)  # the emulator keeps the caller's vertex order
 
     def set_fixed_mask(self, fixed_mask):
         self.fixed = fixed_mask
@@ -54,9 +64,12 @@ class FakeDeviceMesh:
         self.evals += 1
         kw = dict(self.pack)
         g, k, c = self.gamma, self.kappa, self.c0
+        # a tilt-only evaluation runs pass B on the device, which leaves the RAW gradients of the modules
+        tilt_only = (not opts.get("want_grad", True) and opts.get("want_tilt_grad", False)
+                     and bool(opts["modules"] & L.MOD_TILT))
         out = H.emulate(pos, self.tri, modules=opts["modules"], flags=opts.get("flags", 0),
-                        want_grad=opts.get("want_grad", True), is_boundary=self.is_boundary, body_mask=self.body_mask,
-                        tilts=self.tilts, gamma=g if np.ndim(g) else None, gamma_u=g if not np.ndim(g) else 1.0,
+                        want_grad=opts.get("want_grad", True) or tilt_only, is_boundary=self.is_boundary,
+                        body_mask=self.body_mask, tilts=self.tilts, gamma=g if np.ndim(g) else None, gamma_u=g if not np.ndim(g) else 1.0,
                         kappa=k if np.ndim(k) else None, kappa_u=0.0 if np.ndim(k) else float(k),
                         c0=c if np.ndim(c) else None, c0_u=0.0 if np.ndim(c) else float(c), k_tilt=self.k_tilt, **kw)
         sc = np.zeros(L.SC_COUNT)
@@ -80,9 +93,10 @@ class FakeDeviceMesh:
                 g_out = np.where(np.asarray(self.fixed, bool)[:, None], 0.0, g_out)
         new = {L.ARR_E_VERTEX: out["e_vertex"], L.ARR_K_VECS: out["k_vecs"], L.ARR_A_VOR: out["a_vor"],
                L.ARR_A_EFF: out["a_eff"], L.ARR_TILT_GRAD: out["tilt_grad"]}
-        if opts.get("want_grad", True):  # an energy-only evaluation leaves the gradients alone, like the device
+        if opts.get("want_grad", True) or tilt_only:  # an energy-only evaluation leaves the gradients alone
             new.update({L.ARR_GRAD: g_out, L.ARR_VOLGRAD: gc})
         self.arrays.update(new)
+        self.scalars = sc.copy()
         if grad is not None:
             grad[:] = g_out
         if volgrad is not None:
@@ -92,12 +106,26 @@ class FakeDeviceMesh:
         return EvalResult(sc)
 
     def download(self, which):
-        if which == L.ARR_POSITIONS:
-            return np.array(self.pos)
         return np.array(self.arrays[which])
 
     def upload(self, which, host):
         self.arrays[which] = np.array(host, dtype=np.float64)
+
+    def device_view(self, which):
+        return self.arrays[which]  # writes land in the array, as through ms_ctx_device_ptr
+
+    def read_scalars(self):
+        return EvalResult(self.scalars.copy())
+
+    def sync(self):
+        pass
+
+    # positions, trial positions and search direction live in ``arrays`` like the other named arrays
+    pos = property(lambda self: self.arrays[L.ARR_POSITIONS],
+                   lambda self, v: self.arrays.__setitem__(L.ARR_POSITIONS, v))
+    trial = property(lambda self: self.arrays[L.ARR_TRIAL], lambda self, v: self.arrays.__setitem__(L.ARR_TRIAL, v))
+    dir = property(lambda self: self.arrays[L.ARR_DIRECTION],
+                   lambda self, v: self.arrays.__setitem__(L.ARR_DIRECTION, v))
 
     # -- leaflet modules (emulated ms_leaflet.cuh bodies) --
     def set_leaflet(self, leaflet, **desc):
@@ -219,6 +247,9 @@ class FakeDeviceMesh:
     def set_positions(self, pos):
         self.pos = np.array(pos, dtype=np.float64)
 
+    def set_direction(self, d):
+        self.dir = np.array(d, dtype=np.float64)
+
     def eval(self, opts):
         p = self.trial if opts.get("use_trial") else self.pos
         return self.eval_host(opts, p)
@@ -227,20 +258,19 @@ class FakeDeviceMesh:
         self.dir = scale * self.arrays[L.ARR_GRAD]
 
     def axpy(self, dst, src, alpha, skip_fixed=True):
-        x = self.arrays[src] if src != L.ARR_POSITIONS else self.pos
-        upd = alpha * x
+        upd = alpha * self.arrays[src]
         if skip_fixed and self.fixed is not None:
             upd[np.asarray(self.fixed, bool)] = 0.0
-        if dst == L.ARR_POSITIONS:
-            self.pos = self.pos + upd
-        elif dst == L.ARR_TRIAL:
-            self.trial = self.trial + upd
-        else:
-            self.arrays[dst] = self.arrays[dst] + upd
+        self.arrays[dst] = self.arrays[dst] + upd
+
+    def dots(self):
+        g, gc = self.arrays[L.ARR_GRAD], self.arrays[L.ARR_VOLGRAD]
+        sc = self.scalars
+        sc[L.SC_G_G], sc[L.SC_G_GC], sc[L.SC_GC_GC] = (g * g).sum(), (g * gc).sum(), (gc * gc).sum()
 
     def cg_direction(self, restart):
         g = self.arrays[L.ARR_GRAD]
-        if restart or getattr(self, "_pg", None) is None:
+        if restart or self._pg is None:
             self.dir = -g
             return
         beta = np.einsum("ij,ij->i", g, g - self._pg) / (np.einsum("ij,ij->i", self._pg, self._pg) + 1e-20)
@@ -263,22 +293,24 @@ class FakeDeviceMesh:
         t, p = self.tri, self.pos
         e = np.concatenate([p[t[:, 2]] - p[t[:, 1]], p[t[:, 0]] - p[t[:, 2]], p[t[:, 1]] - p[t[:, 0]]])
         g = self.arrays[L.ARR_GRAD]
-        return (float(np.sqrt((e * e).sum(axis=1).min())), float(np.sqrt((self.dir**2).sum(axis=1).max())),
+        min_edge = float(np.sqrt((e * e).sum(axis=1).min())) if self.nf else 0.0
+        return (min_edge, float(np.sqrt((self.dir**2).sum(axis=1).max())),
                 float((g * self.dir).sum()), float((g * g).sum()))
 
     def normal_change_ok(self, limit=0.5):
+        # the rule of ms_ctx_normal_change_ok (include/ms_b200.h)
+        if not (0.0 <= limit <= np.pi):
+            raise L.B200Error("limit_radians must lie in [0, pi]")
         t = self.tri
         def normals(p):
             return np.cross(p[t[:, 1]] - p[t[:, 0]], p[t[:, 2]] - p[t[:, 0]])
         n0, n1 = normals(self.pos), normals(self.trial)
         m0, m1 = np.linalg.norm(n0, axis=1), np.linalg.norm(n1, axis=1)
         good = m0 > 1e-12
-        if not good.any():
-            return True
-        if (m1[good] < 1e-12).any():
-            return False
-        d = np.clip((n0[good] * n1[good]).sum(axis=1) / (m0[good] * m1[good]), -1.0, 1.0)
-        return bool(np.all(np.arccos(d) <= limit))
+        with np.errstate(invalid="ignore", divide="ignore"):
+            d = np.clip((n0[good] * n1[good]).sum(axis=1) / (m0[good] * m1[good]), -1.0, 1.0)  # NaN stays NaN
+            bad = (m1[good] < 1e-12) | ~(d >= np.cos(limit))
+        return not bool(bad.any())
 
     def close(self):
         pass
