@@ -388,6 +388,32 @@ MS_API int ms_ctx_axpy(ms_ctx* ctx, int dst, int src, double alpha, int32_t skip
  * alone.  Single-context meshes only: a partition context (n_owned < nv), rounds < 0, or a context without topology or
  * positions returns an error; rounds == 0 does nothing. */
 MS_API int ms_ctx_vertex_average(ms_ctx* ctx, const int32_t* group, int32_t rounds);
+/* Equiangulation (the `u` command; geometry/equiangulate.py::equiangulate_triangles, criterion of
+ * runtime/equiangulation.py:151-233): sweeps of Delaunay edge flips over the resident triangle rows, at most
+ * max_iterations of them, stopping after the first sweep without a flip.  An interior edge a-b (exactly two facets,
+ * opposite directions) flips to c-d when the angles at c and d, measured in the tangent plane, add up to more than
+ * pi + 1e-3, not both a and b are fixed, c != d, c-d is not an edge yet and the new facets (a, d, c) and (b, c, d) are
+ * not degenerate and turn their normals by less than 120 degrees.  Candidates are taken in ascending edge key
+ * min*nv + max of the CALLER's vertex numbering; one is skipped when an earlier flip of the same sweep touched one of
+ * its facets or made its new diagonal.  The rows, flip count and sweep count (sweeps that flipped) are those of the
+ * host twin, except where an angle sum lies within a few ulp of the threshold (acos is the platform's).  No atomics
+ * on floating-point data: repeated calls give identical rows.  Facets keep their rows, so positions, the fixed and
+ * boundary masks, kappa / c0, tilts, per-facet surface tension and body membership stay.  After a call that flipped,
+ * the rows are packed again and everything derived from the connectivity is dropped as ms_ctx_set_topology drops it:
+ * leaflet selections (call ms_ctx_set_leaflet again), vertex normals, the conjugate-gradient history, a pending
+ * projection.  If the new rows do not pack (a vertex of more than 48 facets, max_local), the call returns that error
+ * and the context keeps its previous rows and packing.  Synchronous.  Single-context meshes only: a partition context
+ * (n_owned < nv), max_iterations < 0, a context without topology or positions, or a vertex index outside [0, nv)
+ * returns an error.  n_flips / n_sweeps may be NULL. */
+MS_API int ms_ctx_equiangulate(ms_ctx* ctx, int32_t max_iterations, int64_t* n_flips, int32_t* n_sweeps);
+/* Diagnostics of the last ms_ctx_equiangulate: *n_sweeps_run = sweeps run (including a last one without flips);
+ * rounds[i] = selection rounds of sweep i (0 for a sweep without candidates), at most `capacity` entries;
+ * ms4 = device time of all sweeps (CUDA events), then host-clock times of the row download, the host packing and the
+ * upload of the new packing.  rounds / ms4 may be NULL. */
+MS_API int ms_ctx_equiangulate_stats(const ms_ctx* ctx, double* ms4, int32_t* rounds, int32_t capacity,
+                                     int32_t* n_sweeps_run);
+/* the current (nf,3) triangle rows in the caller's vertex numbering */
+MS_API int ms_ctx_get_triangles(const ms_ctx* ctx, int32_t* out);
 /* per-vertex Polak-Ribiere direction (runtime/steppers/conjugate_gradient.py:63-119); restart != 0 or no
  * committed history: direction = -gradient.  ms_ctx_cg_commit stores gradient and direction of an
  * accepted step as the history of the next one. */

@@ -173,6 +173,9 @@ SIGNATURES = {
     "ms_ctx_direction_from_gradient": (ctypes.c_int, [_V, _f64]),
     "ms_ctx_axpy": (ctypes.c_int, [_V, ctypes.c_int, ctypes.c_int, _f64, _i32]),
     "ms_ctx_vertex_average": (ctypes.c_int, [_V, _I, _i32]),
+    "ms_ctx_equiangulate": (ctypes.c_int, [_V, _i32, ctypes.POINTER(_i64), ctypes.POINTER(_i32)]),
+    "ms_ctx_equiangulate_stats": (ctypes.c_int, [_V, _D, _I, _i32, ctypes.POINTER(_i32)]),
+    "ms_ctx_get_triangles": (ctypes.c_int, [_V, _I]),
     "ms_ctx_cg_direction": (ctypes.c_int, [_V, _i32]),
     "ms_ctx_cg_commit": (ctypes.c_int, [_V]),
     "ms_ctx_line_search_stats": (ctypes.c_int, [_V, _D]),

@@ -493,6 +493,32 @@ class DeviceMesh:
                 raise ValueError(f"group must have shape ({self.nv},)")
         L.check(self._lib.ms_ctx_vertex_average(self._h, L.iptr(g), int(rounds)))
 
+    def equiangulate(self, max_iterations: int = 100) -> int:
+        """Delaunay edge flips of the resident triangle rows (``ms_ctx_equiangulate``), the device twin of
+        ``geometry.equiangulate.equiangulate_triangles`` with the context's fixed mask; returns the number of flips.
+        After a call that flipped, the leaflet selections must be set again (``set_leaflet``)."""
+        flips, sweeps = ctypes.c_int64(0), ctypes.c_int32(0)
+        L.check(self._lib.ms_ctx_equiangulate(self._h, int(max_iterations), ctypes.byref(flips), ctypes.byref(sweeps)))
+        self.last_equiangulate_sweeps = int(sweeps.value)
+        return int(flips.value)
+
+    def equiangulate_stats(self) -> dict:
+        """Sweeps run by the last ``equiangulate``, the selection rounds of each, and its times in ms: device time of
+        the sweeps, row download, host packing, upload."""
+        n = ctypes.c_int32(0)
+        L.check(self._lib.ms_ctx_equiangulate_stats(self._h, None, None, 0, ctypes.byref(n)))
+        ms = np.zeros(4)
+        rounds = np.zeros(max(int(n.value), 1), dtype=np.int32)
+        L.check(self._lib.ms_ctx_equiangulate_stats(self._h, L.dptr(ms), L.iptr(rounds), int(n.value), ctypes.byref(n)))
+        return {"sweeps_run": int(n.value), "rounds": rounds[:int(n.value)].tolist(), "sweep_ms": float(ms[0]),
+                "d2h_ms": float(ms[1]), "pack_ms": float(ms[2]), "upload_ms": float(ms[3])}
+
+    def triangles(self) -> np.ndarray:
+        """The current (nf,3) triangle rows in the caller's vertex numbering."""
+        out = np.empty((self.nf, 3), dtype=np.int32)
+        L.check(self._lib.ms_ctx_get_triangles(self._h, L.iptr(out)))
+        return out
+
     def cg_direction(self, restart: bool) -> None:
         L.check(self._lib.ms_ctx_cg_direction(self._h, int(bool(restart))))
 

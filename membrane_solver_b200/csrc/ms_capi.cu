@@ -5,6 +5,7 @@
 #include <nvtx3/nvToolsExt.h>
 
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -134,6 +135,12 @@ struct ms_ctx {
   DevBuf<int32_t> d_tri, d_csr_ptr, d_csr_idx;
   DevBuf<double> d_bt_corner, d_bt_base, d_bt_facet_e, d_bt_e;
   DevBuf<int32_t> d_va_group;  // pin groups of ms_ctx_vertex_average (internal order)
+  // host copies that outlive a re-pack of flipped rows (ms_ctx_equiangulate): per-facet gamma and body membership
+  std::vector<double> h_gamma;
+  std::vector<uint8_t> h_body;
+  // the last ms_ctx_equiangulate: selection rounds of every sweep run; ms of sweeps, D2H of the rows, pack, upload
+  std::vector<int32_t> eq_rounds;
+  double eq_ms[4] = {0, 0, 0, 0};
   int64_t n_send_rows = 0;
   // leaflet tilt modules (ms_leaflet.cuh): per-leaflet selections, parameters and tilt fields
   struct Leaflet {
@@ -450,6 +457,115 @@ void morton_permutation(const std::vector<double>& pos, int32_t nv, std::vector<
   if (identity) perm.clear();
 }
 
+// Packs triangle rows (internal vertex order) into `out` with the context's pack parameters.  A vertex of valence V
+// needs V rounds, i.e. V * threads record slots, and a patch holds at most kPatchSlotCap of them: meshes with
+// high-valence vertices (a disk centre, a cone apex) are packed with narrower rounds (96 -> 64 -> 32 lanes: valence
+// up to 16 / 24 / 48).  Changes nothing in the context.
+int pack_rows(const ms_ctx* c, int32_t nv, int32_t n_owned, int32_t nf, const int32_t* tri, const uint8_t* body_mask,
+              ms::PackedMesh& out) {
+  ms::PackParams used_params = c->pack_params;
+  int prc = ms::pack_patches(nv, nf, tri, body_mask, used_params, out, n_owned);
+  while (prc == -3 && used_params.threads > 32) {
+    used_params.threads = used_params.threads > 64 ? 64 : 32;
+    prc = ms::pack_patches(nv, nf, tri, body_mask, used_params, out, n_owned);
+  }
+  if (prc == -2) return fail(-8, "a vertex neighbourhood exceeds max_local; raise it with ms_ctx_set_pack_params");
+  if (prc == -3) return fail(-8, "a vertex has more than 48 incident facets: its rounds do not fit a patch");
+  if (prc) return fail(-1, "pack_patches failed");
+  if (out.max_owned > ms::kPatchOwnedCap || out.max_local > ms::kPatchLocalCap || out.max_slots > ms::kPatchSlotCap)
+    return fail(-8, "a patch exceeds the compiled shared-memory capacities");
+  return 0;
+}
+
+// Makes `packed` the context's packing and uploads it: patch ranges, interior-then-boundary patch order, headers,
+// halo ids and facet records.
+int upload_packing(ms_ctx* c, ms::PackedMesh&& packed, int32_t n_owned) {
+  c->packed = std::move(packed);
+  const ms::PackedMesh& pk = c->packed;
+  const size_t np = pk.patches.size();
+  c->v_lo.resize(np + 1);
+  for (size_t p = 0; p < np; ++p) c->v_lo[p] = pk.patches[p].v_lo;
+  c->v_lo[np] = n_owned;
+  {
+    std::vector<int32_t> order;
+    std::vector<int32_t> boundary;
+    for (size_t p = 0; p < np; ++p) {
+      const ms::PatchHeader& h = pk.patches[p];
+      bool ghost = false;
+      for (int32_t j = 0; j < h.n_halo && !ghost; ++j) ghost = pk.halo_ids[size_t(h.halo_off) + size_t(j)] >= n_owned;
+      (ghost ? boundary : order).push_back(int32_t(p));
+    }
+    c->n_interior = int32_t(order.size());
+    order.insert(order.end(), boundary.begin(), boundary.end());
+    if (int rc = c->d_patch_order.ensure(order.size() + 1)) return rc;
+    if (!order.empty()) CU(cudaMemcpy(c->d_patch_order.p, order.data(), order.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  }
+  if (int rc = c->d_patches.ensure(np + 1)) return rc;
+  if (int rc = c->d_halo.ensure(pk.halo_ids.size())) return rc;
+  if (int rc = c->d_recs.ensure(pk.recs.size())) return rc;
+  {  // sentinel header: closes the record range of the last patch
+    std::vector<ms::PatchHeader> hdr(pk.patches);
+    ms::PatchHeader end;
+    std::memset(&end, 0, sizeof(end));
+    end.v_lo = n_owned;
+    end.halo_off = int32_t(pk.halo_ids.size());
+    end.slot_off = int64_t(pk.recs.size());
+    hdr.push_back(end);
+    CU(cudaMemcpy(c->d_patches.p, hdr.data(), hdr.size() * sizeof(ms::PatchHeader), cudaMemcpyHostToDevice));
+  }
+  if (!pk.halo_ids.empty())
+    CU(cudaMemcpy(c->d_halo.p, pk.halo_ids.data(), pk.halo_ids.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+#ifdef MS_SELF_CHECK
+  if (std::getenv("MS_SELF_CHECK_INJECT")) {
+    // negative control of the self-check: slot 1 of every patch's first round repeats slot 0, so two lanes of one
+    // warp read-modify-write the same owned rows at once -- the row locks must report it
+    ms::PackedMesh& bad = c->packed;
+    for (const ms::PatchHeader& h : bad.patches)
+      if (h.n_rounds > 0 && (bad.recs[size_t(h.slot_off)].flags & ms::REC_VALID))
+        bad.recs[size_t(h.slot_off) + 1] = bad.recs[size_t(h.slot_off)];
+  }
+#endif
+  if (!pk.recs.empty())
+    CU(cudaMemcpy(c->d_recs.p, pk.recs.data(), pk.recs.size() * sizeof(ms::FacetRec), cudaMemcpyHostToDevice));
+  return 0;
+}
+
+// Per-facet surface tension of the record slots (slot_gamma) from the context's host copy and current packing.
+int upload_slot_gamma(ms_ctx* c) {
+  const ms::PackedMesh& pk = c->packed;
+  std::vector<double> slot_gamma(pk.slot_facet.size(), 0.0);
+  for (size_t s = 0; s < slot_gamma.size(); ++s)
+    if (pk.slot_facet[s] >= 0) slot_gamma[s] = c->h_gamma[size_t(pk.slot_facet[s])];
+  if (int rc = c->d_slot_gamma.ensure(slot_gamma.size())) return rc;
+  if (!slot_gamma.empty())
+    CU(cudaMemcpy(c->d_slot_gamma.p, slot_gamma.data(), slot_gamma.size() * sizeof(double), cudaMemcpyHostToDevice));
+  return 0;
+}
+
+// Forgets everything derived from the connectivity: it is rebuilt on first use (triangle rows, corner CSR,
+// bending-tilt buffers, pipelined-evaluation orders) or must be set again by the caller (leaflet selections, vertex
+// normals).  The conjugate-gradient history and a pending projection go too.
+void drop_connectivity_state(ms_ctx* c) {
+  c->proj.active = false;
+  c->bt_ready = false;
+  c->tri_ready = false;
+  c->csr_ready = false;
+  c->pipe_ready = false;
+  for (auto& lf : c->leaflet) {
+    lf.set = lf.has_fixed = lf.has_minv = false;
+    lf.trial.release(); lf.dir.release(); lf.minv.release();
+    lf.fixed.release();
+  }
+  c->vnormals_ready = false;
+  c->d_vnormals.release();
+  c->d_rowsq.release();
+  c->d_lf_corner.release(); c->d_lf_vbuf.release(); c->d_lf_shape.release(); c->d_lf_tilt.release();
+  c->d_lf_corner2.release(); c->d_lf_vbuf2.release(); c->d_lf_shape2.release(); c->d_lf_tilt2.release();
+  c->d_lf_facet_e.release();
+  c->d_cg_prev_g.release();
+  c->d_cg_prev_d.release();
+}
+
 template <typename T>
 std::vector<T> permuted(const T* src, const std::vector<int32_t>& perm) {
   std::vector<T> out(perm.size());
@@ -618,86 +734,19 @@ int ms_ctx_set_topology_partition(ms_ctx* c, int32_t nv, int32_t n_owned, int32_
     CU(cudaMemcpy(c->d_perm.p, c->perm.data(), size_t(nv) * sizeof(int32_t), cudaMemcpyHostToDevice));
     if (int rc = c->d_stage.ensure(size_t(ms::kSeedStride) * size_t(nv))) return rc;
   }
-  // A vertex of valence V needs V rounds, i.e. V * threads record slots, and a patch holds at most
-  // kPatchSlotCap of them: meshes with high-valence vertices (a disk centre, a cone apex) are packed with
-  // narrower rounds (96 -> 64 -> 32 lanes: valence up to 16 / 24 / 48).
-  ms::PackParams used_params = c->pack_params;
-  int prc = ms::pack_patches(nv, nf, tri, body_mask, used_params, c->packed, n_owned);
-  while (prc == -3 && used_params.threads > 32) {
-    used_params.threads = used_params.threads > 64 ? 64 : 32;
-    prc = ms::pack_patches(nv, nf, tri, body_mask, used_params, c->packed, n_owned);
-  }
-  if (prc == -2) return fail(-8, "a vertex neighbourhood exceeds max_local; raise it with ms_ctx_set_pack_params");
-  if (prc == -3) return fail(-8, "a vertex has more than 48 incident facets: its rounds do not fit a patch");
-  if (prc) return fail(-1, "pack_patches failed");
+  ms::PackedMesh packed;
+  if (int rc = pack_rows(c, nv, n_owned, nf, tri, body_mask, packed)) return rc;
   c->nv = nv;
   c->nf = nf;
   c->h_tri.assign(tri, tri + 3 * size_t(nf));
-  c->bt_ready = false;
-  c->tri_ready = false;
-  c->csr_ready = false;
+  if (body_mask) c->h_body.assign(body_mask, body_mask + size_t(nf)); else c->h_body.clear();
+  c->h_gamma.clear();
   c->has_positions = false;
-  c->pipe_ready = false;
-  for (auto& lf : c->leaflet) {  // per-leaflet arrays are sized for the previous vertex count
-    lf.set = lf.has_fixed = lf.has_minv = false;
-    lf.tilts.release(); lf.tilt_grad.release(); lf.trial.release(); lf.dir.release(); lf.minv.release();
-    lf.fixed.release();
+  drop_connectivity_state(c);
+  for (auto& lf : c->leaflet) {  // per-leaflet tilt fields are sized for the previous vertex count
+    lf.tilts.release(); lf.tilt_grad.release();
   }
-  c->vnormals_ready = false;
-  c->d_vnormals.release();
-  c->d_rowsq.release();
-  c->d_lf_corner.release(); c->d_lf_vbuf.release(); c->d_lf_shape.release(); c->d_lf_tilt.release();
-  c->d_lf_corner2.release(); c->d_lf_vbuf2.release(); c->d_lf_shape2.release(); c->d_lf_tilt2.release();
-  c->d_lf_facet_e.release();
-  const ms::PackedMesh& pk = c->packed;
-  const size_t np = pk.patches.size();
-  c->v_lo.resize(np + 1);
-  for (size_t p = 0; p < np; ++p) c->v_lo[p] = pk.patches[p].v_lo;
-  c->v_lo[np] = n_owned;
-  {
-    std::vector<int32_t> order;
-    std::vector<int32_t> boundary;
-    for (size_t p = 0; p < np; ++p) {
-      const ms::PatchHeader& h = pk.patches[p];
-      bool ghost = false;
-      for (int32_t j = 0; j < h.n_halo && !ghost; ++j) ghost = pk.halo_ids[size_t(h.halo_off) + size_t(j)] >= n_owned;
-      (ghost ? boundary : order).push_back(int32_t(p));
-    }
-    c->n_interior = int32_t(order.size());
-    order.insert(order.end(), boundary.begin(), boundary.end());
-    if (int rc = c->d_patch_order.ensure(order.size() + 1)) return rc;
-    if (!order.empty()) CU(cudaMemcpy(c->d_patch_order.p, order.data(), order.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-  }
-
-  if (prc == 0 && (pk.max_owned > ms::kPatchOwnedCap || pk.max_local > ms::kPatchLocalCap || pk.max_slots > ms::kPatchSlotCap))
-    return fail(-8, "a patch exceeds the compiled shared-memory capacities");
-  if (int rc = c->d_patches.ensure(np + 1)) return rc;
-  if (int rc = c->d_halo.ensure(pk.halo_ids.size())) return rc;
-  if (int rc = c->d_recs.ensure(pk.recs.size())) return rc;
-  {  // sentinel header: closes the record range of the last patch
-    std::vector<ms::PatchHeader> hdr(pk.patches);
-    ms::PatchHeader end;
-    std::memset(&end, 0, sizeof(end));
-    end.v_lo = n_owned;
-    end.halo_off = int32_t(pk.halo_ids.size());
-    end.slot_off = int64_t(pk.recs.size());
-    hdr.push_back(end);
-    CU(cudaMemcpy(c->d_patches.p, hdr.data(), hdr.size() * sizeof(ms::PatchHeader), cudaMemcpyHostToDevice));
-  }
-  if (!pk.halo_ids.empty())
-    CU(cudaMemcpy(c->d_halo.p, pk.halo_ids.data(), pk.halo_ids.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-#ifdef MS_SELF_CHECK
-  if (std::getenv("MS_SELF_CHECK_INJECT")) {
-    // negative control of the self-check: slot 1 of every patch's first round repeats slot 0, so two lanes of one
-    // warp read-modify-write the same owned rows at once -- the row locks must report it
-    ms::PackedMesh& bad = c->packed;
-    for (const ms::PatchHeader& h : bad.patches)
-      if (h.n_rounds > 0 && (bad.recs[size_t(h.slot_off)].flags & ms::REC_VALID))
-        bad.recs[size_t(h.slot_off) + 1] = bad.recs[size_t(h.slot_off)];
-  }
-#endif
-  if (!pk.recs.empty())
-    CU(cudaMemcpy(c->d_recs.p, pk.recs.data(), pk.recs.size() * sizeof(ms::FacetRec), cudaMemcpyHostToDevice));
+  if (int rc = upload_packing(c, std::move(packed), n_owned)) return rc;
 
   c->has_boundary = is_boundary != nullptr;
   c->has_fixed = fixed_mask != nullptr;
@@ -733,8 +782,6 @@ int ms_ctx_set_topology_partition(ms_ctx* c, int32_t nv, int32_t n_owned, int32_
   }
   // per-entity parameter arrays belong to the previous topology
   c->has_gamma = c->has_kappa = c->has_c0 = false;
-  c->d_cg_prev_g.release();
-  c->d_cg_prev_d.release();
   c->d_tilts.release();
   c->d_tilt_sq.release();
   c->d_tilt_grad.release();
@@ -825,14 +872,10 @@ int ms_ctx_set_surface_tension(ms_ctx* c, const double* gamma, double gamma_unif
   if (int rc = check_ctx(c, true)) return rc;
   c->gamma_u = gamma_uniform;
   c->has_gamma = false;
+  c->h_gamma.clear();
   if (!gamma) return 0;
-  const ms::PackedMesh& pk = c->packed;
-  std::vector<double> slot_gamma(pk.slot_facet.size(), 0.0);
-  for (size_t s = 0; s < slot_gamma.size(); ++s)
-    if (pk.slot_facet[s] >= 0) slot_gamma[s] = gamma[pk.slot_facet[s]];
-  if (int rc = c->d_slot_gamma.ensure(slot_gamma.size())) return rc;
-  if (!slot_gamma.empty())
-    CU(cudaMemcpy(c->d_slot_gamma.p, slot_gamma.data(), slot_gamma.size() * sizeof(double), cudaMemcpyHostToDevice));
+  c->h_gamma.assign(gamma, gamma + size_t(c->nf));
+  if (int rc = upload_slot_gamma(c)) return rc;
   c->has_gamma = true;
   return 0;
 }
@@ -2185,6 +2228,137 @@ int ms_ctx_vertex_average(ms_ctx* c, const int32_t* group, int32_t rounds) {
   }
   if (rounds & 1)
     CU(cudaMemcpyAsync(c->d_pos.p, c->d_trial.p, 3 * nv * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+  return 0;
+}
+
+int ms_ctx_equiangulate(ms_ctx* c, int32_t max_iterations, int64_t* n_flips, int32_t* n_sweeps) {
+  if (int rc = check_ctx(c, true)) return rc;
+  if (c->n_owned != c->nv) return fail(-5, "equiangulation is not available on a partitioned context");
+  if (max_iterations < 0) return fail(-1, "max_iterations must be >= 0");
+  if (!c->has_positions) return fail(-4, "no positions have been set (MS_ARR_POSITIONS)");
+  for (int32_t x : c->h_tri)
+    if (x < 0 || x >= c->nv) return fail(-1, "a facet has a vertex index outside [0, nv)");
+  c->eq_rounds.clear();
+  std::fill(c->eq_ms, c->eq_ms + 4, 0.0);
+  if (n_flips) *n_flips = 0;
+  if (n_sweeps) *n_sweeps = 0;
+  if (max_iterations == 0 || c->nf == 0) return 0;
+  if (int rc = ensure_tri(c)) return rc;
+  NvtxRange range("ms_b200 equiangulate");
+  using clock = std::chrono::steady_clock;
+  auto ms_since = [](clock::time_point t0) { return std::chrono::duration<double, std::milli>(clock::now() - t0).count(); };
+  const size_t nh = 3 * size_t(c->nf), nc_max = nh / 2 + 1;
+  constexpr int kBatch = 8;  // selection rounds between two reads of the undecided counters
+  // sweep scratch, released on return: sorted half-edge keys, candidates, conflict lists, round states, counters
+  DevBuf<uint64_t> key_in, keys, nkey;
+  DevBuf<int32_t> h_in, order, cand_pos, h1, h2, slot, nkey_cand, nkey_pos, counters;
+  DevBuf<uint8_t> flag, state0, state1, temp;
+  size_t tb_edges = 0, tb_cands = 0;
+  CU(ms::eq_temp_bytes(int64_t(nh), &tb_edges));
+  CU(ms::eq_temp_bytes(int64_t(nc_max), &tb_cands));
+  const size_t tb = std::max(tb_edges, tb_cands);
+  for (int rc : {key_in.ensure(nh), keys.ensure(nh), nkey.ensure(nc_max), h_in.ensure(nh), order.ensure(nh),
+                 cand_pos.ensure(nh), h1.ensure(nc_max), h2.ensure(nc_max), slot.ensure(nh), nkey_cand.ensure(nc_max),
+                 nkey_pos.ensure(nc_max), counters.ensure(kBatch + 2), flag.ensure(nh), state0.ensure(nc_max),
+                 state1.ensure(nc_max), temp.ensure(tb + 1)})
+    if (rc) return rc;
+  ms::EqMesh m{c->nv, c->nf, c->d_tri.p, c->d_pos.p, c->has_fixed ? c->d_fixed.p : nullptr,
+               c->perm.empty() ? nullptr : c->d_perm.p, keys.p, order.p};
+  ms::EqCands s{0, h1.p, h2.p, slot.p, nkey.p, nkey_cand.p, nkey_pos.p};
+  uint8_t* state[2] = {state0.p, state1.p};
+  int32_t h_counters[kBatch + 2];
+  int64_t total = 0;
+  int32_t sweeps = 0;
+  struct Events {  // the sweeps' device time; the context's own events belong to ms_ctx_timer_*
+    cudaEvent_t e[2] = {nullptr, nullptr};
+    ~Events() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
+  } ev;
+  CU(cudaEventCreate(&ev.e[0]));
+  CU(cudaEventCreate(&ev.e[1]));
+  CU(cudaEventRecord(ev.e[0], c->stream));
+  for (int32_t sweep = 0; sweep < max_iterations; ++sweep) {
+    CU(ms::launch_eq_sort_edges(m, key_in.p, h_in.p, keys.p, order.p, temp.p, tb, c->stream));
+    CU(ms::launch_eq_candidates(m, flag.p, cand_pos.p, counters.p + kBatch, temp.p, tb, c->stream));
+    CU(cudaMemcpyAsync(h_counters + kBatch, counters.p + kBatch, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    s.n = h_counters[kBatch];
+    if (s.n == 0) {
+      c->eq_rounds.push_back(0);
+      break;
+    }
+    // the sort inputs are free again: they hold the candidates' new-diagonal keys and ids
+    CU(ms::launch_eq_conflicts(m, s.n, cand_pos.p, s, key_in.p, h_in.p, temp.p, tb, c->stream));
+    CU(cudaMemsetAsync(state[0], 0, size_t(s.n), c->stream));
+    int32_t done = -1;  // the round after which no candidate was undecided
+    for (int32_t r0 = 0; done < 0; r0 += kBatch) {
+      if (r0 > s.n) return fail(-1, "equiangulation: the selection rounds do not converge");  // cannot happen
+      CU(cudaMemsetAsync(counters.p, 0, kBatch * sizeof(int32_t), c->stream));
+      for (int k = 0; k < kBatch; ++k)
+        CU(ms::launch_eq_round(s, state[(r0 + k) & 1], state[(r0 + k + 1) & 1], k ? counters.p + k - 1 : nullptr,
+                               counters.p + k, c->stream));
+      CU(cudaMemcpyAsync(h_counters, counters.p, kBatch * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+      CU(cudaStreamSynchronize(c->stream));
+      for (int k = 0; k < kBatch && done < 0; ++k)
+        if (h_counters[k] == 0) done = r0 + k;
+    }
+    CU(cudaMemsetAsync(counters.p + kBatch + 1, 0, sizeof(int32_t), c->stream));
+    CU(ms::launch_eq_apply(s, state[(done + 1) & 1], c->d_tri.p, counters.p + kBatch + 1, c->stream));
+    CU(cudaMemcpyAsync(h_counters + kBatch + 1, counters.p + kBatch + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    c->eq_rounds.push_back(done + 1);
+    total += h_counters[kBatch + 1];
+    ++sweeps;
+  }
+  CU(cudaEventRecord(ev.e[1], c->stream));
+  CU(cudaEventSynchronize(ev.e[1]));
+  float sweep_ms = 0.f;
+  CU(cudaEventElapsedTime(&sweep_ms, ev.e[0], ev.e[1]));
+  c->eq_ms[0] = sweep_ms;
+  if (total > 0) {
+    // facet rows stay in place, so per-facet and per-vertex data survive; only the packing follows the new rows
+    auto t0 = clock::now();
+    std::vector<int32_t> rows(nh);
+    CU(cudaMemcpy(rows.data(), c->d_tri.p, nh * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    c->eq_ms[1] = ms_since(t0);
+    t0 = clock::now();
+    ms::PackedMesh packed;
+    const int rc = pack_rows(c, c->nv, c->nv, c->nf, rows.data(), c->h_body.empty() ? nullptr : c->h_body.data(), packed);
+    c->eq_ms[2] = ms_since(t0);
+    if (rc) {  // the flipped rows do not pack: back to the rows and packing the context had
+      const std::string why = g_err;
+      CU(cudaMemcpy(c->d_tri.p, c->h_tri.data(), nh * sizeof(int32_t), cudaMemcpyHostToDevice));
+      return fail(rc, "equiangulation: " + why + "; the context keeps its previous triangles");
+    }
+    t0 = clock::now();
+    c->h_tri.swap(rows);
+    drop_connectivity_state(c);
+    c->tri_ready = true;  // d_tri holds the new rows
+    if (int rc2 = upload_packing(c, std::move(packed), c->nv)) return rc2;
+    if (c->has_gamma)
+      if (int rc2 = upload_slot_gamma(c)) return rc2;
+    c->eq_ms[3] = ms_since(t0);
+  }
+  if (n_flips) *n_flips = total;
+  if (n_sweeps) *n_sweeps = sweeps;
+  return 0;
+}
+
+int ms_ctx_equiangulate_stats(const ms_ctx* c, double* ms4, int32_t* rounds, int32_t capacity, int32_t* n_sweeps_run) {
+  if (!c || !n_sweeps_run) return fail(-1, "null argument");
+  *n_sweeps_run = int32_t(c->eq_rounds.size());
+  if (ms4) std::copy(c->eq_ms, c->eq_ms + 4, ms4);
+  if (rounds)
+    for (int32_t i = 0; i < capacity && size_t(i) < c->eq_rounds.size(); ++i) rounds[i] = c->eq_rounds[size_t(i)];
+  return 0;
+}
+
+int ms_ctx_get_triangles(const ms_ctx* c, int32_t* out) {
+  if (!c || !out) return fail(-1, "null argument");
+  if (!c->have_topology) return fail(-2, "ms_ctx_set_topology has not been called");
+  for (size_t i = 0; i < c->h_tri.size(); ++i) {
+    const int32_t x = c->h_tri[i];
+    out[i] = (!c->perm.empty() && x >= 0 && x < c->nv) ? c->perm[size_t(x)] : x;
+  }
   return 0;
 }
 

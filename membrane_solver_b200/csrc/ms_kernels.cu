@@ -23,6 +23,10 @@
 // Reference functions replaced: see the header of ms_math.cuh.
 #include "ms_kernels.cuh"
 
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_select.cuh>
+#include <cub/iterator/counting_input_iterator.cuh>
+
 #include "ms_bt.cuh"
 #include "ms_patch_body.cuh"
 
@@ -1417,6 +1421,62 @@ __global__ void __launch_bounds__(128) k_vertex_average(const VaMesh m, double* 
   st3(out, v, va_vertex(m, v));
 }
 
+// --- equiangulation (ms_equiangulate.cuh): one thread per half-edge, sorted edge, or candidate ---
+__global__ void __launch_bounds__(256) k_eq_keys(const EqMesh m, uint64_t* __restrict__ key, int32_t* __restrict__ h_out) {
+  const int64_t h = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (h >= 3 * int64_t(m.nf)) return;
+  key[h] = eq_key(m, eq_tail(m, h), eq_head(m, h));
+  h_out[h] = int32_t(h);
+}
+
+__global__ void __launch_bounds__(256) k_eq_flag(const EqMesh m, uint8_t* __restrict__ flag) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= 3 * int64_t(m.nf)) return;
+  int64_t h1 = 0, h2 = 0;
+  flag[i] = eq_interior(m, i, h1, h2) && eq_should_flip(m, h1, h2);
+}
+
+__global__ void __launch_bounds__(256) k_eq_cands(const EqMesh m, int32_t nc, const int32_t* __restrict__ cand_pos,
+                                                  int32_t* __restrict__ h1, int32_t* __restrict__ h2,
+                                                  int32_t* __restrict__ slot_cand, uint64_t* __restrict__ nkey,
+                                                  int32_t* __restrict__ id) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= nc) return;
+  const int32_t a = m.order[cand_pos[i]], b = m.order[cand_pos[i] + 1];
+  h1[i] = a;
+  h2[i] = b;
+  slot_cand[a] = i;
+  slot_cand[b] = i;
+  nkey[i] = eq_key(m, eq_apex(m, a), eq_apex(m, b));
+  id[i] = i;
+}
+
+__global__ void __launch_bounds__(256) k_eq_nkey_pos(int32_t nc, const int32_t* __restrict__ nkey_cand,
+                                                     int32_t* __restrict__ nkey_pos) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p < nc) nkey_pos[nkey_cand[p]] = p;
+}
+
+// one Jacobi round; a round after the one that left no candidate undecided returns at once
+__global__ void __launch_bounds__(256) k_eq_round(const EqCands s, const uint8_t* __restrict__ in, uint8_t* __restrict__ out,
+                                                  const int32_t* __restrict__ prev_undecided, int32_t* undecided) {
+  if (prev_undecided && *prev_undecided == 0) return;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const uint8_t st = i < s.n ? eq_round(s, in, i) : uint8_t(EQ_SELECTED);
+  if (i < s.n) out[i] = st;
+  const unsigned open = __ballot_sync(0xffffffffu, st == EQ_UNDECIDED);
+  if (open && (threadIdx.x & 31) == 0) atomicAdd(undecided, __popc(open));
+}
+
+__global__ void __launch_bounds__(256) k_eq_apply(const EqCands s, const uint8_t* __restrict__ state, int32_t* tri,
+                                                  int32_t* flips) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const bool sel = i < s.n && state[i] == EQ_SELECTED;
+  if (sel) eq_apply(tri, s.h1[i], s.h2[i]);
+  const unsigned mask = __ballot_sync(0xffffffffu, sel);
+  if (mask && (threadIdx.x & 31) == 0) atomicAdd(flips, __popc(mask));
+}
+
 // t -= (t.n) n  (runtime/projections/tilt.py:8-14)
 __global__ void __launch_bounds__(256) k_project_tangent(int64_t nv, const double* __restrict__ normals, double* t) {
   const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -2092,6 +2152,69 @@ cudaError_t launch_vertex_normals(int32_t nv, const int32_t* tri, const int32_t*
 
 cudaError_t launch_vertex_average(const VaMesh& m, double* out, cudaStream_t st) {
   if (m.nv > 0) k_vertex_average<<<blocks_for(m.nv, 128), 128, 0, st>>>(m, out);
+  return cudaGetLastError();
+}
+
+int eq_key_bits(int32_t nv) {
+  const uint64_t top = nv > 1 ? uint64_t(nv) * uint64_t(nv) - 1 : 1;
+  int bits = 0;
+  while (bits < 64 && (top >> bits)) ++bits;
+  return bits;
+}
+
+cudaError_t eq_temp_bytes(int64_t n_half_edges, size_t* bytes) {
+  size_t a = 0, b = 0;
+  const int n = int(n_half_edges);
+  cudaError_t e = cub::DeviceRadixSort::SortPairs(nullptr, a, (const uint64_t*)nullptr, (uint64_t*)nullptr,
+                                                  (const int32_t*)nullptr, (int32_t*)nullptr, n);
+  if (e != cudaSuccess) return e;
+  e = cub::DeviceSelect::Flagged(nullptr, b, cub::CountingInputIterator<int32_t>(0), (const uint8_t*)nullptr,
+                                 (int32_t*)nullptr, (int32_t*)nullptr, n);
+  *bytes = a > b ? a : b;
+  return e;
+}
+
+cudaError_t launch_eq_sort_edges(const EqMesh& m, uint64_t* key_in, int32_t* h_in, uint64_t* keys, int32_t* order,
+                                 void* temp, size_t temp_bytes, cudaStream_t st) {
+  const int64_t n = 3 * int64_t(m.nf);
+  if (n == 0) return cudaSuccess;
+  k_eq_keys<<<blocks_for(n, 256), 256, 0, st>>>(m, key_in, h_in);
+  if (cudaError_t e = cudaGetLastError()) return e;
+  return cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_in, keys, h_in, order, int(n), 0, eq_key_bits(m.nv), st);
+}
+
+cudaError_t launch_eq_candidates(const EqMesh& m, uint8_t* flag, int32_t* cand_pos, int32_t* n_cand, void* temp,
+                                 size_t temp_bytes, cudaStream_t st) {
+  const int64_t n = 3 * int64_t(m.nf);
+  if (n == 0) return cudaMemsetAsync(n_cand, 0, sizeof(int32_t), st);
+  k_eq_flag<<<blocks_for(n, 256), 256, 0, st>>>(m, flag);
+  if (cudaError_t e = cudaGetLastError()) return e;
+  return cub::DeviceSelect::Flagged(temp, temp_bytes, cub::CountingInputIterator<int32_t>(0), flag, cand_pos, n_cand,
+                                    int(n), st);
+}
+
+cudaError_t launch_eq_conflicts(const EqMesh& m, int32_t nc, const int32_t* cand_pos, const EqCands& s,
+                                uint64_t* nkey_in, int32_t* id_in, void* temp, size_t temp_bytes, cudaStream_t st) {
+  if (cudaError_t e = cudaMemsetAsync(const_cast<int32_t*>(s.slot_cand), 0xff, 3 * size_t(m.nf) * sizeof(int32_t), st)) return e;
+  if (nc == 0) return cudaSuccess;
+  k_eq_cands<<<blocks_for(nc, 256), 256, 0, st>>>(m, nc, cand_pos, const_cast<int32_t*>(s.h1), const_cast<int32_t*>(s.h2),
+                                                  const_cast<int32_t*>(s.slot_cand), nkey_in, id_in);
+  if (cudaError_t e = cudaGetLastError()) return e;
+  if (cudaError_t e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, nkey_in, const_cast<uint64_t*>(s.nkey), id_in,
+                                                      const_cast<int32_t*>(s.nkey_cand), nc, 0, eq_key_bits(m.nv), st))
+    return e;
+  k_eq_nkey_pos<<<blocks_for(nc, 256), 256, 0, st>>>(nc, s.nkey_cand, const_cast<int32_t*>(s.nkey_pos));
+  return cudaGetLastError();
+}
+
+cudaError_t launch_eq_round(const EqCands& s, const uint8_t* in, uint8_t* out, const int32_t* prev_undecided,
+                            int32_t* undecided, cudaStream_t st) {
+  if (s.n > 0) k_eq_round<<<blocks_for(s.n, 256), 256, 0, st>>>(s, in, out, prev_undecided, undecided);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_eq_apply(const EqCands& s, const uint8_t* state, int32_t* tri, int32_t* flips, cudaStream_t st) {
+  if (s.n > 0) k_eq_apply<<<blocks_for(s.n, 256), 256, 0, st>>>(s, state, tri, flips);
   return cudaGetLastError();
 }
 

@@ -10,6 +10,7 @@
 #include "ms_leaflet.cuh"
 #include "ms_math.cuh"
 #include "ms_pack.h"
+#include "ms_equiangulate.cuh"
 #include "ms_vertex_average.cuh"
 
 namespace ms {
@@ -317,5 +318,24 @@ cudaError_t launch_masked_norm2(int64_t nv, double* g, const uint8_t* fixed, dou
 
 // --- vertex averaging (the `V` command): one thread per vertex, m.pos -> out (a different buffer) ---
 cudaError_t launch_vertex_average(const VaMesh& m, double* out, cudaStream_t st);
+
+// --- equiangulation (the `u` command), one sweep in four steps (ms_equiangulate.cuh) ---
+// scratch of the sorts and the candidate selection for up to n_half_edges items
+cudaError_t eq_temp_bytes(int64_t n_half_edges, size_t* bytes);
+// half-edge keys (caller numbering) sorted stably with their half-edge ids into keys / order (= m.keys / m.order)
+cudaError_t launch_eq_sort_edges(const EqMesh& m, uint64_t* key_in, int32_t* h_in, uint64_t* keys, int32_t* order,
+                                 void* temp, size_t temp_bytes, cudaStream_t st);
+// sorted positions of the interior edges that pass eq_should_flip, in ascending key; their count to *n_cand (device)
+cudaError_t launch_eq_candidates(const EqMesh& m, uint8_t* flag, int32_t* cand_pos, int32_t* n_cand, void* temp,
+                                 size_t temp_bytes, cudaStream_t st);
+// fills s.h1 / s.h2 / s.slot_cand / s.nkey / s.nkey_cand / s.nkey_pos of the nc candidates
+cudaError_t launch_eq_conflicts(const EqMesh& m, int32_t nc, const int32_t* cand_pos, const EqCands& s,
+                                uint64_t* nkey_in, int32_t* id_in, void* temp, size_t temp_bytes, cudaStream_t st);
+// one selection round in -> out; adds the candidates it leaves undecided to *undecided; does nothing when
+// *prev_undecided (the previous round's count, may be null) is 0
+cudaError_t launch_eq_round(const EqCands& s, const uint8_t* in, uint8_t* out, const int32_t* prev_undecided,
+                            int32_t* undecided, cudaStream_t st);
+// rewrites the rows of the selected candidates; adds their number to *flips
+cudaError_t launch_eq_apply(const EqCands& s, const uint8_t* state, int32_t* tri, int32_t* flips, cudaStream_t st);
 
 }  // namespace ms

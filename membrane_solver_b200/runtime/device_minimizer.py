@@ -109,6 +109,18 @@ class DeviceMinimizer:
         self._cg_have_history = False
         self._cg_iter = 0
 
+    # -- the u command (commands/mesh_ops.py) ----------------------------------------------------------
+    def equiangulate(self, max_iterations: int = 100) -> int:
+        """Equiangulation on the device (``DeviceMesh.equiangulate``), then, with ``enforce_volume``, the hard volume
+        projection of the ``mesh_operation`` context (12 iterations).  The conjugate-gradient history is discarded,
+        as after ``vertex_average``.  Returns the number of flips."""
+        flips = self.dm.equiangulate(int(max_iterations))
+        if self.enforce_volume:
+            self._enforce(trial=False, max_iter=12)
+        self._cg_have_history = False
+        self._cg_iter = 0
+        return flips
+
     # -- one line search (line_search.py:267-430) --------------------------------------------------
     def _line_search(self, step_size: float):
         dm = self.dm
