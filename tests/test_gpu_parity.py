@@ -11,7 +11,7 @@ import ctypes
 import numpy as np
 import pytest
 
-from ms_test_helpers import golden_ids, golden_module_files, rel_err
+from ms_test_helpers import golden_ids, golden_module_files, rel_err, volgrad_close
 
 pytestmark = pytest.mark.gpu
 
@@ -514,16 +514,6 @@ def test_full_size_invariants(L):
 
 
 # -------------------------------------------------------------- parity at size (BASELINE.json configs[2], configs[4])
-def _volgrad_close(got, want, pos):
-    """dV/dx_v = 1/6 sum_i p_i x p_(i+1) cancels from O(|p|^2) summands down to O(h^2): on fine meshes the
-    reference's own result moves by more than 1e-12 of its magnitude when its sum is re-ordered.  The bound is
-    therefore 1e-12 relative to the size of the summands, and 1e-10 relative to max |dV/dx|."""
-    err = float(np.abs(np.asarray(got) - np.asarray(want)).max())
-    summand = float((np.asarray(pos) ** 2).sum(axis=1).max()) / 6.0
-    assert err <= TOL * summand, (err, summand)
-    assert err <= 1e-10 * float(np.abs(want).max()), (err, float(np.abs(want).max()))
-
-
 def test_million_facet_icosphere_vs_oracle(L):
     """1 003 520 facets: the largest mesh on which the whole-mesh oracle runs in seconds; energies, gradient and
     dV/dx of the fused evaluation and of the KKT-projected evaluation at 1e-12 relative."""
@@ -544,7 +534,7 @@ def test_million_facet_icosphere_vs_oracle(L):
     g = dm.download(L.ARR_GRAD)
     gv = dm.download(L.ARR_VOLGRAD)
     assert rel_err(g, want["grad"]) <= TOL
-    _volgrad_close(gv, want["vol_grad"], pos)
+    volgrad_close(gv, want["vol_grad"], pos)
     rp = dm.eval(dm.options(mods, constraint_mode=0))
     lam = float(np.vdot(want["grad"], want["vol_grad"]) / np.vdot(want["vol_grad"], want["vol_grad"]))
     assert abs(rp.kkt_lambda - lam) <= 1e-10 * abs(lam)
@@ -575,7 +565,7 @@ def test_bending_cube_r8_vs_oracle(L):
     _scalar_close(r.e_bending, want["E_bending"])
     _scalar_close(r.volume, want["volume"])
     assert rel_err(dm.download(L.ARR_GRAD), want["grad"]) <= 2e-12
-    _volgrad_close(dm.download(L.ARR_VOLGRAD), want["vol_grad"], pos)
+    volgrad_close(dm.download(L.ARR_VOLGRAD), want["vol_grad"], pos)
     dm.close()
 
 
@@ -642,32 +632,42 @@ def test_pipelined_host_evaluation_matches_staged_path(L):
     nv, nf = pos.shape[0], tri.shape[0]
     rng = np.random.default_rng(11)
     pos = pos * (1.0 + 0.01 * rng.standard_normal((nv, 1)))
-    dm = _ctx(nv, tri, body_mask=np.ones(nf, np.uint8))
-    dm.set_surface_tension(1.0)
-    dm.set_bending_params(1.3, 0.02)
-    for mods, kw in ((L.MOD_SURFACE | L.MOD_BENDING | L.MOD_VOLUME, {}),
-                     (L.MOD_SURFACE | L.MOD_BENDING | L.MOD_VOLUME, dict(constraint_mode=0)),
-                     (L.MOD_SURFACE | L.MOD_VOLUME, {}),
-                     (L.MOD_SURFACE | L.MOD_BENDING | L.MOD_VOLUME, dict(want_grad=0))):
+    dm = _ctx(nv, tri, body_mask=np.ones(nf, np.uint8), fixed_mask=(rng.random(nv) < 0.05).astype(np.uint8))
+    kappa, c0 = 1.0 + 0.3 * rng.random(nv), 0.05 * rng.random(nv)
+    gamma = 1.0 + 0.2 * rng.random(nf)
+    sbv = L.MOD_SURFACE | L.MOD_BENDING | L.MOD_VOLUME
+    # (modules, options, per-vertex kappa / c0, per-facet gamma)
+    for mods, kw, per_vertex, per_facet in (
+            (sbv, {}, False, False),
+            (sbv, dict(constraint_mode=0), False, False),
+            (L.MOD_SURFACE | L.MOD_VOLUME, {}, False, False),
+            (sbv, dict(want_grad=0), False, False),
+            (sbv, {}, True, False),                                 # kind 3 through the pipeline
+            (L.MOD_SURFACE | L.MOD_VOLUME, {}, False, True),        # kind 0 pass B summing the scalars itself
+            (sbv, dict(use_trial=1), False, False),                 # the rows travel into the trial positions
+            (sbv, dict(constraint_mode=1, k_vol=2.0, v_target=3.9, apply_fixed=1), False, False)):
+        dm.set_bending_params(kappa if per_vertex else 1.3, c0 if per_vertex else 0.02)
+        dm.set_surface_tension(gamma if per_facet else 1.0)
         opts = dm.options(mods, **kw)
-        dm.set_positions(pos)
+        target = L.ARR_TRIAL if kw.get("use_trial") else L.ARR_POSITIONS
+        dm.upload(target, pos)
         want = dm.eval(opts)
         want_g, want_v = dm.download(L.ARR_GRAD), dm.download(L.ARR_VOLGRAD)
-        dm.set_positions(np.zeros_like(pos))       # the pipelined call must bring every row itself
+        dm.upload(target, np.zeros_like(pos))      # the pipelined call must bring every row itself
         g, v = np.full_like(pos, np.nan), np.full_like(pos, np.nan)
         got = dm.eval_host(opts, pos, grad=g, volgrad=v)
         for name in ("e_surface", "e_bending", "area", "volume"):
             _scalar_close(getattr(got, name), getattr(want, name))
         if kw.get("want_grad", 1):
             if "constraint_mode" in kw:
-                assert rel_err(g, want_g) <= 1e-12      # lambda comes from the re-grouped sums
+                assert rel_err(g, want_g) <= 1e-12      # the coefficient comes from the re-grouped sums
             else:
                 assert np.array_equal(g, want_g)
             assert np.array_equal(v, want_v)
             g2 = np.empty_like(pos)
             dm.eval_host(opts, pos, grad=g2)
             assert np.array_equal(g2, g)               # and it repeats bitwise
-        assert np.array_equal(dm.download(L.ARR_POSITIONS), pos)
+        assert np.array_equal(dm.download(target), pos)
     dm.close()
 
 
