@@ -440,7 +440,8 @@ class DeviceMesh:
 
     def eval_partition(self, opts, exchange_positions: bool = True, in_kernel: bool = False) -> None:
         """One partitioned evaluation with the transport folded into the compute launches (5 launches), or, with
-        ``in_kernel``, carried out inside the patch kernels behind the interior patches (3 launches)."""
+        ``in_kernel``, carried out inside the patch kernels behind the interior patches (2 launches: pass A and pass B, the
+        last CTA of the last pass gathering the scalars; a pack of fewer than 64 threads falls back to the fused pull)."""
         flags = int(bool(exchange_positions)) | (2 if in_kernel else 0)
         L.check(self._lib.ms_ctx_eval_partition(self._h, ctypes.byref(opts), flags))
 

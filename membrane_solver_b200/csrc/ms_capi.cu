@@ -1622,7 +1622,13 @@ int ms_ctx_halo_prepare(ms_ctx* c) {
   if (int rc = check_ctx(c, true)) return rc;
   if (int rc = ensure_flag_words(c)) return rc;
   if (int rc = peer_tables(c)) return rc;
-  CU(ms::launch_halo_warmup(c->d_flag_words.p, c->d_scalars.p, c->d_halo_error.p, c->stream));
+  // the tickets of the fused finalisation, the push kernel and the in-kernel pulls: allocated here, not inside the
+  // lock-step sequence (zeroed once only: d_ticket[2] must stay in step with the host mirror pull_arrived)
+  if (!c->d_ticket.p) {
+    if (int rc = c->d_ticket.ensure(4)) return rc;
+    CU(cudaMemsetAsync(c->d_ticket.p, 0, 4 * sizeof(unsigned int), c->stream));
+  }
+  CU(ms::launch_halo_warmup(c->d_flag_words.p, c->d_scalars.p, c->d_halo_error.p, c->d_ticket.p + 1, c->stream));
   CU(cudaDeviceSynchronize());
   return 0;
 }

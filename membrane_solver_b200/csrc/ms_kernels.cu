@@ -2373,7 +2373,8 @@ cudaError_t launch_allreduce_peer(double* scalars, int n, unsigned long long* ow
 
 // First launches load the kernels' code (lazy module loading), which may synchronise the device: do them once,
 // with no work, before contexts start waiting for each other.
-cudaError_t launch_halo_warmup(unsigned long long* words, double* scalars, int* error, cudaStream_t st) {
+cudaError_t launch_halo_warmup(unsigned long long* words, double* scalars, int* error, unsigned int* push_ticket,
+                               cudaStream_t st) {
   k_halo_signal<<<1, 1, 0, st>>>(words + 3, 0ull);
   k_halo_pull<<<1, 256, 0, st>>>(0, 3, nullptr, nullptr, 0, 0, 0ull, nullptr, nullptr, nullptr, error);
   k_allreduce_publish<<<1, 32, 0, st>>>(scalars, 0, words, 0ull);
@@ -2384,6 +2385,11 @@ cudaError_t launch_halo_warmup(unsigned long long* words, double* scalars, int* 
   k_halo_exchange<<<1, 256, 0, st>>>(words + 3, 0, 3, nullptr, nullptr, 0, 0, 0ull, nullptr, nullptr, nullptr, error);
   k_reduce_partials<<<1, kReduceRows * kPartialStride, 0, st>>>(nullptr, 0, nullptr, 0, 0u, scalars);
   k_kkt_coefficient<<<1, 1, 0, st>>>(scalars, -1, 0, 0.0, 0.0);
+  // push transport: no row, no destination (the single block takes the ticket and puts it back to 0); no rank to wait
+  // for, no scalar written
+  k_halo_push<<<1, 256, 0, st>>>(0, 3, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0, 0ull, 0, 0, 0ull,
+                                 push_ticket);
+  k_allreduce_local_coef<<<1, 64, 0, st>>>(words, 0, 0, 0ull, scalars, -2, 0, 0.0, 0.0, error);
   return cudaGetLastError();
 }
 

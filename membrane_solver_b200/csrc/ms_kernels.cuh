@@ -282,7 +282,8 @@ cudaError_t launch_halo_exchange(unsigned long long* own_flag, int n_ghost, int 
 cudaError_t launch_allreduce_gather_coef(double* scalars, int n, unsigned long long* const* peer_words, int n_slots,
                                          unsigned long long epoch, int mode, int has_gc, double k_vol, double v_target,
                                          int* error, cudaStream_t st);
-cudaError_t launch_halo_warmup(unsigned long long* words, double* scalars, int* error, cudaStream_t st);
+cudaError_t launch_halo_warmup(unsigned long long* words, double* scalars, int* error, unsigned int* push_ticket,
+                               cudaStream_t st);
 constexpr int kFlagWords = 1024;  // exported block (words): [0..3] epoch flags of the pull transport, [8..39] 2 x 16 scalar
                                   // slots of the pull all-reduce; push transport: [64 + 64 kind + src] arrival epochs of
                                   // the halo rows (kind 0 positions, 1 seeds) and [192 + src] of the scalars pushed by

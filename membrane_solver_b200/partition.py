@@ -118,6 +118,27 @@ def ghost_sources(local: LocalMesh) -> tuple[np.ndarray, np.ndarray]:
     return owners.astype(np.int32), rows.astype(np.int32)
 
 
+def push_targets(local: LocalMesh, sends: list[tuple[int, np.ndarray]], table) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """For every row of ``local`` that another rank lists as a ghost: (that rank, the row here, the row THERE), the
+    arguments of ``ms_ctx_set_push_targets``.  ``sends``: ``send_lists(local, ...)``; ``table[d]``: rank d's
+    ``(n_owned, recv_blocks)``.  A destination's ghosts are ordered by global id and grouped by source rank
+    (``LocalMesh.recv_blocks``), and ``send_lists`` gives this rank's rows for it in the same order."""
+    from . import _lib as L
+
+    slots, src, dst = [], [], []
+    for d, rows in sends:
+        n_owned_d, blocks_d = table[d]
+        first = [b[1] for b in blocks_d if b[0] == local.rank]
+        counts = [b[2] for b in blocks_d if b[0] == local.rank]
+        if len(first) != 1 or counts[0] != rows.size:
+            raise L.B200Error("send list and receive block of a neighbour disagree")
+        slots.append(np.full(rows.size, d, dtype=np.int32))
+        src.append(rows.astype(np.int32))
+        dst.append((n_owned_d + first[0] + np.arange(rows.size)).astype(np.int32))
+    cat = lambda xs: np.concatenate(xs) if xs else np.zeros(0, dtype=np.int32)  # noqa: E731
+    return cat(slots), cat(src), cat(dst)
+
+
 class HaloExchange:
     """Exchanges the ghost rows of per-vertex arrays between ranks (torch.distributed).
 
@@ -277,22 +298,7 @@ class PartitionedMesh:
         return int(flag.item()) == 1
 
     def _push_targets(self, table):
-        """For every row of this rank that another rank lists as a ghost: (that rank, the row here, the row THERE).
-        A destination's ghosts are ordered by global id and grouped by source rank (``LocalMesh.recv_blocks``), and
-        ``send_lists`` gives this rank's rows for it in the same order."""
-        local = self.local
-        slots, src, dst = [], [], []
-        for d, rows in self.halo.sends:
-            n_owned_d, blocks_d = table[d]
-            first = [b[1] for b in blocks_d if b[0] == local.rank]
-            counts = [b[2] for b in blocks_d if b[0] == local.rank]
-            if len(first) != 1 or counts[0] != rows.size:
-                raise self.L.B200Error("send list and receive block of a neighbour disagree")
-            slots.append(np.full(rows.size, d, dtype=np.int32))
-            src.append(rows.astype(np.int32))
-            dst.append((n_owned_d + first[0] + np.arange(rows.size)).astype(np.int32))
-        cat = lambda xs: np.concatenate(xs) if xs else np.zeros(0, dtype=np.int32)  # noqa: E731
-        return cat(slots), cat(src), cat(dst)
+        return push_targets(self.local, self.halo.sends, table)
 
     def exchange(self, which: int) -> None:
         if self.transport == "peer":
