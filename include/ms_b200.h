@@ -414,6 +414,28 @@ MS_API int ms_ctx_equiangulate_stats(const ms_ctx* ctx, double* ms4, int32_t* ro
                                      int32_t* n_sweeps_run);
 /* the current (nf,3) triangle rows in the caller's vertex numbering */
 MS_API int ms_ctx_get_triangles(const ms_ctx* ctx, int32_t* out);
+/* Refinement (the `r` command; geometry/refine.py::refine_triangles applied `levels` times, in the CALLER's vertex
+ * numbering): every edge a-b gets the midpoint 0.5 * (pos[a] + pos[b]), vertex nv + e for the e-th distinct edge key
+ * min*nv + max in ascending order; old vertices keep their ids; facet f = (v0, v1, v2) becomes rows f, nf + f,
+ * 2 nf + f and 3 nf + f: (v0, m01, m20), (v1, m12, m01), (v2, m20, m12), (m01, m12, m20).  A midpoint is fixed when
+ * both ends are, and a boundary vertex when both ends are and its edge has one facet.  Children take their parent's
+ * per-facet surface tension and body membership (child j of the result descends from facet j mod nf); uniform
+ * parameters stay.  The internal vertex order becomes the Morton order of the refined positions, so the context is
+ * what ms_ctx_set_vertex_order_hint(refined positions) + ms_ctx_set_topology + upload of the positions would make:
+ * the same packing and bitwise the same evaluations.  Everything derived from the connectivity is dropped as
+ * ms_ctx_set_topology drops it (leaflet selections, vertex normals, the conjugate-gradient history, a pending
+ * projection), and so are the trial positions, the direction and the per-vertex outputs of earlier evaluations.
+ * If the refined rows do not pack, or an allocation fails before the new mesh is complete, the call returns that
+ * error and the context keeps its previous mesh.  No atomics: repeated calls give identical results.  Synchronous.
+ * Refused (error, context unchanged): a partition context (n_owned < nv), levels < 0, no topology or no positions, a
+ * vertex index outside [0, nv), a refined mesh of more than 2^31 - 1 vertices or facets, and a context holding
+ * per-vertex kappa / c0 or a tilt field (their midpoint values are not defined here: refine on the host and set the
+ * topology again).  levels == 0 does nothing.  nv_out / nf_out (may be NULL) receive the new sizes. */
+MS_API int ms_ctx_refine(ms_ctx* ctx, int32_t levels, int32_t* nv_out, int32_t* nf_out);
+/* Times of the last ms_ctx_refine in ms: device time of the levels, the Morton order and the gathers (CUDA events),
+ * then host-clock times of the download of the rows and the order, the host packing, and the commit with the upload
+ * of the new packing. */
+MS_API int ms_ctx_refine_stats(const ms_ctx* ctx, double* ms4);
 /* per-vertex Polak-Ribiere direction (runtime/steppers/conjugate_gradient.py:63-119); restart != 0 or no
  * committed history: direction = -gradient.  ms_ctx_cg_commit stores gradient and direction of an
  * accepted step as the history of the next one. */

@@ -176,6 +176,8 @@ SIGNATURES = {
     "ms_ctx_equiangulate": (ctypes.c_int, [_V, _i32, ctypes.POINTER(_i64), ctypes.POINTER(_i32)]),
     "ms_ctx_equiangulate_stats": (ctypes.c_int, [_V, _D, _I, _i32, ctypes.POINTER(_i32)]),
     "ms_ctx_get_triangles": (ctypes.c_int, [_V, _I]),
+    "ms_ctx_refine": (ctypes.c_int, [_V, _i32, ctypes.POINTER(_i32), ctypes.POINTER(_i32)]),
+    "ms_ctx_refine_stats": (ctypes.c_int, [_V, _D]),
     "ms_ctx_cg_direction": (ctypes.c_int, [_V, _i32]),
     "ms_ctx_cg_commit": (ctypes.c_int, [_V]),
     "ms_ctx_line_search_stats": (ctypes.c_int, [_V, _D]),

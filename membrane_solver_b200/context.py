@@ -514,6 +514,24 @@ class DeviceMesh:
         return {"sweeps_run": int(n.value), "rounds": rounds[:int(n.value)].tolist(), "sweep_ms": float(ms[0]),
                 "d2h_ms": float(ms[1]), "pack_ms": float(ms[2]), "upload_ms": float(ms[3])}
 
+    def refine(self, levels: int = 1) -> np.ndarray:
+        """1 -> 4 midpoint refinement of the resident mesh, ``levels`` times (``ms_ctx_refine``), the device twin of
+        ``geometry.refine.refine_triangles`` with the context's fixed mask.  Updates ``nv`` / ``nf`` and returns the
+        composed ``parent`` (refined facet -> original facet).  The leaflet selections must be set again."""
+        nf0 = self.nf
+        nv, nf = ctypes.c_int32(0), ctypes.c_int32(0)
+        L.check(self._lib.ms_ctx_refine(self._h, int(levels), ctypes.byref(nv), ctypes.byref(nf)))
+        self.nv = self.n_owned = int(nv.value)
+        self.nf = int(nf.value)
+        return np.arange(self.nf, dtype=np.int64) % max(nf0, 1)
+
+    def refine_stats(self) -> dict:
+        """Times of the last ``refine`` in ms: device time, download of rows and order, host packing, commit and
+        upload."""
+        ms = np.zeros(4)
+        L.check(self._lib.ms_ctx_refine_stats(self._h, L.dptr(ms)))
+        return {"device_ms": float(ms[0]), "d2h_ms": float(ms[1]), "pack_ms": float(ms[2]), "upload_ms": float(ms[3])}
+
     def triangles(self) -> np.ndarray:
         """The current (nf,3) triangle rows in the caller's vertex numbering."""
         out = np.empty((self.nf, 3), dtype=np.int32)

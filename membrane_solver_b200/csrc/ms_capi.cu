@@ -55,6 +55,10 @@ struct DevBuf {
     p = nullptr;
     n = 0;
   }
+  void swap(DevBuf& o) {
+    std::swap(p, o.p);
+    std::swap(n, o.n);
+  }
   ~DevBuf() { release(); }
 };
 
@@ -141,6 +145,7 @@ struct ms_ctx {
   // the last ms_ctx_equiangulate: selection rounds of every sweep run; ms of sweeps, D2H of the rows, pack, upload
   std::vector<int32_t> eq_rounds;
   double eq_ms[4] = {0, 0, 0, 0};
+  double rf_ms[4] = {0, 0, 0, 0};  // the last ms_ctx_refine: device ms, D2H of rows and order, pack, commit + upload
   int64_t n_send_rows = 0;
   // leaflet tilt modules (ms_leaflet.cuh): per-leaflet selections, parameters and tilt fields
   struct Leaflet {
@@ -420,35 +425,12 @@ int download_rows(ms_ctx* c, const double* src_dev, double* host, int width) {
 
 // Morton (Z-curve) order of the hint positions: contiguous row ranges become compact surface
 // patches, which is what keeps the ring-facet recomputation of the patch kernels small.
+// ms_ctx_refine computes the same order on the device (ms_refine.cuh).
 void morton_permutation(const std::vector<double>& pos, int32_t nv, std::vector<int32_t>& perm) {
-  double lo[3] = {1e300, 1e300, 1e300}, hi[3] = {-1e300, -1e300, -1e300};
-  for (int32_t v = 0; v < nv; ++v)
-    for (int k = 0; k < 3; ++k) {
-      const double x = pos[3 * size_t(v) + k];
-      if (x < lo[k]) lo[k] = x;
-      if (x > hi[k]) hi[k] = x;
-    }
-  auto spread = [](uint64_t x) {
-    x &= 0x1FFFFFull;
-    x = (x | (x << 32)) & 0x1F00000000FFFFull;
-    x = (x | (x << 16)) & 0x1F0000FF0000FFull;
-    x = (x | (x << 8)) & 0x100F00F00F00F00Full;
-    x = (x | (x << 4)) & 0x10C30C30C30C30C3ull;
-    x = (x | (x << 2)) & 0x1249249249249249ull;
-    return x;
-  };
+  ms::MortonBox box = ms::morton_box_empty();
+  for (int32_t v = 0; v < nv; ++v) ms::morton_box_add(box, &pos[3 * size_t(v)]);
   std::vector<uint64_t> key(size_t(nv), 0);
-  for (int32_t v = 0; v < nv; ++v) {
-    uint64_t q[3];
-    for (int k = 0; k < 3; ++k) {
-      const double span = hi[k] - lo[k];
-      double t = span > 0 ? (pos[3 * size_t(v) + k] - lo[k]) / span * 2097151.0 : 0.0;
-      if (!(t >= 0)) t = 0;  // also catches NaN
-      if (t > 2097151.0) t = 2097151.0;
-      q[k] = uint64_t(t);
-    }
-    key[size_t(v)] = spread(q[0]) | (spread(q[1]) << 1) | (spread(q[2]) << 2);
-  }
+  for (int32_t v = 0; v < nv; ++v) key[size_t(v)] = ms::morton_key(box, &pos[3 * size_t(v)]);
   perm.resize(size_t(nv));
   std::iota(perm.begin(), perm.end(), 0);
   std::stable_sort(perm.begin(), perm.end(), [&](int32_t a, int32_t b) { return key[size_t(a)] < key[size_t(b)]; });
@@ -2365,6 +2347,181 @@ int ms_ctx_get_triangles(const ms_ctx* c, int32_t* out) {
     const int32_t x = c->h_tri[i];
     out[i] = (!c->perm.empty() && x >= 0 && x < c->nv) ? c->perm[size_t(x)] : x;
   }
+  return 0;
+}
+
+int ms_ctx_refine(ms_ctx* c, int32_t levels, int32_t* nv_out, int32_t* nf_out) {
+  if (int rc = check_ctx(c, true)) return rc;
+  if (c->n_owned != c->nv) return fail(-5, "refinement is not available on a partitioned context");
+  if (levels < 0) return fail(-1, "levels must be >= 0");
+  if (!c->has_positions) return fail(-4, "no positions have been set (MS_ARR_POSITIONS)");
+  for (int32_t x : c->h_tri)
+    if (x < 0 || x >= c->nv) return fail(-1, "a facet has a vertex index outside [0, nv)");
+  bool tilt_field = c->d_tilts.p != nullptr;
+  for (const auto& lf : c->leaflet) tilt_field = tilt_field || lf.tilts.p != nullptr;
+  if (c->has_kappa || c->has_c0 || tilt_field)
+    return fail(-6, "refinement does not set per-vertex kappa / c0 or tilts at the midpoints: refine on the host "
+                    "(geometry/refine.py refine_triangles), then ms_ctx_set_topology and upload them again");
+  // without facets every level only renumbers the vertices: one level gives the result of any number
+  const int32_t runs = c->nf == 0 ? std::min(levels, 1) : levels;
+  for (int64_t l = 0, nf = c->nf; l < runs; ++l, nf *= 4) {
+    if (3 * nf > INT32_MAX) return fail(-1, "refinement: more than 2^31 - 1 half-edges in a level");
+    if (4 * nf > INT32_MAX) return fail(-1, "refinement: more than 2^31 - 1 facets");
+  }
+  std::fill(c->rf_ms, c->rf_ms + 4, 0.0);
+  if (nv_out) *nv_out = c->nv;
+  if (nf_out) *nf_out = c->nf;
+  if (runs == 0) return 0;
+  if (int rc = ensure_tri(c)) return rc;
+  NvtxRange range("ms_b200 refine");
+  using clock = std::chrono::steady_clock;
+  auto ms_since = [](clock::time_point t0) { return std::chrono::duration<double, std::milli>(clock::now() - t0).count(); };
+  struct Events {  // the device time; the context's own events belong to ms_ctx_timer_*
+    cudaEvent_t e[2] = {nullptr, nullptr};
+    ~Events() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
+  } ev;
+  CU(cudaEventCreate(&ev.e[0]));
+  CU(cudaEventCreate(&ev.e[1]));
+  const int32_t nf0 = c->nf;
+  const bool fx = c->has_fixed, bd = c->has_boundary;
+  // Scratch, released on return; the context changes only after everything is built, allocated and packed.
+  // Levels run in the caller's numbering (the first reads the context's rows through key_id) into double buffers.
+  DevBuf<double> lpos[2];
+  DevBuf<uint8_t> lfixed[2], lbnd[2], temp;
+  DevBuf<int32_t> ltri[2], h_in, order, flag, scan, edge, head;
+  DevBuf<uint64_t> key_in, keys;
+  ms::EqMesh m{c->nv, c->nf, c->d_tri.p, c->d_pos.p, fx ? c->d_fixed.p : nullptr,
+               c->perm.empty() ? nullptr : c->d_perm.p, nullptr, nullptr};
+  const uint8_t* bnd = bd ? c->d_boundary.p : nullptr;
+  CU(cudaEventRecord(ev.e[0], c->stream));
+  for (int32_t l = 0; l < runs; ++l) {
+    const size_t nh = 3 * size_t(m.nf);
+    size_t tb = 0;
+    CU(ms::rf_temp_bytes(int64_t(nh), &tb));
+    for (int rc : {key_in.ensure(nh), keys.ensure(nh), h_in.ensure(nh), order.ensure(nh), flag.ensure(nh),
+                   scan.ensure(nh), edge.ensure(nh + 1), head.ensure(nh + 1), temp.ensure(tb + 1)})
+      if (rc) return rc;
+    CU(ms::launch_eq_sort_edges(m, key_in.p, h_in.p, keys.p, order.p, temp.p, tb, c->stream));
+    m.keys = keys.p;
+    m.order = order.p;
+    CU(ms::launch_rf_edges(m, flag.p, scan.p, edge.p, head.p, temp.p, tb, c->stream));
+    int32_t ne = 0;
+    if (nh) {
+      CU(cudaMemcpyAsync(&ne, scan.p + nh - 1, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+      CU(cudaStreamSynchronize(c->stream));
+    }
+    if (int64_t(m.nv) + ne > INT32_MAX) return fail(-1, "refinement: more than 2^31 - 1 vertices");
+    const size_t nv2 = size_t(m.nv) + size_t(ne), nf2 = 4 * size_t(m.nf);
+    const int i = l & 1;
+    for (int rc : {lpos[i].ensure(3 * nv2), fx ? lfixed[i].ensure(nv2) : 0, bd ? lbnd[i].ensure(nv2) : 0,
+                   ltri[i].ensure(3 * nf2)})
+      if (rc) return rc;
+    const ms::RfMesh r{m, bnd, head.p, edge.p, ne};
+    const ms::RfOut o{lpos[i].p, lfixed[i].p, lbnd[i].p, ltri[i].p};
+    CU(ms::launch_rf_build(r, o, c->stream));
+    m = ms::EqMesh{int32_t(nv2), int32_t(nf2), ltri[i].p, lpos[i].p, fx ? lfixed[i].p : nullptr, nullptr, nullptr, nullptr};
+    bnd = bd ? lbnd[i].p : nullptr;
+  }
+  // the internal vertex order of the refined mesh: the Morton order of its positions, as set_topology would choose it
+  const size_t nv2 = size_t(m.nv), nf2 = size_t(m.nf), n3 = 3 * nv2;
+  DevBuf<ms::MortonBox> boxes;
+  DevBuf<int32_t> perm2, inv2, tri_int, bnd32;
+  DevBuf<double> pos_int, grad, volgrad, seeds, stage;
+  DevBuf<uint8_t> fixed_int, bnd_int;
+  {
+    size_t tb = 0;
+    CU(ms::rf_temp_bytes(int64_t(nv2), &tb));
+    for (int rc : {boxes.ensure(1 + ms::kRfBoxBlocks), key_in.ensure(nv2), keys.ensure(nv2), h_in.ensure(nv2),
+                   perm2.ensure(nv2), inv2.ensure(nv2), temp.ensure(tb + 1), tri_int.ensure(3 * nf2 + 1),
+                   pos_int.ensure(n3), grad.ensure(n3), volgrad.ensure(n3), seeds.ensure(ms::kSeedStride * nv2),
+                   fx ? fixed_int.ensure(nv2) : 0, bd ? bnd_int.ensure(nv2) : 0, bd ? bnd32.ensure(nv2 + 1) : 0})
+      if (rc) return rc;
+    CU(ms::launch_rf_morton(m.pos, m.nv, boxes.p, key_in.p, h_in.p, keys.p, perm2.p, inv2.p, temp.p, tb, c->stream));
+  }
+  CU(ms::launch_gather_rows(m.pos, 3, perm2.p, int64_t(nv2), pos_int.p, c->stream));
+  CU(ms::launch_rf_renumber(m.tri, int64_t(3 * nf2), inv2.p, tri_int.p, c->stream));
+  if (fx) CU(ms::launch_rf_gather_flags(m.fixed, perm2.p, int64_t(nv2), fixed_int.p, nullptr, c->stream));
+  if (bd) {
+    CU(cudaMemsetAsync(bnd32.p, 0, (nv2 + 1) * sizeof(int32_t), c->stream));
+    CU(ms::launch_rf_gather_flags(bnd, perm2.p, int64_t(nv2), bnd_int.p, bnd32.p, c->stream));
+  }
+  if (n3) {
+    CU(cudaMemsetAsync(grad.p, 0, n3 * sizeof(double), c->stream));
+    CU(cudaMemsetAsync(volgrad.p, 0, n3 * sizeof(double), c->stream));
+  }
+  CU(cudaEventRecord(ev.e[1], c->stream));
+  CU(cudaEventSynchronize(ev.e[1]));
+  float dev_ms = 0.f;
+  CU(cudaEventElapsedTime(&dev_ms, ev.e[0], ev.e[1]));
+  c->rf_ms[0] = dev_ms;
+  // only the rows (for the packer and h_tri) and the order come back
+  auto t0 = clock::now();
+  std::vector<int32_t> rows(3 * nf2), new_perm(nv2);
+  if (nf2) CU(cudaMemcpy(rows.data(), tri_int.p, 3 * nf2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
+  if (nv2) CU(cudaMemcpy(new_perm.data(), perm2.p, nv2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
+  c->rf_ms[1] = ms_since(t0);
+  t0 = clock::now();
+  bool identity = true;
+  for (size_t v = 0; v < nv2 && identity; ++v) identity = new_perm[v] == int32_t(v);
+  if (identity) new_perm.clear();
+  if (!new_perm.empty())
+    if (int rc = stage.ensure(ms::kSeedStride * nv2)) return rc;
+  // children inherit their parent's per-facet values: child j of the last level descends from facet j mod nf0
+  std::vector<uint8_t> body;
+  std::vector<double> gamma;
+  if (!c->h_body.empty()) {
+    body.resize(nf2);
+    for (size_t j = 0; j < nf2; ++j) body[j] = c->h_body[j % size_t(nf0)];
+  }
+  if (!c->h_gamma.empty()) {
+    gamma.resize(nf2);
+    for (size_t j = 0; j < nf2; ++j) gamma[j] = c->h_gamma[j % size_t(nf0)];
+  }
+  ms::PackedMesh packed;
+  const int prc = pack_rows(c, m.nv, m.nv, m.nf, rows.data(), body.empty() ? nullptr : body.data(), packed);
+  c->rf_ms[2] = ms_since(t0);
+  if (prc) return fail(prc, "refinement: " + std::string(g_err) + "; the context keeps its previous mesh");
+  // commit
+  t0 = clock::now();
+  c->nv = c->n_owned = m.nv;
+  c->nf = m.nf;
+  c->h_tri.swap(rows);
+  c->perm.swap(new_perm);
+  c->h_body.swap(body);
+  c->h_gamma.swap(gamma);
+  c->d_pos.swap(pos_int);
+  c->d_grad.swap(grad);
+  c->d_volgrad.swap(volgrad);
+  c->d_seeds.swap(seeds);
+  c->d_tri.swap(tri_int);
+  if (!c->perm.empty()) {
+    c->d_perm.swap(perm2);
+    c->d_stage.swap(stage);
+  }
+  if (fx) c->d_fixed.swap(fixed_int);
+  if (bd) {
+    c->d_boundary.swap(bnd_int);
+    c->d_boundary32.swap(bnd32);
+  }
+  drop_connectivity_state(c);
+  c->tri_ready = true;  // d_tri holds the new rows
+  // per-vertex arrays of the previous size: produced again on demand
+  for (DevBuf<double>* b : {&c->d_trial, &c->d_dir, &c->d_tilt_grad, &c->d_tilt_sq, &c->d_kvecs, &c->d_avor, &c->d_aeff,
+                            &c->d_evert})
+    b->release();
+  for (auto& lf : c->leaflet) lf.tilt_grad.release();
+  if (int rc = upload_packing(c, std::move(packed), c->nv)) return rc;
+  if (c->has_gamma)
+    if (int rc = upload_slot_gamma(c)) return rc;
+  c->rf_ms[3] = ms_since(t0);
+  if (nv_out) *nv_out = c->nv;
+  if (nf_out) *nf_out = c->nf;
+  return 0;
+}
+
+int ms_ctx_refine_stats(const ms_ctx* c, double* ms4) {
+  if (!c || !ms4) return fail(-1, "null argument");
+  std::copy(c->rf_ms, c->rf_ms + 4, ms4);
   return 0;
 }
 

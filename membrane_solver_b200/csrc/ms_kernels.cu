@@ -23,7 +23,10 @@
 // Reference functions replaced: see the header of ms_math.cuh.
 #include "ms_kernels.cuh"
 
+#include <algorithm>
+
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <cub/iterator/counting_input_iterator.cuh>
 
@@ -1477,6 +1480,91 @@ __global__ void __launch_bounds__(256) k_eq_apply(const EqCands s, const uint8_t
   if (mask && (threadIdx.x & 31) == 0) atomicAdd(flips, __popc(mask));
 }
 
+// --- refinement (ms_refine.cuh): one thread per sorted half-edge, vertex row or facet ---
+__global__ void __launch_bounds__(256) k_rf_head_flags(const uint64_t* __restrict__ keys, int64_t n,
+                                                       int32_t* __restrict__ flag) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < n) flag[i] = rf_head(keys, i);
+}
+
+// scan = inclusive sum of the head flags: sorted position i belongs to edge scan[i] - 1
+__global__ void __launch_bounds__(256) k_rf_edges(const uint64_t* __restrict__ keys, const int32_t* __restrict__ order,
+                                                  const int32_t* __restrict__ scan, int64_t n, int32_t* __restrict__ edge,
+                                                  int32_t* __restrict__ head) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const int32_t e = scan[i] - 1;
+  edge[order[i]] = e;
+  if (rf_head(keys, i)) head[e] = int32_t(i);
+  if (i == n - 1) head[e + 1] = int32_t(n);
+}
+
+// rows [0, nv): the old vertices; rows [nv, nv + n_edges): the midpoints
+__global__ void __launch_bounds__(256) k_rf_vertices(const RfMesh r, const RfOut o) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < r.m.nv) rf_vertex(r, o, int32_t(i));
+  else if (i < int64_t(r.m.nv) + r.n_edges) rf_midpoint(r, o, int32_t(i - r.m.nv));
+}
+
+__global__ void __launch_bounds__(256) k_rf_children(const RfMesh r, const RfOut o) {
+  const int64_t f = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (f < r.m.nf) rf_children(r, o, int32_t(f));
+}
+
+// Bounding box of n positions: one box per block into boxes[1 + block], then boxes[0] from those (no atomics).
+__device__ void rf_block_box(MortonBox b, MortonBox* out) {
+  __shared__ MortonBox s[256];
+  s[threadIdx.x] = b;
+  __syncthreads();
+  for (int w = 128; w > 0; w >>= 1) {
+    if (int(threadIdx.x) < w) morton_box_merge(s[threadIdx.x], s[threadIdx.x + w]);
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *out = s[0];
+}
+
+__global__ void __launch_bounds__(256) k_rf_box_blocks(const double* __restrict__ pos, int64_t n, MortonBox* boxes) {
+  MortonBox b = morton_box_empty();
+  for (int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; v < n; v += int64_t(gridDim.x) * blockDim.x)
+    morton_box_add(b, pos + 3 * v);
+  rf_block_box(b, boxes + 1 + blockIdx.x);
+}
+
+__global__ void __launch_bounds__(256) k_rf_box_final(MortonBox* boxes, int n_blocks) {
+  MortonBox b = morton_box_empty();
+  for (int i = threadIdx.x; i < n_blocks; i += blockDim.x) morton_box_merge(b, boxes[1 + i]);
+  rf_block_box(b, boxes);
+}
+
+__global__ void __launch_bounds__(256) k_rf_morton_keys(const double* __restrict__ pos, int64_t n,
+                                                        const MortonBox* __restrict__ box, uint64_t* __restrict__ key,
+                                                        int32_t* __restrict__ id) {
+  const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (v >= n) return;
+  key[v] = morton_key(*box, pos + 3 * v);
+  id[v] = int32_t(v);
+}
+
+__global__ void __launch_bounds__(256) k_rf_invert(const int32_t* __restrict__ perm, int64_t n, int32_t* __restrict__ inv) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < n) inv[perm[i]] = int32_t(i);
+}
+
+__global__ void __launch_bounds__(256) k_rf_renumber(const int32_t* __restrict__ rows, int64_t n,
+                                                     const int32_t* __restrict__ inv, int32_t* __restrict__ out) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = inv[rows[i]];
+}
+
+__global__ void __launch_bounds__(256) k_rf_gather_flags(const uint8_t* __restrict__ src, const int32_t* __restrict__ perm,
+                                                         int64_t n, uint8_t* __restrict__ out, int32_t* __restrict__ out32) {
+  const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint8_t x = src[perm[i]];
+  out[i] = x;
+  if (out32) out32[i] = x ? 1 : 0;
+}
+
 // t -= (t.n) n  (runtime/projections/tilt.py:8-14)
 __global__ void __launch_bounds__(256) k_project_tangent(int64_t nv, const double* __restrict__ normals, double* t) {
   const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -2215,6 +2303,59 @@ cudaError_t launch_eq_round(const EqCands& s, const uint8_t* in, uint8_t* out, c
 
 cudaError_t launch_eq_apply(const EqCands& s, const uint8_t* state, int32_t* tri, int32_t* flips, cudaStream_t st) {
   if (s.n > 0) k_eq_apply<<<blocks_for(s.n, 256), 256, 0, st>>>(s, state, tri, flips);
+  return cudaGetLastError();
+}
+
+cudaError_t rf_temp_bytes(int64_t n, size_t* bytes) {
+  size_t a = 0, b = 0;
+  if (cudaError_t e = eq_temp_bytes(n, &a)) return e;
+  cudaError_t e = cub::DeviceScan::InclusiveSum(nullptr, b, (const int32_t*)nullptr, (int32_t*)nullptr, int(n));
+  *bytes = std::max(a, b);
+  return e;
+}
+
+cudaError_t launch_rf_edges(const EqMesh& m, int32_t* flag, int32_t* scan, int32_t* edge, int32_t* head, void* temp,
+                            size_t temp_bytes, cudaStream_t st) {
+  const int64_t n = 3 * int64_t(m.nf);
+  if (n == 0) return cudaSuccess;
+  k_rf_head_flags<<<blocks_for(n, 256), 256, 0, st>>>(m.keys, n, flag);
+  if (cudaError_t e = cudaGetLastError()) return e;
+  if (cudaError_t e = cub::DeviceScan::InclusiveSum(temp, temp_bytes, flag, scan, int(n), st)) return e;
+  k_rf_edges<<<blocks_for(n, 256), 256, 0, st>>>(m.keys, m.order, scan, n, edge, head);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rf_build(const RfMesh& r, const RfOut& o, cudaStream_t st) {
+  const int64_t nv_out = int64_t(r.m.nv) + r.n_edges;
+  if (nv_out > 0) k_rf_vertices<<<blocks_for(nv_out, 256), 256, 0, st>>>(r, o);
+  if (cudaError_t e = cudaGetLastError()) return e;
+  if (r.m.nf > 0) k_rf_children<<<blocks_for(r.m.nf, 256), 256, 0, st>>>(r, o);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rf_morton(const double* pos, int32_t n, MortonBox* boxes, uint64_t* key_in, int32_t* id_in,
+                             uint64_t* key_out, int32_t* perm, int32_t* inv, void* temp, size_t temp_bytes,
+                             cudaStream_t st) {
+  if (n <= 0) return cudaSuccess;
+  const int nb = std::min(kRfBoxBlocks, blocks_for(n, 256));
+  k_rf_box_blocks<<<nb, 256, 0, st>>>(pos, n, boxes);
+  k_rf_box_final<<<1, 256, 0, st>>>(boxes, nb);
+  k_rf_morton_keys<<<blocks_for(n, 256), 256, 0, st>>>(pos, n, boxes, key_in, id_in);
+  if (cudaError_t e = cudaGetLastError()) return e;
+  // 3 x 21 key bits; the radix sort is stable, so equal keys keep ascending ids, as std::stable_sort orders them
+  if (cudaError_t e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_in, key_out, id_in, perm, n, 0, 63, st)) return e;
+  k_rf_invert<<<blocks_for(n, 256), 256, 0, st>>>(perm, n, inv);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rf_renumber(const int32_t* rows, int64_t n, const int32_t* inv, int32_t* out, cudaStream_t st) {
+  if (n > 0) k_rf_renumber<<<blocks_for(n, 256), 256, 0, st>>>(rows, n, inv, out);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_rf_gather_flags(const uint8_t* src, const int32_t* perm, int64_t n, uint8_t* out, int32_t* out32,
+                                   cudaStream_t st) {
+  if (n > 0) k_rf_gather_flags<<<blocks_for(n, 256), 256, 0, st>>>(src, perm, n, out, out32);
   return cudaGetLastError();
 }
 

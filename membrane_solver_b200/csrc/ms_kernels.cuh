@@ -11,6 +11,7 @@
 #include "ms_math.cuh"
 #include "ms_pack.h"
 #include "ms_equiangulate.cuh"
+#include "ms_refine.cuh"
 #include "ms_vertex_average.cuh"
 
 namespace ms {
@@ -338,5 +339,26 @@ cudaError_t launch_eq_round(const EqCands& s, const uint8_t* in, uint8_t* out, c
                             int32_t* undecided, cudaStream_t st);
 // rewrites the rows of the selected candidates; adds their number to *flips
 cudaError_t launch_eq_apply(const EqCands& s, const uint8_t* state, int32_t* tri, int32_t* flips, cudaStream_t st);
+
+
+// --- refinement (the `r` command), one level in three steps, then the Morton order (ms_refine.cuh) ---
+constexpr int kRfBoxBlocks = 296;  // blocks of the bounding-box reduction; boxes holds 1 + kRfBoxBlocks entries
+// scratch of the key sorts and the scan for up to n items (half-edges of a level, or vertex rows)
+cudaError_t rf_temp_bytes(int64_t n, size_t* bytes);
+// from the sorted keys (m.keys / m.order, launch_eq_sort_edges): edge[h] = edge of half-edge h, head[e] = sorted
+// position where the run of edge e starts and head[n_edges] = 3 nf; scan[3 nf - 1] = n_edges (device)
+cudaError_t launch_rf_edges(const EqMesh& m, int32_t* flag, int32_t* scan, int32_t* edge, int32_t* head, void* temp,
+                            size_t temp_bytes, cudaStream_t st);
+// the refined vertex rows, flags and facet rows of one level into o
+cudaError_t launch_rf_build(const RfMesh& r, const RfOut& o, cudaStream_t st);
+// perm (new -> old) = morton_permutation of the n positions, before dropping an identity; inv = its inverse
+cudaError_t launch_rf_morton(const double* pos, int32_t n, MortonBox* boxes, uint64_t* key_in, int32_t* id_in,
+                             uint64_t* key_out, int32_t* perm, int32_t* inv, void* temp, size_t temp_bytes,
+                             cudaStream_t st);
+// out[i] = inv[rows[i]]
+cudaError_t launch_rf_renumber(const int32_t* rows, int64_t n, const int32_t* inv, int32_t* out, cudaStream_t st);
+// out[i] = src[perm[i]], and out32[i] = out[i] != 0 when out32 is set
+cudaError_t launch_rf_gather_flags(const uint8_t* src, const int32_t* perm, int64_t n, uint8_t* out, int32_t* out32,
+                                   cudaStream_t st);
 
 }  // namespace ms

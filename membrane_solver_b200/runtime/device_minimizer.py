@@ -121,6 +121,16 @@ class DeviceMinimizer:
         self._cg_iter = 0
         return flips
 
+    # -- the r command (commands/mesh_ops.py) ----------------------------------------------------------
+    def refine(self, n: int = 1):
+        """``n`` levels of midpoint refinement on the device (``DeviceMesh.refine``).  The reference projects no
+        volume after ``r`` (the midpoints of a closed surface lie inside it), so neither does this; step size and
+        ``v_target`` stay, the conjugate-gradient history is discarded.  Returns the composed ``parent``."""
+        parent = self.dm.refine(int(n))
+        self._cg_have_history = False
+        self._cg_iter = 0
+        return parent
+
     # -- one line search (line_search.py:267-430) --------------------------------------------------
     def _line_search(self, step_size: float):
         dm = self.dm

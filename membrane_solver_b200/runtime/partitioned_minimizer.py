@@ -15,7 +15,8 @@ energy/volume allreduce for line search".  ``DeviceMinimizer`` (``runtime/device
   ``<g,d>`` and ``<g,g>`` over OWNED rows (sum);
 * the normal-flip guard (``runtime/topology.py:13-48``) first brings the ghost rows of the trial positions, then
   every rank checks its facets and the verdicts are AND-ed.
-* vertex averaging (the ``V`` command) and equiangulation (``u``) are refused: they run on a single GPU only.
+* vertex averaging (the ``V`` command), equiangulation (``u``) and refinement (``r``) are refused: they run on a
+  single GPU only.
 
 All ranks call the same sequence (the loop control depends only on reduced values), which is what the peer-memory
 transport's lock-step flags need.
@@ -61,6 +62,9 @@ class PartitionedDevice:
 
     def equiangulate(self, max_iterations: int = 100) -> int:
         raise L.B200Error("equiangulation (u) runs on a single GPU only: re-assemble the mesh on one device")
+
+    def refine(self, levels: int = 1):
+        raise L.B200Error("refinement (r) runs on a single GPU only: re-assemble the mesh on one device")
 
     def make_trial(self, alpha: float) -> None:
         self.dm.make_trial(alpha)
