@@ -160,6 +160,11 @@ MS_API int ms_ctx_pack_send(ms_ctx* ctx, int which, void* out_device);
  * independently of the topology versions. */
 MS_API int ms_ctx_set_fixed_mask(ms_ctx* ctx, const uint8_t* fixed_mask);
 MS_API int ms_ctx_pack_info(const ms_ctx* ctx, ms_pack_info* info);
+/* Copy of the current packing (built on the device, byte for byte what the host packer ms::pack_patches makes of the
+ * internal-order rows), sized by ms_ctx_pack_info: n_patches headers of 32 bytes, n_halo halo vertex rows, n_slots
+ * facet records of 8 bytes (a, b, c, flags as uint16) and n_slots facet rows (-1 for an empty slot).  Any pointer may
+ * be NULL.  Synchronous. */
+MS_API int ms_ctx_get_packing(const ms_ctx* ctx, void* headers, int32_t* halo_ids, void* recs, int32_t* slot_facet);
 /* patch p owns vertex rows [v_lo[p], v_lo[p+1]); v_lo has n_patches+1 entries */
 MS_API int ms_ctx_patch_ranges(const ms_ctx* ctx, int32_t* v_lo);
 /* halo vertex rows referenced by patches [patch_begin, patch_begin+patch_count) that lie
@@ -408,8 +413,8 @@ MS_API int ms_ctx_vertex_average(ms_ctx* ctx, const int32_t* group, int32_t roun
 MS_API int ms_ctx_equiangulate(ms_ctx* ctx, int32_t max_iterations, int64_t* n_flips, int32_t* n_sweeps);
 /* Diagnostics of the last ms_ctx_equiangulate: *n_sweeps_run = sweeps run (including a last one without flips);
  * rounds[i] = selection rounds of sweep i (0 for a sweep without candidates), at most `capacity` entries;
- * ms4 = device time of all sweeps (CUDA events), then host-clock times of the row download, the host packing and the
- * upload of the new packing.  rounds / ms4 may be NULL. */
+ * ms4 = device time of all sweeps (CUDA events), the host-clock time of the row download, the device packing of the
+ * new rows (CUDA events) and the host-clock time of the commit of the new packing.  rounds / ms4 may be NULL. */
 MS_API int ms_ctx_equiangulate_stats(const ms_ctx* ctx, double* ms4, int32_t* rounds, int32_t capacity,
                                      int32_t* n_sweeps_run);
 /* the current (nf,3) triangle rows in the caller's vertex numbering */
@@ -433,8 +438,8 @@ MS_API int ms_ctx_get_triangles(const ms_ctx* ctx, int32_t* out);
  * topology again).  levels == 0 does nothing.  nv_out / nf_out (may be NULL) receive the new sizes. */
 MS_API int ms_ctx_refine(ms_ctx* ctx, int32_t levels, int32_t* nv_out, int32_t* nf_out);
 /* Times of the last ms_ctx_refine in ms: device time of the levels, the Morton order and the gathers (CUDA events),
- * then host-clock times of the download of the rows and the order, the host packing, and the commit with the upload
- * of the new packing. */
+ * the host-clock time of the download of the rows and the order, the device packing of the refined rows (CUDA
+ * events), and the host-clock time of the per-facet inheritance and the commit of the new mesh. */
 MS_API int ms_ctx_refine_stats(const ms_ctx* ctx, double* ms4);
 /* per-vertex Polak-Ribiere direction (runtime/steppers/conjugate_gradient.py:63-119); restart != 0 or no
  * committed history: direction = -gradient.  ms_ctx_cg_commit stores gradient and direction of an

@@ -116,6 +116,7 @@ SIGNATURES = {
     "ms_ctx_pack_send": (ctypes.c_int, [_V, ctypes.c_int, _V]),
     "ms_ctx_set_fixed_mask": (ctypes.c_int, [_V, ctypes.POINTER(ctypes.c_uint8)]),
     "ms_ctx_pack_info": (ctypes.c_int, [_V, ctypes.POINTER(PackInfo)]),
+    "ms_ctx_get_packing": (ctypes.c_int, [_V, _V, _I, _V, _I]),
     "ms_ctx_patch_ranges": (ctypes.c_int, [_V, _I]),
     "ms_ctx_halo_rows": (ctypes.c_int, [_V, _i32, _i32, _i32, _i32, _I, ctypes.POINTER(_i64)]),
     "ms_ctx_set_surface_tension": (ctypes.c_int, [_V, _D, _f64]),

@@ -146,6 +146,20 @@ class DeviceMesh:
         L.check(self._lib.ms_ctx_pack_info(self._h, ctypes.byref(info)))
         return {name: int(getattr(info, name)) for name, _ in L.PackInfo._fields_}
 
+    def packing(self) -> dict:
+        """The current packing as NumPy arrays (``ms_ctx_get_packing``): ``headers`` ((n_patches, 32) uint8, the
+        32-byte patch headers), ``halo_ids`` (int32), ``recs`` ((n_slots, 4) uint16: a, b, c, flags) and ``slot_facet``
+        (int32, -1 for an empty slot).  It is what the host packer makes of the internal-order rows."""
+        info = self.pack_info()
+        out = {"headers": np.zeros((info["n_patches"], 32), dtype=np.uint8),
+               "halo_ids": np.zeros(info["n_halo"], dtype=np.int32),
+               "recs": np.zeros((info["n_slots"], 4), dtype=np.uint16),
+               "slot_facet": np.zeros(info["n_slots"], dtype=np.int32)}
+        L.check(self._lib.ms_ctx_get_packing(self._h, out["headers"].ctypes.data_as(ctypes.c_void_p),
+                                             L.iptr(out["halo_ids"]), out["recs"].ctypes.data_as(ctypes.c_void_p),
+                                             L.iptr(out["slot_facet"])))
+        return out
+
     def patch_ranges(self) -> np.ndarray:
         n = self.pack_info()["n_patches"]
         out = np.empty(n + 1, dtype=np.int32)
@@ -505,7 +519,7 @@ class DeviceMesh:
 
     def equiangulate_stats(self) -> dict:
         """Sweeps run by the last ``equiangulate``, the selection rounds of each, and its times in ms: device time of
-        the sweeps, row download, host packing, upload."""
+        the sweeps, row download, device packing of the new rows (CUDA events), commit of the new packing."""
         n = ctypes.c_int32(0)
         L.check(self._lib.ms_ctx_equiangulate_stats(self._h, None, None, 0, ctypes.byref(n)))
         ms = np.zeros(4)
@@ -526,8 +540,8 @@ class DeviceMesh:
         return np.arange(self.nf, dtype=np.int64) % max(nf0, 1)
 
     def refine_stats(self) -> dict:
-        """Times of the last ``refine`` in ms: device time, download of rows and order, host packing, commit and
-        upload."""
+        """Times of the last ``refine`` in ms: device time, download of rows and order, device packing of the refined
+        rows (CUDA events), per-facet inheritance and commit."""
         ms = np.zeros(4)
         L.check(self._lib.ms_ctx_refine_stats(self._h, L.dptr(ms)))
         return {"device_ms": float(ms[0]), "d2h_ms": float(ms[1]), "pack_ms": float(ms[2]), "upload_ms": float(ms[3])}

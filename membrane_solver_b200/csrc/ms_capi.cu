@@ -84,12 +84,14 @@ struct ms_ctx {
   int32_t nv = 0, nf = 0;
   int32_t n_owned = 0;  // vertex rows owned by this context's patches (== nv unless partitioned)
   ms::PackParams pack_params;
-  ms::PackedMesh packed;  // recs / slot_facet kept on the host for gamma repacking
+  ms::PackedMesh packed;  // headers, halo ids and statistics; the records and slot facets live on the device only
+  int64_t n_slots = 0;    // record slots of the packing (d_recs, d_slot_facet)
   std::vector<int32_t> v_lo;
 
   DevBuf<ms::PatchHeader> d_patches;
   DevBuf<int32_t> d_halo;
   DevBuf<ms::FacetRec> d_recs;
+  DevBuf<int32_t> d_slot_facet;  // facet row of each record slot, -1 for an empty one
   DevBuf<double> d_slot_gamma;
   DevBuf<uint8_t> d_boundary, d_fixed;
   DevBuf<int32_t> d_boundary32;  // boundary flags as int32: staged into shared memory with 4-byte cp.async
@@ -142,10 +144,10 @@ struct ms_ctx {
   // host copies that outlive a re-pack of flipped rows (ms_ctx_equiangulate): per-facet gamma and body membership
   std::vector<double> h_gamma;
   std::vector<uint8_t> h_body;
-  // the last ms_ctx_equiangulate: selection rounds of every sweep run; ms of sweeps, D2H of the rows, pack, upload
+  // the last ms_ctx_equiangulate: selection rounds of every sweep run; ms of sweeps, D2H of the rows, device pack, commit
   std::vector<int32_t> eq_rounds;
   double eq_ms[4] = {0, 0, 0, 0};
-  double rf_ms[4] = {0, 0, 0, 0};  // the last ms_ctx_refine: device ms, D2H of rows and order, pack, commit + upload
+  double rf_ms[4] = {0, 0, 0, 0};  // the last ms_ctx_refine: device ms, D2H of rows and order, device pack, commit
   int64_t n_send_rows = 0;
   // leaflet tilt modules (ms_leaflet.cuh): per-leaflet selections, parameters and tilt fields
   struct Leaflet {
@@ -371,16 +373,27 @@ int ensure_tri(ms_ctx* c) {
   return 0;
 }
 
-// triangle rows and the vertex -> corner CSR (corner id 3 f + k, facet-major) on the device, once per topology
+// The vertex -> corner CSR (corner id 3 f + k, facet-major; ms::build_corner_csr) of device rows, by one stable sort of
+// the corner keys: ptr gets nv + 1 offsets, idx 3 nf + 1 entries.
+int corner_csr_device(ms_ctx* c, int32_t nv, int32_t nf, const int32_t* tri, DevBuf<int32_t>& ptr, DevBuf<int32_t>& idx) {
+  const size_t n = 3 * size_t(nf);
+  size_t tb = 0;
+  CU(ms::pk_temp_bytes(int64_t(n), &tb));
+  DevBuf<int32_t> key_in, id_in, key_out;
+  DevBuf<uint8_t> temp;
+  for (int rc : {key_in.ensure(n + 1), id_in.ensure(n + 1), key_out.ensure(n + 1), temp.ensure(tb + 1), ptr.ensure(size_t(nv) + 1),
+                 idx.ensure(n + 1)})
+    if (rc) return rc;
+  CU(ms::launch_pk_corner_csr(tri, nv, nf, key_in.p, id_in.p, key_out.p, idx.p, ptr.p, temp.p, tb, c->stream));
+  CU(cudaStreamSynchronize(c->stream));  // the scratch is released on return
+  return 0;
+}
+
+// triangle rows and the vertex -> corner CSR on the device, once per topology (the packing leaves its CSR behind)
 int ensure_corner_csr(ms_ctx* c) {
   if (c->csr_ready) return 0;
-  std::vector<int32_t> ptr, idx;
-  ms::build_corner_csr(c->nv, c->nf, c->h_tri.data(), ptr, idx);
   if (int rc = ensure_tri(c)) return rc;
-  if (int rc = c->d_csr_ptr.ensure(ptr.size())) return rc;
-  if (int rc = c->d_csr_idx.ensure(idx.size() + 1)) return rc;
-  CU(cudaMemcpy(c->d_csr_ptr.p, ptr.data(), ptr.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-  if (!idx.empty()) CU(cudaMemcpy(c->d_csr_idx.p, idx.data(), idx.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  if (int rc = corner_csr_device(c, c->nv, c->nf, c->d_tri.p, c->d_csr_ptr, c->d_csr_idx)) return rc;
   c->csr_ready = true;
   return 0;
 }
@@ -439,30 +452,138 @@ void morton_permutation(const std::vector<double>& pos, int32_t nv, std::vector<
   if (identity) perm.clear();
 }
 
-// Packs triangle rows (internal vertex order) into `out` with the context's pack parameters.  A vertex of valence V
-// needs V rounds, i.e. V * threads record slots, and a patch holds at most kPatchSlotCap of them: meshes with
+// A packing built on the device (ms_pack_device.cuh): headers with the closing sentinel, halo ids, records and slot
+// facets on the device; headers, halo ids and statistics also in `host` (its recs / slot_facet stay empty); and the
+// corner CSR of the rows it packed.
+struct DevPacking {
+  ms::PackedMesh host;
+  int64_t n_slots = 0;
+  DevBuf<ms::PatchHeader> patches;
+  DevBuf<int32_t> halo, slot_facet, csr_ptr, csr_idx;
+  DevBuf<ms::FacetRec> recs;
+};
+
+// ms::pack_patches on the device, with its return codes (0, -1, -2, -3); other codes are CUDA or internal failures.
+// tri and body (nf bytes or nullptr) are device arrays.  Changes nothing in the context.
+int pack_device(ms_ctx* c, int32_t nv, int32_t n_owned, int32_t nf, const int32_t* tri, const uint8_t* body,
+                const ms::PackParams& prm, DevPacking& out) {
+  if (n_owned < 0 || n_owned > nv) n_owned = nv;
+  if (nv < 0 || nf < 0 || (nf > 0 && !tri) || prm.threads <= 0 || prm.max_owned <= 0 || prm.max_local <= 0 ||
+      prm.max_local > 65535 || prm.max_slots < prm.threads || prm.fill_pct < 10 || prm.fill_pct > 100)
+    return -1;
+  cudaStream_t st = c->stream;
+  ms::PackedMesh& pk = out.host;
+  pk = ms::PackedMesh();
+  pk.nv = nv;
+  pk.nf = nf;
+  pk.params = prm;
+  pk.n_owned_vertices = n_owned;
+  if (int rc = corner_csr_device(c, nv, nf, tri, out.csr_ptr, out.csr_idx)) return rc;
+  const int64_t chunk = ms::pk_chunk_rows(prm), n_chunks = (int64_t(n_owned) + chunk - 1) / chunk;
+  std::vector<unsigned long long> hb(3 * size_t(n_chunks) + 1);
+  {
+    DevBuf<unsigned long long> bounds;
+    if (int rc = bounds.ensure(hb.size())) return rc;
+    CU(ms::launch_pk_bounds(prm, out.csr_ptr.p, n_owned, tri, nv, nf, bounds.p, n_chunks, bounds.p + 3 * n_chunks, st));
+    CU(cudaMemcpyAsync(hb.data(), bounds.p, hb.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+  }
+  pk.n_valid = int64_t(hb[3 * size_t(n_chunks)]);
+  const std::vector<int64_t> b64(hb.begin(), hb.end() - 1);
+  std::vector<ms::PkChunk> ck(static_cast<size_t>(n_chunks));
+  const ms::PkPlan plan = ms::pk_plan(prm, n_owned, b64.data(), ck.data(), n_chunks);
+  // scratch and staging, released on return
+  DevBuf<int64_t> scratch, s_slot, bases;
+  DevBuf<ms::PatchHeader> s_hdr;
+  DevBuf<int32_t> s_halo, s_fac;
+  DevBuf<ms::FacetRec> s_rec;
+  DevBuf<ms::PkChunk> d_ck;
+  DevBuf<unsigned long long> hx;
+  for (int rc : {scratch.ensure(size_t(plan.scratch_words / 2) + 1), s_slot.ensure(size_t(plan.ent) + 1),
+                 bases.ensure(3 * size_t(n_chunks) + 1), s_hdr.ensure(size_t(plan.hdr) + 1),
+                 s_halo.ensure(size_t(plan.halo) + 1), s_fac.ensure(size_t(plan.ent) + 1), s_rec.ensure(size_t(plan.ent) + 1),
+                 d_ck.ensure(size_t(n_chunks) + 1), hx.ensure(2)})
+    if (rc) return rc;
+  const ms::PkStage stage{s_hdr.p, s_halo.p, s_rec.p, s_fac.p, s_slot.p};
+  const ms::PkMesh m{nv, nf, n_owned, tri, body, out.csr_ptr.p, out.csr_idx.p, prm};
+  if (n_chunks) CU(cudaMemcpyAsync(d_ck.p, ck.data(), ck.size() * sizeof(ms::PkChunk), cudaMemcpyHostToDevice, st));
+  CU(ms::launch_pk_chunks(m, reinterpret_cast<int32_t*>(scratch.p), stage, d_ck.p, n_chunks, st));
+  if (n_chunks) CU(cudaMemcpyAsync(ck.data(), d_ck.p, ck.size() * sizeof(ms::PkChunk), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  for (const ms::PkChunk& k : ck) {  // the first failing chunk decides, as on the host
+    if (k.rc == ms::kPkInternal) return fail(-9, "device packer: a scratch bound did not hold");
+    if (k.rc) return k.rc;
+  }
+  std::vector<int64_t> hbase(3 * size_t(n_chunks));
+  int64_t np = 0, nh = 0, ns = 0;
+  for (size_t i = 0; i < ck.size(); ++i) {
+    const ms::PkChunk& k = ck[i];
+    hbase[3 * i] = np;
+    hbase[3 * i + 1] = nh;
+    hbase[3 * i + 2] = ns;
+    np += k.n_patches;
+    nh += k.n_halo;
+    ns += k.n_slots;
+    pk.max_owned = std::max(pk.max_owned, k.max_owned);
+    pk.max_local = std::max(pk.max_local, k.max_local);
+    pk.max_rounds = std::max(pk.max_rounds, k.max_rounds);
+    pk.max_slots = std::max(pk.max_slots, k.max_slots);
+    pk.n_round_slots += k.n_round_slots;
+    pk.n_listed += k.n_listed;
+    pk.n_lane_conflicts += k.n_lane_conflicts;
+  }
+  if (nh > INT32_MAX) return fail(-8, "the packing has more than 2^31 - 1 halo entries");
+  for (int rc : {out.patches.ensure(size_t(np) + 1), out.halo.ensure(size_t(nh) + 1), out.recs.ensure(size_t(ns) + 1),
+                 out.slot_facet.ensure(size_t(ns) + 1)})
+    if (rc) return rc;
+  if (n_chunks) CU(cudaMemcpyAsync(bases.p, hbase.data(), hbase.size() * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+  CU(ms::launch_pk_concat(stage, d_ck.p, bases.p, n_chunks, out.patches.p, out.halo.p, out.recs.p, out.slot_facet.p, ns, st));
+  ms::PatchHeader end;  // sentinel header: closes the record range of the last patch
+  std::memset(&end, 0, sizeof(end));
+  end.v_lo = n_owned;
+  end.halo_off = int32_t(nh);
+  end.slot_off = ns;
+  CU(cudaMemcpyAsync(out.patches.p + np, &end, sizeof(end), cudaMemcpyHostToDevice, st));
+  CU(ms::launch_pk_hw_excess(out.patches.p, int32_t(np), out.recs.p, prm.threads, hx.p, st));
+  unsigned long long hw[2] = {0, 0};
+  CU(cudaMemcpyAsync(hw, hx.p, sizeof(hw), cudaMemcpyDeviceToHost, st));
+  pk.patches.resize(size_t(np));
+  pk.halo_ids.resize(size_t(nh));
+  if (np) CU(cudaMemcpyAsync(pk.patches.data(), out.patches.p, size_t(np) * sizeof(ms::PatchHeader), cudaMemcpyDeviceToHost, st));
+  if (nh) CU(cudaMemcpyAsync(pk.halo_ids.data(), out.halo.p, size_t(nh) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  pk.n_hw_groups = int64_t(hw[0]);
+  pk.n_hw_excess = int64_t(hw[1]);
+  out.n_slots = ns;
+  return 0;
+}
+
+// Packs device triangle rows (internal vertex order) into `out` with the context's pack parameters.  A vertex of
+// valence V needs V rounds, i.e. V * threads record slots, and a patch holds at most kPatchSlotCap of them: meshes with
 // high-valence vertices (a disk centre, a cone apex) are packed with narrower rounds (96 -> 64 -> 32 lanes: valence
-// up to 16 / 24 / 48).  Changes nothing in the context.
-int pack_rows(const ms_ctx* c, int32_t nv, int32_t n_owned, int32_t nf, const int32_t* tri, const uint8_t* body_mask,
-              ms::PackedMesh& out) {
+// up to 16 / 24 / 48).  body: nf bytes on the device or nullptr.  Changes nothing in the context.
+int pack_rows(ms_ctx* c, int32_t nv, int32_t n_owned, int32_t nf, const int32_t* tri, const uint8_t* body,
+              DevPacking& out) {
   ms::PackParams used_params = c->pack_params;
-  int prc = ms::pack_patches(nv, nf, tri, body_mask, used_params, out, n_owned);
+  int prc = pack_device(c, nv, n_owned, nf, tri, body, used_params, out);
   while (prc == -3 && used_params.threads > 32) {
     used_params.threads = used_params.threads > 64 ? 64 : 32;
-    prc = ms::pack_patches(nv, nf, tri, body_mask, used_params, out, n_owned);
+    prc = pack_device(c, nv, n_owned, nf, tri, body, used_params, out);
   }
   if (prc == -2) return fail(-8, "a vertex neighbourhood exceeds max_local; raise it with ms_ctx_set_pack_params");
   if (prc == -3) return fail(-8, "a vertex has more than 48 incident facets: its rounds do not fit a patch");
-  if (prc) return fail(-1, "pack_patches failed");
-  if (out.max_owned > ms::kPatchOwnedCap || out.max_local > ms::kPatchLocalCap || out.max_slots > ms::kPatchSlotCap)
+  if (prc == -1) return fail(-1, "pack_patches failed");
+  if (prc) return prc;
+  const ms::PackedMesh& pk = out.host;
+  if (pk.max_owned > ms::kPatchOwnedCap || pk.max_local > ms::kPatchLocalCap || pk.max_slots > ms::kPatchSlotCap)
     return fail(-8, "a patch exceeds the compiled shared-memory capacities");
   return 0;
 }
 
-// Makes `packed` the context's packing and uploads it: patch ranges, interior-then-boundary patch order, headers,
-// halo ids and facet records.
-int upload_packing(ms_ctx* c, ms::PackedMesh&& packed, int32_t n_owned) {
-  c->packed = std::move(packed);
+// Makes `packed` the context's packing: patch ranges, interior-then-boundary patch order, and the device arrays
+// (headers, halo ids, records, slot facets, corner CSR) it built.  The caller has dropped the connectivity state.
+int upload_packing(ms_ctx* c, DevPacking&& packed, int32_t n_owned) {
+  c->packed = std::move(packed.host);
   const ms::PackedMesh& pk = c->packed;
   const size_t np = pk.patches.size();
   c->v_lo.resize(np + 1);
@@ -482,45 +603,35 @@ int upload_packing(ms_ctx* c, ms::PackedMesh&& packed, int32_t n_owned) {
     if (int rc = c->d_patch_order.ensure(order.size() + 1)) return rc;
     if (!order.empty()) CU(cudaMemcpy(c->d_patch_order.p, order.data(), order.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
   }
-  if (int rc = c->d_patches.ensure(np + 1)) return rc;
-  if (int rc = c->d_halo.ensure(pk.halo_ids.size())) return rc;
-  if (int rc = c->d_recs.ensure(pk.recs.size())) return rc;
-  {  // sentinel header: closes the record range of the last patch
-    std::vector<ms::PatchHeader> hdr(pk.patches);
-    ms::PatchHeader end;
-    std::memset(&end, 0, sizeof(end));
-    end.v_lo = n_owned;
-    end.halo_off = int32_t(pk.halo_ids.size());
-    end.slot_off = int64_t(pk.recs.size());
-    hdr.push_back(end);
-    CU(cudaMemcpy(c->d_patches.p, hdr.data(), hdr.size() * sizeof(ms::PatchHeader), cudaMemcpyHostToDevice));
-  }
-  if (!pk.halo_ids.empty())
-    CU(cudaMemcpy(c->d_halo.p, pk.halo_ids.data(), pk.halo_ids.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+  c->n_slots = packed.n_slots;
+  c->d_patches.swap(packed.patches);
+  c->d_halo.swap(packed.halo);
+  c->d_recs.swap(packed.recs);
+  c->d_slot_facet.swap(packed.slot_facet);
+  c->d_csr_ptr.swap(packed.csr_ptr);
+  c->d_csr_idx.swap(packed.csr_idx);
+  c->csr_ready = true;
 #ifdef MS_SELF_CHECK
   if (std::getenv("MS_SELF_CHECK_INJECT")) {
     // negative control of the self-check: slot 1 of every patch's first round repeats slot 0, so two lanes of one
     // warp read-modify-write the same owned rows at once -- the row locks must report it
-    ms::PackedMesh& bad = c->packed;
-    for (const ms::PatchHeader& h : bad.patches)
-      if (h.n_rounds > 0 && (bad.recs[size_t(h.slot_off)].flags & ms::REC_VALID))
-        bad.recs[size_t(h.slot_off) + 1] = bad.recs[size_t(h.slot_off)];
+    CU(ms::launch_pk_inject(c->d_patches.p, int32_t(np), c->d_recs.p, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
   }
 #endif
-  if (!pk.recs.empty())
-    CU(cudaMemcpy(c->d_recs.p, pk.recs.data(), pk.recs.size() * sizeof(ms::FacetRec), cudaMemcpyHostToDevice));
   return 0;
 }
 
-// Per-facet surface tension of the record slots (slot_gamma) from the context's host copy and current packing.
+// Per-facet surface tension of the record slots (slot_gamma): the context's host copy gathered through the device
+// slot facets.
 int upload_slot_gamma(ms_ctx* c) {
-  const ms::PackedMesh& pk = c->packed;
-  std::vector<double> slot_gamma(pk.slot_facet.size(), 0.0);
-  for (size_t s = 0; s < slot_gamma.size(); ++s)
-    if (pk.slot_facet[s] >= 0) slot_gamma[s] = c->h_gamma[size_t(pk.slot_facet[s])];
-  if (int rc = c->d_slot_gamma.ensure(slot_gamma.size())) return rc;
-  if (!slot_gamma.empty())
-    CU(cudaMemcpy(c->d_slot_gamma.p, slot_gamma.data(), slot_gamma.size() * sizeof(double), cudaMemcpyHostToDevice));
+  DevBuf<double> gamma;
+  if (int rc = gamma.ensure(size_t(c->nf) + 1)) return rc;
+  if (int rc = c->d_slot_gamma.ensure(size_t(c->n_slots) + 1)) return rc;
+  if (c->nf)
+    CU(cudaMemcpyAsync(gamma.p, c->h_gamma.data(), size_t(c->nf) * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  CU(ms::launch_pk_slot_gamma(c->d_slot_facet.p, c->n_slots, gamma.p, c->d_slot_gamma.p, c->stream));
+  CU(cudaStreamSynchronize(c->stream));  // gamma is released on return
   return 0;
 }
 
@@ -716,8 +827,17 @@ int ms_ctx_set_topology_partition(ms_ctx* c, int32_t nv, int32_t n_owned, int32_
     CU(cudaMemcpy(c->d_perm.p, c->perm.data(), size_t(nv) * sizeof(int32_t), cudaMemcpyHostToDevice));
     if (int rc = c->d_stage.ensure(size_t(ms::kSeedStride) * size_t(nv))) return rc;
   }
-  ms::PackedMesh packed;
-  if (int rc = pack_rows(c, nv, n_owned, nf, tri, body_mask, packed)) return rc;
+  // the internal-order rows (and the body flags) go up once and are packed there
+  DevBuf<int32_t> tri_dev;
+  DevBuf<uint8_t> body_dev;
+  if (int rc = tri_dev.ensure(3 * size_t(nf) + 1)) return rc;
+  if (nf) CU(cudaMemcpy(tri_dev.p, tri, 3 * size_t(nf) * sizeof(int32_t), cudaMemcpyHostToDevice));
+  if (body_mask) {
+    if (int rc = body_dev.ensure(size_t(nf) + 1)) return rc;
+    if (nf) CU(cudaMemcpy(body_dev.p, body_mask, size_t(nf), cudaMemcpyHostToDevice));
+  }
+  DevPacking packed;
+  if (int rc = pack_rows(c, nv, n_owned, nf, tri_dev.p, body_mask ? body_dev.p : nullptr, packed)) return rc;
   c->nv = nv;
   c->nf = nf;
   c->h_tri.assign(tri, tri + 3 * size_t(nf));
@@ -728,6 +848,8 @@ int ms_ctx_set_topology_partition(ms_ctx* c, int32_t nv, int32_t n_owned, int32_
   for (auto& lf : c->leaflet) {  // per-leaflet tilt fields are sized for the previous vertex count
     lf.tilts.release(); lf.tilt_grad.release();
   }
+  c->d_tri.swap(tri_dev);
+  c->tri_ready = true;  // d_tri holds the rows
   if (int rc = upload_packing(c, std::move(packed), n_owned)) return rc;
 
   c->has_boundary = is_boundary != nullptr;
@@ -807,7 +929,7 @@ int ms_ctx_pack_info(const ms_ctx* c, ms_pack_info* info) {
   info->max_local = pk.max_local;
   info->max_rounds = pk.max_rounds;
   info->max_slots = pk.max_slots;
-  info->n_slots = int64_t(pk.recs.size());
+  info->n_slots = c->n_slots;
   info->n_listed = pk.n_listed;
   info->n_valid = pk.n_valid;
   info->n_halo = int64_t(pk.halo_ids.size());
@@ -815,6 +937,19 @@ int ms_ctx_pack_info(const ms_ctx* c, ms_pack_info* info) {
   info->n_lane_conflicts = pk.n_lane_conflicts;
   info->n_hw_groups = pk.n_hw_groups;
   info->n_hw_excess = pk.n_hw_excess;
+  return 0;
+}
+
+int ms_ctx_get_packing(const ms_ctx* c, void* headers, int32_t* halo_ids, void* recs, int32_t* slot_facet) {
+  if (int rc = check_ctx(c, true)) return rc;
+  const ms::PackedMesh& pk = c->packed;
+  if (headers && !pk.patches.empty()) std::memcpy(headers, pk.patches.data(), pk.patches.size() * sizeof(ms::PatchHeader));
+  if (halo_ids && !pk.halo_ids.empty()) std::memcpy(halo_ids, pk.halo_ids.data(), pk.halo_ids.size() * sizeof(int32_t));
+  const size_t ns = size_t(c->n_slots);
+  if (recs && ns) CU(cudaMemcpyAsync(recs, c->d_recs.p, ns * sizeof(ms::FacetRec), cudaMemcpyDeviceToHost, c->stream));
+  if (slot_facet && ns)
+    CU(cudaMemcpyAsync(slot_facet, c->d_slot_facet.p, ns * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));
   return 0;
 }
 
@@ -2303,20 +2438,30 @@ int ms_ctx_equiangulate(ms_ctx* c, int32_t max_iterations, int64_t* n_flips, int
   CU(cudaEventElapsedTime(&sweep_ms, ev.e[0], ev.e[1]));
   c->eq_ms[0] = sweep_ms;
   if (total > 0) {
-    // facet rows stay in place, so per-facet and per-vertex data survive; only the packing follows the new rows
-    auto t0 = clock::now();
-    std::vector<int32_t> rows(nh);
-    CU(cudaMemcpy(rows.data(), c->d_tri.p, nh * sizeof(int32_t), cudaMemcpyDeviceToHost));
-    c->eq_ms[1] = ms_since(t0);
-    t0 = clock::now();
-    ms::PackedMesh packed;
-    const int rc = pack_rows(c, c->nv, c->nv, c->nf, rows.data(), c->h_body.empty() ? nullptr : c->h_body.data(), packed);
-    c->eq_ms[2] = ms_since(t0);
+    // facet rows stay in place, so per-facet and per-vertex data survive; only the packing follows the new rows,
+    // packed where they are
+    DevBuf<uint8_t> body_dev;
+    if (!c->h_body.empty()) {
+      if (int rc = body_dev.ensure(size_t(c->nf))) return rc;
+      CU(cudaMemcpyAsync(body_dev.p, c->h_body.data(), size_t(c->nf), cudaMemcpyHostToDevice, c->stream));
+    }
+    CU(cudaEventRecord(ev.e[0], c->stream));
+    DevPacking packed;
+    const int rc = pack_rows(c, c->nv, c->nv, c->nf, c->d_tri.p, body_dev.p, packed);
+    CU(cudaEventRecord(ev.e[1], c->stream));
+    CU(cudaEventSynchronize(ev.e[1]));
+    float pack_ms = 0.f;
+    CU(cudaEventElapsedTime(&pack_ms, ev.e[0], ev.e[1]));
+    c->eq_ms[2] = pack_ms;
     if (rc) {  // the flipped rows do not pack: back to the rows and packing the context had
       const std::string why = g_err;
       CU(cudaMemcpy(c->d_tri.p, c->h_tri.data(), nh * sizeof(int32_t), cudaMemcpyHostToDevice));
       return fail(rc, "equiangulation: " + why + "; the context keeps its previous triangles");
     }
+    auto t0 = clock::now();
+    std::vector<int32_t> rows(nh);
+    CU(cudaMemcpy(rows.data(), c->d_tri.p, nh * sizeof(int32_t), cudaMemcpyDeviceToHost));
+    c->eq_ms[1] = ms_since(t0);
     t0 = clock::now();
     c->h_tri.swap(rows);
     drop_connectivity_state(c);
@@ -2454,8 +2599,34 @@ int ms_ctx_refine(ms_ctx* c, int32_t levels, int32_t* nv_out, int32_t* nf_out) {
   float dev_ms = 0.f;
   CU(cudaEventElapsedTime(&dev_ms, ev.e[0], ev.e[1]));
   c->rf_ms[0] = dev_ms;
-  // only the rows (for the packer and h_tri) and the order come back
+  // children inherit their parent's per-facet values: child j of the last level descends from facet j mod nf0
   auto t0 = clock::now();
+  std::vector<uint8_t> body;
+  std::vector<double> gamma;
+  DevBuf<uint8_t> body_dev;
+  if (!c->h_body.empty()) {
+    body.resize(nf2);
+    for (size_t j = 0; j < nf2; ++j) body[j] = c->h_body[j % size_t(nf0)];
+    if (int rc = body_dev.ensure(nf2)) return rc;
+    CU(cudaMemcpyAsync(body_dev.p, body.data(), nf2, cudaMemcpyHostToDevice, c->stream));
+  }
+  if (!c->h_gamma.empty()) {
+    gamma.resize(nf2);
+    for (size_t j = 0; j < nf2; ++j) gamma[j] = c->h_gamma[j % size_t(nf0)];
+  }
+  const double inherit_ms = ms_since(t0);
+  // the refined rows are packed where they are
+  CU(cudaEventRecord(ev.e[0], c->stream));
+  DevPacking packed;
+  const int prc = pack_rows(c, m.nv, m.nv, m.nf, tri_int.p, body_dev.p, packed);
+  CU(cudaEventRecord(ev.e[1], c->stream));
+  CU(cudaEventSynchronize(ev.e[1]));
+  float pack_ms = 0.f;
+  CU(cudaEventElapsedTime(&pack_ms, ev.e[0], ev.e[1]));
+  c->rf_ms[2] = pack_ms;
+  if (prc) return fail(prc, "refinement: " + std::string(g_err) + "; the context keeps its previous mesh");
+  // only the rows (for h_tri) and the order come back
+  t0 = clock::now();
   std::vector<int32_t> rows(3 * nf2), new_perm(nv2);
   if (nf2) CU(cudaMemcpy(rows.data(), tri_int.p, 3 * nf2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
   if (nv2) CU(cudaMemcpy(new_perm.data(), perm2.p, nv2 * sizeof(int32_t), cudaMemcpyDeviceToHost));
@@ -2466,23 +2637,7 @@ int ms_ctx_refine(ms_ctx* c, int32_t levels, int32_t* nv_out, int32_t* nf_out) {
   if (identity) new_perm.clear();
   if (!new_perm.empty())
     if (int rc = stage.ensure(ms::kSeedStride * nv2)) return rc;
-  // children inherit their parent's per-facet values: child j of the last level descends from facet j mod nf0
-  std::vector<uint8_t> body;
-  std::vector<double> gamma;
-  if (!c->h_body.empty()) {
-    body.resize(nf2);
-    for (size_t j = 0; j < nf2; ++j) body[j] = c->h_body[j % size_t(nf0)];
-  }
-  if (!c->h_gamma.empty()) {
-    gamma.resize(nf2);
-    for (size_t j = 0; j < nf2; ++j) gamma[j] = c->h_gamma[j % size_t(nf0)];
-  }
-  ms::PackedMesh packed;
-  const int prc = pack_rows(c, m.nv, m.nv, m.nf, rows.data(), body.empty() ? nullptr : body.data(), packed);
-  c->rf_ms[2] = ms_since(t0);
-  if (prc) return fail(prc, "refinement: " + std::string(g_err) + "; the context keeps its previous mesh");
   // commit
-  t0 = clock::now();
   c->nv = c->n_owned = m.nv;
   c->nf = m.nf;
   c->h_tri.swap(rows);
@@ -2513,7 +2668,7 @@ int ms_ctx_refine(ms_ctx* c, int32_t levels, int32_t* nv_out, int32_t* nf_out) {
   if (int rc = upload_packing(c, std::move(packed), c->nv)) return rc;
   if (c->has_gamma)
     if (int rc = upload_slot_gamma(c)) return rc;
-  c->rf_ms[3] = ms_since(t0);
+  c->rf_ms[3] = ms_since(t0) + inherit_ms;
   if (nv_out) *nv_out = c->nv;
   if (nf_out) *nf_out = c->nf;
   return 0;

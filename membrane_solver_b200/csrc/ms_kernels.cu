@@ -2568,4 +2568,192 @@ cudaError_t launch_scale(const double* x, double scale, double* out, int64_t n, 
   return cudaGetLastError();
 }
 
+// --- patch packing (ms_pack_device.cuh): one warp per chunk, one thread per corner / vertex row / slot ---
+namespace {
+
+struct PkWarp {
+  __device__ int lane() const { return int(threadIdx.x & 31); }
+  __device__ int size() const { return 32; }
+  __device__ void sync() const { __syncwarp(); }
+  __device__ uint32_t ballot(bool p) const { return __ballot_sync(0xffffffffu, p); }
+  __device__ uint32_t lt_mask() const { return (1u << lane()) - 1u; }
+  __device__ int bcast(int x) const { return __shfl_sync(0xffffffffu, x, 0); }
+  __device__ uint64_t min64(uint64_t x) const {
+    for (int o = 16; o > 0; o >>= 1) {
+      const uint64_t y = __shfl_xor_sync(0xffffffffu, x, o);
+      x = y < x ? y : x;
+    }
+    return x;
+  }
+};
+
+__global__ void __launch_bounds__(256) k_pk_corner_keys(const int32_t* __restrict__ tri, int32_t nv, int64_t n,
+                                                        int32_t* __restrict__ key, int32_t* __restrict__ id) {
+  const int64_t c = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (c >= n) return;
+  key[c] = pk_corner_key(tri, nv, c);
+  id[c] = int32_t(c);
+}
+
+// ptr[v] = first sorted position whose key is >= v
+__global__ void __launch_bounds__(256) k_pk_csr_ptr(const int32_t* __restrict__ skey, int64_t n, int32_t nv,
+                                                    int32_t* __restrict__ ptr) {
+  const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (v > nv) return;
+  int64_t lo = 0, hi = n;
+  while (lo < hi) {
+    const int64_t mid = (lo + hi) / 2;
+    if (skey[mid] < v) lo = mid + 1; else hi = mid;
+  }
+  ptr[v] = int32_t(lo);
+}
+
+__global__ void __launch_bounds__(256) k_pk_bounds(const PackParams p, const int32_t* __restrict__ csr_ptr,
+                                                   int32_t n_owned, unsigned long long* __restrict__ bounds) {
+  const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (v >= n_owned) return;
+  const int64_t chunk = pk_chunk_rows(p), c = v / chunk;
+  const int32_t c1 = int32_t((c + 1) * chunk < n_owned ? (c + 1) * chunk : n_owned);
+  int64_t window, deg;
+  pk_row_bounds(p, csr_ptr, int32_t(v), c1, &window, &deg);
+  atomicMax(bounds + 3 * c, (unsigned long long)window);
+  atomicMax(bounds + 3 * c + 1, (unsigned long long)deg);
+  if (v == c * chunk) bounds[3 * c + 2] = (unsigned long long)(csr_ptr[c1] - csr_ptr[v]);
+}
+
+__global__ void __launch_bounds__(256) k_pk_valid(const int32_t* __restrict__ tri, int32_t nv, int32_t nf,
+                                                  unsigned long long* __restrict__ n_valid) {
+  const int64_t f = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  const bool ok = f < nf && pk_valid(tri + 3 * f, nv);
+  const unsigned mask = __ballot_sync(0xffffffffu, ok);
+  if (mask && (threadIdx.x & 31) == 0) atomicAdd(n_valid, (unsigned long long)__popc(mask));
+}
+
+__global__ void __launch_bounds__(32) k_pk_chunks(const PkMesh m, int32_t* scratch, const PkStage st, PkChunk* chunks) {
+  PkWarp w;
+  const int64_t c = blockIdx.x, chunk = pk_chunk_rows(m.prm);
+  const int32_t v1 = int32_t((c + 1) * chunk < m.n_owned ? (c + 1) * chunk : m.n_owned);
+  pk_chunk(w, m, scratch, st, chunks[c], int32_t(c * chunk), v1);
+}
+
+// one block per chunk: its headers (offsets made global), halo ids and listed records into the concatenation
+__global__ void __launch_bounds__(256) k_pk_concat(const PkStage st, const PkChunk* __restrict__ chunks,
+                                                   const int64_t* __restrict__ bases, PatchHeader* hdr, int32_t* halo,
+                                                   FacetRec* recs, int32_t* slot_facet) {
+  const PkChunk& k = chunks[blockIdx.x];
+  const int64_t hb = bases[3 * blockIdx.x], lb = bases[3 * blockIdx.x + 1], sb = bases[3 * blockIdx.x + 2];
+  for (int64_t j = threadIdx.x; j < k.n_patches; j += blockDim.x) {
+    PatchHeader h = st.hdr[k.hdr_off + j];
+    h.halo_off += int32_t(lb);
+    h.slot_off += sb;
+    hdr[hb + j] = h;
+  }
+  for (int64_t j = threadIdx.x; j < k.n_halo; j += blockDim.x) halo[lb + j] = st.halo[k.halo_off + j];
+  for (int64_t e = k.ent_off + threadIdx.x; e < k.ent_off + k.n_listed; e += blockDim.x) {
+    recs[sb + st.ent_slot[e]] = st.ent_rec[e];
+    slot_facet[sb + st.ent_slot[e]] = st.ent_fac[e];
+  }
+}
+
+// one block per patch, one thread per (round, half-warp)
+__global__ void __launch_bounds__(128) k_pk_hw_excess(const PatchHeader* __restrict__ hdr, const FacetRec* __restrict__ recs,
+                                                      int32_t T, unsigned long long* out) {
+  const PatchHeader h = hdr[blockIdx.x];
+  const int nhw = pk_n_hw(T);
+  int64_t groups = 0, excess = 0;
+  for (int64_t g = threadIdx.x; g < int64_t(h.n_rounds) * nhw; g += blockDim.x) {
+    const int hw = int(g % nhw);
+    pk_hw_excess(recs + h.slot_off + (g / nhw) * T + hw * 16, T - hw * 16 < 16 ? T - hw * 16 : 16, &groups, &excess);
+  }
+  if (groups) atomicAdd(out, (unsigned long long)groups);
+  if (excess) atomicAdd(out + 1, (unsigned long long)excess);
+}
+
+__global__ void __launch_bounds__(256) k_pk_slot_gamma(const int32_t* __restrict__ slot_facet, int64_t n,
+                                                       const double* __restrict__ gamma, double* __restrict__ out) {
+  const int64_t s = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (s >= n) return;
+  const int32_t f = slot_facet[s];
+  out[s] = f >= 0 ? gamma[f] : 0.0;
+}
+
+__global__ void __launch_bounds__(256) k_pk_inject(const PatchHeader* __restrict__ hdr, int32_t n, FacetRec* recs) {
+  const int64_t p = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (p >= n) return;
+  const PatchHeader h = hdr[p];
+  if (h.n_rounds > 0 && (recs[h.slot_off].flags & REC_VALID)) recs[h.slot_off + 1] = recs[h.slot_off];
+}
+
+int pk_key_bits(int32_t nv) {
+  int bits = 1;
+  while (bits < 31 && (uint32_t(nv) >> bits)) ++bits;
+  return bits;
+}
+
+}  // namespace
+
+cudaError_t pk_temp_bytes(int64_t n_corners, size_t* bytes) {
+  return cub::DeviceRadixSort::SortPairs(nullptr, *bytes, (const int32_t*)nullptr, (int32_t*)nullptr,
+                                         (const int32_t*)nullptr, (int32_t*)nullptr, int(n_corners));
+}
+
+cudaError_t launch_pk_corner_csr(const int32_t* tri, int32_t nv, int32_t nf, int32_t* key_in, int32_t* id_in,
+                                 int32_t* key_out, int32_t* csr_idx, int32_t* csr_ptr, void* temp, size_t temp_bytes,
+                                 cudaStream_t st) {
+  const int64_t n = 3 * int64_t(nf);
+  if (n > 0) {
+    k_pk_corner_keys<<<blocks_for(n, 256), 256, 0, st>>>(tri, nv, n, key_in, id_in);
+    if (cudaError_t e = cudaGetLastError()) return e;
+    if (cudaError_t e = cub::DeviceRadixSort::SortPairs(temp, temp_bytes, key_in, key_out, id_in, csr_idx, int(n), 0,
+                                                        pk_key_bits(nv), st))
+      return e;
+  }
+  k_pk_csr_ptr<<<blocks_for(int64_t(nv) + 1, 256), 256, 0, st>>>(key_out, n, nv, csr_ptr);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pk_bounds(const PackParams& p, const int32_t* csr_ptr, int32_t n_owned, const int32_t* tri,
+                             int32_t nv, int32_t nf, unsigned long long* bounds, int64_t n_chunks,
+                             unsigned long long* n_valid, cudaStream_t st) {
+  if (cudaError_t e = cudaMemsetAsync(bounds, 0, (3 * size_t(n_chunks) + 1) * sizeof(unsigned long long), st)) return e;
+  if (n_owned > 0) k_pk_bounds<<<blocks_for(n_owned, 256), 256, 0, st>>>(p, csr_ptr, n_owned, bounds);
+  if (cudaError_t e = cudaGetLastError()) return e;
+  if (nf > 0) k_pk_valid<<<blocks_for(nf, 256), 256, 0, st>>>(tri, nv, nf, n_valid);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pk_chunks(const PkMesh& m, int32_t* scratch, const PkStage& stage, PkChunk* chunks, int64_t n_chunks,
+                             cudaStream_t st) {
+  if (n_chunks > 0) k_pk_chunks<<<unsigned(n_chunks), 32, 0, st>>>(m, scratch, stage, chunks);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pk_concat(const PkStage& stage, const PkChunk* chunks, const int64_t* bases, int64_t n_chunks,
+                             PatchHeader* hdr, int32_t* halo, FacetRec* recs, int32_t* slot_facet, int64_t n_slots,
+                             cudaStream_t st) {
+  if (n_slots > 0) {
+    if (cudaError_t e = cudaMemsetAsync(recs, 0, size_t(n_slots) * sizeof(FacetRec), st)) return e;
+    if (cudaError_t e = cudaMemsetAsync(slot_facet, 0xff, size_t(n_slots) * sizeof(int32_t), st)) return e;
+  }
+  if (n_chunks > 0) k_pk_concat<<<unsigned(n_chunks), 256, 0, st>>>(stage, chunks, bases, hdr, halo, recs, slot_facet);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pk_hw_excess(const PatchHeader* hdr, int32_t n_patches, const FacetRec* recs, int32_t threads,
+                                unsigned long long* out, cudaStream_t st) {
+  if (cudaError_t e = cudaMemsetAsync(out, 0, 2 * sizeof(unsigned long long), st)) return e;
+  if (n_patches > 0) k_pk_hw_excess<<<unsigned(n_patches), 128, 0, st>>>(hdr, recs, threads, out);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pk_slot_gamma(const int32_t* slot_facet, int64_t n, const double* gamma, double* out, cudaStream_t st) {
+  if (n > 0) k_pk_slot_gamma<<<blocks_for(n, 256), 256, 0, st>>>(slot_facet, n, gamma, out);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pk_inject(const PatchHeader* hdr, int32_t n_patches, FacetRec* recs, cudaStream_t st) {
+  if (n_patches > 0) k_pk_inject<<<blocks_for(n_patches, 256), 256, 0, st>>>(hdr, n_patches, recs);
+  return cudaGetLastError();
+}
+
 }  // namespace ms

@@ -11,6 +11,7 @@
 #include "ms_math.cuh"
 #include "ms_pack.h"
 #include "ms_equiangulate.cuh"
+#include "ms_pack_device.cuh"
 #include "ms_refine.cuh"
 #include "ms_vertex_average.cuh"
 
@@ -360,5 +361,32 @@ cudaError_t launch_rf_renumber(const int32_t* rows, int64_t n, const int32_t* in
 // out[i] = src[perm[i]], and out32[i] = out[i] != 0 when out32 is set
 cudaError_t launch_rf_gather_flags(const uint8_t* src, const int32_t* perm, int64_t n, uint8_t* out, int32_t* out32,
                                    cudaStream_t st);
+
+// --- patch packing on the device (ms_pack_device.cuh): the layout of ms::pack_patches, byte for byte ---
+// scratch of the corner sort for n_corners = 3 nf items
+cudaError_t pk_temp_bytes(int64_t n_corners, size_t* bytes);
+// corner CSR (corner ids 3 f + k by vertex, facet-major; the facets with an index out of range left out): csr_ptr
+// gets nv + 1 offsets, csr_idx 3 nf entries of which the first csr_ptr[nv] are the CSR
+cudaError_t launch_pk_corner_csr(const int32_t* tri, int32_t nv, int32_t nf, int32_t* key_in, int32_t* id_in,
+                                 int32_t* key_out, int32_t* csr_idx, int32_t* csr_ptr, void* temp, size_t temp_bytes,
+                                 cudaStream_t st);
+// per chunk (3 n_chunks + 1 words, zeroed here): the pk_plan bounds; bounds[3 n_chunks] = facets with all indices in range
+cudaError_t launch_pk_bounds(const PackParams& p, const int32_t* csr_ptr, int32_t n_owned, const int32_t* tri,
+                             int32_t nv, int32_t nf, unsigned long long* bounds, int64_t n_chunks,
+                             unsigned long long* n_valid, cudaStream_t st);
+// one warp per chunk: pk_chunk into the staging
+cudaError_t launch_pk_chunks(const PkMesh& m, int32_t* scratch, const PkStage& stage, PkChunk* chunks, int64_t n_chunks,
+                             cudaStream_t st);
+// concatenation in chunk order; bases = (first patch, first halo id, first slot) of every chunk
+cudaError_t launch_pk_concat(const PkStage& stage, const PkChunk* chunks, const int64_t* bases, int64_t n_chunks,
+                             PatchHeader* hdr, int32_t* halo, FacetRec* recs, int32_t* slot_facet, int64_t n_slots,
+                             cudaStream_t st);
+// out[0] = n_hw_groups, out[1] = n_hw_excess of the packing
+cudaError_t launch_pk_hw_excess(const PatchHeader* hdr, int32_t n_patches, const FacetRec* recs, int32_t threads,
+                                unsigned long long* out, cudaStream_t st);
+// out[s] = gamma[slot_facet[s]], 0 for an empty slot
+cudaError_t launch_pk_slot_gamma(const int32_t* slot_facet, int64_t n, const double* gamma, double* out, cudaStream_t st);
+// self-check negative control: slot 1 of every patch's first round repeats slot 0
+cudaError_t launch_pk_inject(const PatchHeader* hdr, int32_t n_patches, FacetRec* recs, cudaStream_t st);
 
 }  // namespace ms

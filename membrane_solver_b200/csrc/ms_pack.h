@@ -1,5 +1,8 @@
 // Host-side packing of a triangle mesh into shared-memory sized vertex patches.
 //
+// The context packs on the device (ms_pack_device.cuh), byte for byte this layout; pack_patches stays as the
+// reference the emulator and the tests compare against (its MS_PACK_THREADS knob concerns only this host version).
+//
 // This replaces, for the device path, what geometry/triangle_rows.py:10-35 and
 // Mesh.triangle_row_cache (geometry/mesh.py:597-624) do for the reference: it
 // turns the (nf,3) int32 triangle rows into the layout the kernels stream.
