@@ -457,6 +457,46 @@ MS_API int ms_ctx_normal_change_ok(ms_ctx* ctx, double limit_radians, int32_t* o
 /* deterministic <g,g>, <g,gC>, <gC,gC> into the scalar vector */
 MS_API int ms_ctx_dots(ms_ctx* ctx);
 
+/* ---- the minimiser loop under device control (runtime/device_minimizer.py: DeviceMinimizer.minimize) ----------
+ * The fields of DeviceMinimizer that the loop reads. */
+typedef struct ms_minimize_opts {
+  uint32_t modules;            /* MS_MOD_SURFACE / _VOLUME / _BENDING / _TILT; the energy is the sum of the surface,
+                                  bending and tilt energies (+ the penalty term) */
+  uint32_t flags;              /* MS_FLAG_* */
+  int32_t volume_mode;         /* -1 none, 0 lagrange (KKT projection of the gradient), 1 penalty */
+  int32_t enforce_volume;      /* hard volume constraint: Newton projection of the positions (needs volume_mode >= 0) */
+  int32_t projection_during;   /* project inside the line search (else: after a step whose volume drifted) */
+  int32_t stepper;             /* 0 gradient descent, 1 per-vertex Polak-Ribiere conjugate gradient */
+  int32_t max_zero_steps, max_iter, restart_interval, reserved;  /* max_iter in [0, 2^20], restart_interval >= 1 */
+  double k_vol, v_target, tol, step_size_floor, beta, c, gamma, alpha_max_factor, edge_fraction, volume_tolerance;
+} ms_minimize_opts;
+
+/* In: step_size, cg_iter, cg_have_history (the minimiser's state).  Out: the same after the call and the result dict
+ * of DeviceMinimizer.minimize (grad_norm only when has_grad_norm); n_history = line searches run (history rows). */
+typedef struct ms_minimize_result {
+  double step_size;
+  int32_t cg_iter, cg_have_history;
+  double energy, grad_norm;
+  int32_t iterations, terminated_early, step_success, has_grad_norm;
+  int32_t n_history, reserved;
+} ms_minimize_result;
+
+/* n_steps steps of DeviceMinimizer.minimize with every decision taken on the device: the host enqueues one CUDA graph
+ * (a WHILE node around a one-thread control kernel and one IF node per action: evaluation, direction, line-search
+ * statistics, trial, normal-flip guard, Newton volume projection, acceptance, drift check) and synchronises ONCE.  The
+ * decisions, positions, energies, step sizes, history and conjugate-gradient state are bitwise those of the host loop
+ * driving the same context through the single calls.  history (may be NULL): 4 doubles per line search (step index,
+ * accepted energy, step size in, success), at most `capacity` rows.  Refused (error, context unchanged): a partition
+ * context (n_owned < nv), no topology or positions, n_steps < 0, options outside the bounds above or with
+ * MS_MOD_BENDING_TILT / MS_MOD_TILT_SMOOTHNESS. */
+MS_API int ms_ctx_minimize(ms_ctx* ctx, const ms_minimize_opts* opts, int32_t n_steps, ms_minimize_result* io,
+                           double* history, int32_t capacity);
+/* The last ms_ctx_minimize: counts7 = {line searches, trials, evaluations, host synchronisations (the blocking waits
+ * of the call: the final synchronise, plus the upload of the triangle rows when the context had not made it yet),
+ * actions, normal-flip guards run, trials the guard rejected}; ms2 = {device time of the graph (CUDA events), host
+ * time to build and instantiate it}.  Either may be NULL. */
+MS_API int ms_ctx_minimize_stats(const ms_ctx* ctx, int64_t* counts7, double* ms2);
+
 /* timing on the context stream (CUDA events) and an L2 flush for benchmarks */
 MS_API int ms_ctx_timer_start(ms_ctx* ctx);
 MS_API int ms_ctx_timer_stop(ms_ctx* ctx, float* milliseconds);

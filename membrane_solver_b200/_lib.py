@@ -92,6 +92,32 @@ class PackInfo(ctypes.Structure):
     ]
 
 
+class MinimizeOpts(ctypes.Structure):
+    """struct ms_minimize_opts (include/ms_b200.h)."""
+    _fields_ = [
+        ("modules", ctypes.c_uint32), ("flags", ctypes.c_uint32),
+        ("volume_mode", ctypes.c_int32), ("enforce_volume", ctypes.c_int32),
+        ("projection_during", ctypes.c_int32), ("stepper", ctypes.c_int32),
+        ("max_zero_steps", ctypes.c_int32), ("max_iter", ctypes.c_int32),
+        ("restart_interval", ctypes.c_int32), ("reserved", ctypes.c_int32),
+        ("k_vol", ctypes.c_double), ("v_target", ctypes.c_double), ("tol", ctypes.c_double),
+        ("step_size_floor", ctypes.c_double), ("beta", ctypes.c_double), ("c", ctypes.c_double),
+        ("gamma", ctypes.c_double), ("alpha_max_factor", ctypes.c_double), ("edge_fraction", ctypes.c_double),
+        ("volume_tolerance", ctypes.c_double),
+    ]
+
+
+class MinimizeResult(ctypes.Structure):
+    """struct ms_minimize_result (include/ms_b200.h)."""
+    _fields_ = [
+        ("step_size", ctypes.c_double), ("cg_iter", ctypes.c_int32), ("cg_have_history", ctypes.c_int32),
+        ("energy", ctypes.c_double), ("grad_norm", ctypes.c_double),
+        ("iterations", ctypes.c_int32), ("terminated_early", ctypes.c_int32),
+        ("step_success", ctypes.c_int32), ("has_grad_norm", ctypes.c_int32),
+        ("n_history", ctypes.c_int32), ("reserved", ctypes.c_int32),
+    ]
+
+
 _D = ctypes.POINTER(ctypes.c_double)
 _I = ctypes.POINTER(ctypes.c_int32)
 _B = ctypes.POINTER(ctypes.c_uint8)
@@ -183,6 +209,8 @@ SIGNATURES = {
     "ms_ctx_cg_commit": (ctypes.c_int, [_V]),
     "ms_ctx_line_search_stats": (ctypes.c_int, [_V, _D]),
     "ms_ctx_normal_change_ok": (ctypes.c_int, [_V, _f64, _I]),
+    "ms_ctx_minimize": (ctypes.c_int, [_V, ctypes.POINTER(MinimizeOpts), _i32, ctypes.POINTER(MinimizeResult), _D, _i32]),
+    "ms_ctx_minimize_stats": (ctypes.c_int, [_V, ctypes.POINTER(_i64), _D]),
     "ms_ctx_timer_start": (ctypes.c_int, [_V]),
     "ms_ctx_timer_stop": (ctypes.c_int, [_V, ctypes.POINTER(ctypes.c_float)]),
     "ms_ctx_sync": (ctypes.c_int, [_V]),

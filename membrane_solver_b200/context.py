@@ -569,6 +569,29 @@ class DeviceMesh:
         L.check(self._lib.ms_ctx_normal_change_ok(self._h, float(limit_radians), ctypes.byref(ok)))
         return bool(ok.value)
 
+    def minimize(self, opts: L.MinimizeOpts, n_steps: int, *, step_size: float, cg_iter: int = 0,
+                 cg_have_history: bool = False) -> tuple[L.MinimizeResult, list]:
+        """``n_steps`` steps of ``DeviceMinimizer.minimize`` under device control (``ms_ctx_minimize``): one CUDA graph,
+        one host synchronisation.  Returns the result struct (step size and conjugate-gradient state after the call
+        included) and the history rows ``(step, accepted energy, step size in, success)``."""
+        res = L.MinimizeResult(step_size=float(step_size), cg_iter=int(cg_iter), cg_have_history=int(bool(cg_have_history)))
+        cap = max(int(n_steps), 0)
+        hist = np.zeros((max(cap, 1), 4))
+        L.check(self._lib.ms_ctx_minimize(self._h, ctypes.byref(opts), int(n_steps), ctypes.byref(res), L.dptr(hist), cap))
+        rows = [(int(h[0]), float(h[1]), float(h[2]), bool(h[3])) for h in hist[:min(res.n_history, cap)]]
+        return res, rows
+
+    def minimize_stats(self) -> dict:
+        """The last ``minimize``: line searches, trials, evaluations, host synchronisations (blocking waits of the
+        call), actions, normal-flip guards run and trials they rejected, the device time of its graph (CUDA events) and
+        the host time spent building the graph, in ms."""
+        n = np.zeros(7, dtype=np.int64)
+        ms = np.zeros(2)
+        L.check(self._lib.ms_ctx_minimize_stats(self._h, n.ctypes.data_as(ctypes.POINTER(ctypes.c_int64)), L.dptr(ms)))
+        return {"steps": int(n[0]), "trials": int(n[1]), "evaluations": int(n[2]), "host_syncs": int(n[3]),
+                "actions": int(n[4]), "guards": int(n[5]), "guard_rejects": int(n[6]), "device_ms": float(ms[0]),
+                "build_ms": float(ms[1])}
+
     def dots(self) -> None:
         L.check(self._lib.ms_ctx_dots(self._h))
 

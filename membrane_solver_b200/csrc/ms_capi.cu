@@ -76,6 +76,11 @@ struct ms_ctx {
   ~ms_ctx() {
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
+    for (cudaEvent_t e : mn_ev)
+      if (e) cudaEventDestroy(e);
+    if (h_min_state) cudaFreeHost(h_min_state);
+    if (h_min_hist) cudaFreeHost(h_min_hist);
+    if (mn_stream) cudaStreamDestroy(mn_stream);
   }
   int device = 0;
   cudaStream_t stream = nullptr;
@@ -188,6 +193,16 @@ struct ms_ctx {
   DevBuf<int> d_halo_error;
   unsigned long long flag_epoch[4] = {0, 0, 0, 0};
   bool vnormals_ready = false;
+  // ms_ctx_minimize: loop state and history on the device, the capture stream of its graph, its statistics
+  DevBuf<ms::MinState> d_min_state;
+  DevBuf<double> d_min_hist;
+  ms::MinState* h_min_state = nullptr;  // pinned staging: the copies around the graph do not block the host
+  double* h_min_hist = nullptr;
+  size_t h_min_hist_n = 0;
+  cudaStream_t mn_stream = nullptr;
+  cudaEvent_t mn_ev[2] = {nullptr, nullptr};
+  int64_t mn_counts[7] = {0, 0, 0, 0, 0, 0, 0};
+  double mn_ms[2] = {0, 0};
 };
 
 namespace {
@@ -2741,18 +2756,9 @@ int ms_ctx_cg_commit(ms_ctx* c) {
   return 0;
 }
 
-int ms_ctx_line_search_stats(ms_ctx* c, double* out4) {
-  if (int rc = check_ctx(c, true)) return rc;
-  if (!out4) return fail(-1, "null argument");
-  if (!c->d_dir.p) return fail(-4, "no search direction exists (ms_ctx_direction_from_gradient / MS_ARR_DIRECTION)");
-  if (int rc = ensure_tri(c)) return rc;
-  if (int rc = c->d_ls_bits.ensure(4)) return rc;
-  const double big = 1.0e300, zero = 0.0;
-  unsigned long long init[4];
-  std::memcpy(&init[0], &big, 8);
-  std::memcpy(&init[1], &zero, 8);
-  init[2] = init[3] = 0;
-  CU(cudaMemcpyAsync(c->d_ls_bits.p, init, sizeof(init), cudaMemcpyHostToDevice, c->stream));
+// the reductions of ms_ctx_line_search_stats, left on the device (d_ls_bits, scalars); needs d_tri and d_ls_bits
+static int enqueue_line_search_stats(ms_ctx* c) {
+  CU(ms::launch_ls_init(c->d_ls_bits.p, c->stream));
   CU(ms::launch_min_edge2(c->d_tri.p, c->nf, c->nv, c->d_pos.p, c->d_ls_bits.p, c->stream));
   CU(ms::launch_max_row_norm2(c->d_dir.p, c->n_owned, c->d_ls_bits.p + 1, c->stream));
   // <g,g>, <g,d>, <d,d> with the deterministic two-level sum; they land in the scalar vector
@@ -2763,18 +2769,22 @@ int ms_ctx_line_search_stats(ms_ctx* c, double* out4) {
   else
     CU(ms::launch_dots(c->d_grad.p, c->d_dir.p, 3 * int64_t(c->n_owned), c->d_dot_partials.p, kDotBlocks,
                        c->d_scalars.p, c->stream));
+  return 0;
+}
+
+int ms_ctx_line_search_stats(ms_ctx* c, double* out4) {
+  if (int rc = check_ctx(c, true)) return rc;
+  if (!out4) return fail(-1, "null argument");
+  if (!c->d_dir.p) return fail(-4, "no search direction exists (ms_ctx_direction_from_gradient / MS_ARR_DIRECTION)");
+  if (int rc = ensure_tri(c)) return rc;
+  if (int rc = c->d_ls_bits.ensure(4)) return rc;
+  if (int rc = enqueue_line_search_stats(c)) return rc;
   unsigned long long bits[4];
   double sc[MS_SC_COUNT];
   CU(cudaMemcpyAsync(bits, c->d_ls_bits.p, sizeof(bits), cudaMemcpyDeviceToHost, c->stream));
   CU(cudaMemcpyAsync(sc, c->d_scalars.p, sizeof(sc), cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
-  double e2, d2;
-  std::memcpy(&e2, &bits[0], 8);
-  std::memcpy(&d2, &bits[1], 8);
-  out4[0] = (c->nf > 0 && e2 < 1.0e299) ? std::sqrt(e2) : 0.0;  // minimum edge length
-  out4[1] = std::sqrt(d2);                                       // largest row norm of the direction
-  out4[2] = sc[MS_SC_G_GC];                                      // <gradient, direction>
-  out4[3] = sc[MS_SC_G_G];                                       // <gradient, gradient>
+  ms::ms_min_ls_stats(bits, sc, c->nf, out4);  // min edge length, largest row norm of d, <g,d>, <g,g>
   return 0;
 }
 
@@ -2794,6 +2804,297 @@ int ms_ctx_normal_change_ok(ms_ctx* c, double limit_radians, int32_t* ok) {
   CU(cudaMemcpyAsync(&host_flag, flag, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
   CU(cudaStreamSynchronize(c->stream));
   *ok = host_flag ? 0 : 1;
+  return 0;
+}
+
+// ---- ms_ctx_minimize: the loop of DeviceMinimizer.minimize as one CUDA graph -------------------------------------
+// Graph: WHILE(run) { k_min_control -> IF(act == k) { launches of action k } for every action k the options can
+// reach }.  The control kernel reads the scalars the last action left on the device, advances the state machine of
+// ms_minimize.cuh and opens the IF node of the next action; MN_DONE closes the WHILE node.  Each action's body is
+// captured from the same entry points the host loop calls, so the launches (and their bits) are the same.
+}  // extern "C"
+namespace {
+
+// the evaluation options DeviceMinimizer._opts / _enforce / the drift check build
+ms_eval_opts min_eval_opts(const ms::MinOpts& o, bool want_grad, bool use_trial) {
+  ms_eval_opts e;
+  std::memset(&e, 0, sizeof(e));
+  e.modules = o.modules | (o.volume_mode >= 0 ? MS_MOD_VOLUME : 0u);
+  e.flags = o.flags;
+  e.want_grad = want_grad;
+  e.constraint_mode = o.volume_mode;
+  e.k_vol = o.k_vol;
+  e.v_target = o.v_target;
+  e.apply_fixed = 1;
+  e.use_trial = use_trial;
+  e.patch_count = -1;
+  return e;
+}
+
+ms_eval_opts volume_eval_opts(bool want_grad, bool use_trial) {
+  ms_eval_opts e;
+  std::memset(&e, 0, sizeof(e));
+  e.modules = MS_MOD_VOLUME;
+  e.want_grad = want_grad;
+  e.constraint_mode = -1;
+  e.use_trial = use_trial;
+  e.patch_count = -1;
+  return e;
+}
+
+// record the launches of fn() into `body` (a conditional node's graph) instead of running them
+template <class F>
+int capture_into(ms_ctx* c, cudaGraph_t body, F&& fn) {
+  CU(cudaStreamBeginCaptureToGraph(c->mn_stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed));
+  cudaStream_t saved = c->stream;
+  c->stream = c->mn_stream;
+  const int rc = fn();
+  c->stream = saved;
+  cudaGraph_t g = nullptr;
+  const cudaError_t e = cudaStreamEndCapture(c->mn_stream, &g);
+  if (rc) return rc;
+  CU(e);
+  return 0;
+}
+
+int add_conditional(cudaGraph_t graph, const cudaGraphNode_t* dep, size_t n_dep, cudaGraphConditionalHandle h,
+                    cudaGraphConditionalNodeType type, cudaGraph_t* body) {
+  alignas(cudaGraphNodeParams) unsigned char raw[sizeof(cudaGraphNodeParams)] = {};  // zeroed (no default constructor)
+  cudaGraphNodeParams& p = *reinterpret_cast<cudaGraphNodeParams*>(raw);
+  p.type = cudaGraphNodeTypeConditional;
+  p.conditional.handle = h;
+  p.conditional.type = type;
+  p.conditional.size = 1;
+  cudaGraphNode_t node;
+  CU(cudaGraphAddNode(&node, graph, dep, n_dep, &p));
+  *body = p.conditional.phGraph_out[0];
+  return 0;
+}
+
+struct GraphHolder {
+  cudaGraph_t g = nullptr;
+  cudaGraphExec_t exec = nullptr;
+  ~GraphHolder() {
+    if (exec) cudaGraphExecDestroy(exec);
+    if (g) cudaGraphDestroy(g);
+  }
+};
+
+// the launches of action k (captured into its IF node)
+int minimize_action(ms_ctx* c, const ms::MinOpts& o, int k, ms::MinState* st, const ms_ctx::PendingProjection& p_grad) {
+  const int64_t nv = c->nv;
+  switch (k) {
+    case ms::MN_EVAL_GRAD: {
+      const ms_eval_opts e = min_eval_opts(o, true, false);
+      return ms_ctx_eval_async(c, &e);
+    }
+    case ms::MN_DIRECTION:
+      c->proj = p_grad;  // what the gradient evaluation left
+      if (o.stepper == 0) return ms_ctx_direction_from_gradient(c, -1.0);
+      if (int rc = flush_projection(c)) return rc;
+      CU(ms::launch_cg_direction(c->d_grad.p, c->d_cg_prev_g.p, c->d_cg_prev_d.p, c->has_fixed ? c->d_fixed.p : nullptr,
+                                 nv, c->d_dir.p, c->stream, &st->cg_restart));
+      return ms_ctx_cg_commit(c);
+    case ms::MN_STATS:
+      c->proj = p_grad;
+      if (o.stepper == 1) c->proj.active = false;  // the conjugate-gradient direction applied it in place
+      return enqueue_line_search_stats(c);
+    case ms::MN_EVAL_ENERGY: case ms::MN_EVAL_TRIAL: {
+      const ms_eval_opts e = min_eval_opts(o, false, k == ms::MN_EVAL_TRIAL);
+      return ms_ctx_eval_async(c, &e);
+    }
+    case ms::MN_MAKE_TRIAL:
+      CU(ms::launch_axpy(c->d_pos.p, c->d_dir.p, 0.0, c->d_trial.p, 3 * nv, c->stream, &st->alpha));
+      return 0;
+    case ms::MN_GUARD: {
+      int* flag = reinterpret_cast<int*>(c->d_ls_bits.p + 2);
+      CU(cudaMemsetAsync(flag, 0, sizeof(int), c->stream));
+      CU(ms::launch_normal_change(c->d_tri.p, c->nf, c->nv, c->d_pos.p, c->d_trial.p, std::cos(0.5), flag, c->stream));
+      return 0;
+    }
+    case ms::MN_ENF_EVAL_POS: case ms::MN_ENF_EVAL_TRIAL: {
+      const ms_eval_opts e = volume_eval_opts(true, k == ms::MN_ENF_EVAL_TRIAL);
+      return ms_ctx_eval_async(c, &e);
+    }
+    case ms::MN_ENF_AXPY_POS: case ms::MN_ENF_AXPY_TRIAL:
+      CU(ms::launch_axpy_rows(c->d_volgrad.p, 0.0, c->has_fixed ? c->d_fixed.p : nullptr, nv,
+                              k == ms::MN_ENF_AXPY_TRIAL ? c->d_trial.p : c->d_pos.p, c->stream, &st->neg_lam));
+      return 0;
+    case ms::MN_ACCEPT:
+      CU(cudaMemcpyAsync(c->d_pos.p, c->d_trial.p, 3 * size_t(nv) * sizeof(double), cudaMemcpyDeviceToDevice, c->stream));
+      return 0;
+    case ms::MN_DRIFT_EVAL: {
+      const ms_eval_opts e = volume_eval_opts(false, false);
+      return ms_ctx_eval_async(c, &e);
+    }
+    default: return fail(-1, "unknown action");
+  }
+}
+
+bool action_reachable(const ms::MinOpts& o, int k) {
+  switch (k) {
+    case ms::MN_ENF_EVAL_POS: case ms::MN_ENF_AXPY_POS: return o.enforce_volume != 0;
+    case ms::MN_ENF_EVAL_TRIAL: case ms::MN_ENF_AXPY_TRIAL: return o.enforce_volume && o.projection_during;
+    case ms::MN_DRIFT_EVAL: return o.enforce_volume && o.volume_mode == 0 && !o.projection_during;
+    default: return true;
+  }
+}
+
+// build and instantiate the graph; the host mirrors the captures touch are restored by the caller
+int minimize_build(ms_ctx* c, const ms::MinOpts& o, int32_t hist_cap, const ms_ctx::PendingProjection& p_grad,
+                   int32_t ran_a_grad, GraphHolder& gh) {
+  CU(cudaGraphCreate(&gh.g, 0));
+  ms::MinHandles h;
+  std::memset(&h, 0, sizeof(h));
+  CU(cudaGraphConditionalHandleCreate(&h.run, gh.g, 1, cudaGraphCondAssignDefault));
+  cudaGraph_t loop;
+  if (int rc = add_conditional(gh.g, nullptr, 0, h.run, cudaGraphCondTypeWhile, &loop)) return rc;
+  for (int k = 0; k < ms::MN_ACTIONS; ++k)
+    if (action_reachable(o, k)) {
+      CU(cudaGraphConditionalHandleCreate(&h.act[k], loop, 0, 0));
+      h.present |= 1u << k;
+    }
+  ms::MinState* st = c->d_min_state.p;
+  if (int rc = capture_into(c, loop, [&] {
+        CU(ms::launch_min_control(o, st, c->d_scalars.p, c->d_ls_bits.p, c->nf, c->d_min_hist.p, hist_cap,
+                                  p_grad.active ? 1 : 0, ran_a_grad, h, c->stream));
+        return 0;
+      }))
+    return rc;
+  cudaGraphNode_t ctrl;
+  size_t n_nodes = 1;
+  CU(cudaGraphGetNodes(loop, &ctrl, &n_nodes));
+  for (int k = 0; k < ms::MN_ACTIONS; ++k) {
+    if (!(h.present & (1u << k))) continue;
+    cudaGraph_t body;
+    if (int rc = add_conditional(loop, &ctrl, 1, h.act[k], cudaGraphCondTypeIf, &body)) return rc;
+    if (int rc = capture_into(c, body, [&] { return minimize_action(c, o, k, st, p_grad); })) return rc;
+  }
+  CU(cudaGraphInstantiate(&gh.exec, gh.g, 0));
+  return 0;
+}
+
+}  // namespace
+extern "C" {
+
+int ms_ctx_minimize(ms_ctx* c, const ms_minimize_opts* opts, int32_t n_steps, ms_minimize_result* io, double* history,
+                    int32_t capacity) {
+  if (int rc = check_ctx(c, true)) return rc;
+  if (!opts || !io) return fail(-1, "null argument");
+  if (c->n_owned != c->nv) return fail(-6, "ms_ctx_minimize runs on single-context meshes (not on a partition)");
+  if (n_steps < 0) return fail(-1, "n_steps must be >= 0");
+  if (capacity < 0 || (capacity > 0 && !history)) return fail(-1, "history capacity without a history buffer");
+  if (!ms::ms_min_valid(*opts)) return fail(-1, "ms_minimize_opts outside the supported bounds");
+  if (!c->has_positions) return fail(-4, "no positions uploaded");
+  if (c->packed.patches.empty()) return fail(-2, "the mesh has no patches");
+  const ms::MinOpts o = *opts;
+  const size_t n3 = 3 * size_t(c->nv);
+  // a committed conjugate-gradient pair exists (ms_ctx_cg_direction restarts without one); the buffers allocated below
+  // for the captured launches do not hold one
+  const bool cg_valid = c->d_cg_prev_g.p && c->d_cg_prev_g.n >= n3;
+  int64_t host_syncs = c->tri_ready ? 1 : 2;  // the final synchronise, and the blocking row upload of ensure_tri
+  // every allocation before anything is enqueued: the captured launches must find their buffers in place
+  for (int w : {MS_ARR_TRIAL, MS_ARR_DIRECTION})
+    if (int rc = ensure_array(c, w)) return rc;
+  if (o.modules & MS_MOD_TILT) {
+    if (!c->d_tilts.p) return fail(-5, "tilt module requested but no tilts were uploaded");
+    if (int rc = c->d_tilt_sq.ensure(size_t(c->nv) + 1)) return rc;
+    if (int rc = ensure_array(c, MS_ARR_TILT_GRAD)) return rc;
+  }
+  if (o.stepper == 1) {
+    if (int rc = c->d_cg_prev_g.ensure(n3 + 1)) return rc;
+    if (int rc = c->d_cg_prev_d.ensure(n3 + 1)) return rc;
+  }
+  if (int rc = ensure_tri(c)) return rc;
+  if (int rc = c->d_ls_bits.ensure(4)) return rc;
+  if (!c->d_ticket.p) {
+    if (int rc = c->d_ticket.ensure(4)) return rc;
+    CU(cudaMemsetAsync(c->d_ticket.p, 0, 4 * sizeof(unsigned int), c->stream));
+  }
+  if (int rc = c->d_min_state.ensure(1)) return rc;
+  const int32_t hist_rows = std::max<int32_t>(n_steps, 1);
+  if (int rc = c->d_min_hist.ensure(4 * size_t(hist_rows))) return rc;
+  const size_t rows_back = size_t(std::min(capacity, hist_rows));
+  if (!c->h_min_state) CU(cudaMallocHost(reinterpret_cast<void**>(&c->h_min_state), sizeof(ms::MinState)));
+  if (rows_back > c->h_min_hist_n) {
+    if (c->h_min_hist) cudaFreeHost(c->h_min_hist);
+    c->h_min_hist = nullptr;
+    c->h_min_hist_n = 0;
+    CU(cudaMallocHost(reinterpret_cast<void**>(&c->h_min_hist), 4 * rows_back * sizeof(double)));
+    c->h_min_hist_n = rows_back;
+  }
+  if (!c->mn_stream) CU(cudaStreamCreateWithFlags(&c->mn_stream, cudaStreamNonBlocking));
+  for (cudaEvent_t& e : c->mn_ev)
+    if (!e) CU(cudaEventCreate(&e));
+
+  // the projection an MN_EVAL_GRAD leaves pending, and whether it runs pass A
+  const ms_eval_opts eg = min_eval_opts(o, true, false);
+  ms_ctx::PendingProjection p_grad;
+  projection_of(c, &eg, p_grad.use_gc, p_grad.use_fixed);
+  p_grad.active = p_grad.use_gc || p_grad.use_fixed;
+  const int32_t ran_a_grad = needs_bending(&eg) ? 1 : 0;
+
+  const auto t0 = std::chrono::steady_clock::now();
+  const ms_ctx::PendingProjection proj0 = c->proj;
+  const bool ran_a0 = c->ran_pass_a;
+  GraphHolder gh;
+  const int brc = minimize_build(c, o, hist_rows, p_grad, ran_a_grad, gh);
+  c->proj = proj0;  // the captures ran nothing: the host mirrors stay as they were
+  c->ran_pass_a = ran_a0;
+  if (brc) return brc;
+  c->mn_ms[1] = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+
+  ms::MinState& s = *c->h_min_state;
+  std::memset(&s, 0, sizeof(s));
+  s.step_size = io->step_size;
+  s.cg_iter = io->cg_iter;
+  s.cg_have_history = io->cg_have_history ? 1 : 0;
+  s.cg_valid = cg_valid ? 1 : 0;
+  s.n_steps = n_steps;
+  s.pc = ms::PC_START;
+  s.proj_active = -1;  // unchanged until an action changes it
+  s.last_ran_a = -1;
+  CU(cudaMemcpyAsync(c->d_min_state.p, &s, sizeof(s), cudaMemcpyHostToDevice, c->stream));
+  CU(cudaEventRecord(c->mn_ev[0], c->stream));
+  CU(cudaGraphLaunch(gh.exec, c->stream));
+  CU(cudaEventRecord(c->mn_ev[1], c->stream));
+  CU(cudaMemcpyAsync(&s, c->d_min_state.p, sizeof(s), cudaMemcpyDeviceToHost, c->stream));
+  if (rows_back)
+    CU(cudaMemcpyAsync(c->h_min_hist, c->d_min_hist.p, 4 * rows_back * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  CU(cudaStreamSynchronize(c->stream));  // the one host synchronisation of the call
+  if (rows_back) std::memcpy(history, c->h_min_hist, 4 * rows_back * sizeof(double));
+  float dev_ms = 0.0f;
+  CU(cudaEventElapsedTime(&dev_ms, c->mn_ev[0], c->mn_ev[1]));
+
+  if (s.proj_active == 0) c->proj = ms_ctx::PendingProjection();
+  if (s.proj_active == 1) c->proj = p_grad;
+  if (s.last_ran_a >= 0) c->ran_pass_a = s.last_ran_a != 0;
+  if (s.n_accepted > 0) c->has_positions = true;
+  io->step_size = s.step_size;
+  io->cg_iter = s.cg_iter;
+  io->cg_have_history = s.cg_have_history;
+  io->energy = s.res_energy;
+  io->grad_norm = s.res_has_grad_norm ? s.res_grad_norm : 0.0;
+  io->iterations = s.res_iterations;
+  io->terminated_early = s.res_terminated_early;
+  io->step_success = s.res_step_success;
+  io->has_grad_norm = s.res_has_grad_norm;
+  io->n_history = s.n_hist;
+  c->mn_counts[0] = s.n_hist;
+  c->mn_counts[1] = s.n_trials;
+  c->mn_counts[2] = s.n_evals;
+  c->mn_counts[3] = host_syncs;
+  c->mn_counts[4] = s.n_actions;
+  c->mn_counts[5] = s.n_guards;
+  c->mn_counts[6] = s.n_guard_rejects;
+  c->mn_ms[0] = dev_ms;
+  return 0;
+}
+
+int ms_ctx_minimize_stats(const ms_ctx* c, int64_t* counts7, double* ms2) {
+  if (!c) return fail(-1, "null context");
+  if (counts7) std::copy(c->mn_counts, c->mn_counts + 7, counts7);
+  if (ms2) std::copy(c->mn_ms, c->mn_ms + 2, ms2);
   return 0;
 }
 

@@ -985,10 +985,12 @@ __global__ void __launch_bounds__(256) k_scatter_rows(const double* __restrict__
   out[size_t(rows[r]) * width + c] = src[i];
 }
 
+// alpha_dev (device, may be null) replaces alpha: the device-controlled line search (ms_ctx_minimize)
 __global__ void __launch_bounds__(256) k_axpy(const double* __restrict__ x,
                                               const double* __restrict__ d, double alpha,
-                                              double* out, int64_t n) {
+                                              const double* __restrict__ alpha_dev, double* out, int64_t n) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (alpha_dev) alpha = *alpha_dev;
   if (i < n) out[i] = x[i] + alpha * d[i];
 }
 
@@ -1844,13 +1846,19 @@ __global__ void __launch_bounds__(256) k_normal_change(const int32_t* __restrict
 
 // Per-vertex Polak-Ribiere direction (runtime/steppers/conjugate_gradient.py:84-104):
 //   beta_v = g_v.(g_v - g'_v) / (g'_v.g'_v + 1e-20);  d_v = -g_v + beta_v d'_v, or -g_v where beta_v < 0;
-// fixed rows get a zero direction.
+// fixed rows get a zero direction.  restart (device, may be null) set: d = -1 * g on every row, as launch_scale.
 __global__ void __launch_bounds__(256) k_cg_direction(const double* __restrict__ g, const double* __restrict__ pg,
                                                       const double* __restrict__ pd,
-                                                      const uint8_t* __restrict__ fixed, int64_t nv, double* d) {
+                                                      const uint8_t* __restrict__ fixed, int64_t nv, double* d,
+                                                      const int32_t* __restrict__ restart) {
   const int64_t v = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (v >= nv) return;
   const double gx = g[3 * v], gy = g[3 * v + 1], gz = g[3 * v + 2];
+  if (restart && *restart) {
+    const double scale = -1.0;
+    d[3 * v] = scale * gx; d[3 * v + 1] = scale * gy; d[3 * v + 2] = scale * gz;
+    return;
+  }
   const double px = pg[3 * v], py = pg[3 * v + 1], pz = pg[3 * v + 2];
   const double numer = gx * (gx - px) + gy * (gy - py) + gz * (gz - pz);
   const double denom = (px * px + py * py + pz * pz) + 1.0e-20;
@@ -1865,10 +1873,11 @@ __global__ void __launch_bounds__(256) k_cg_direction(const double* __restrict__
 
 // y[v,:] += alpha * x[v,:] on the rows that are not fixed (constraint projection of the positions).  x may be y
 // (ms_ctx_axpy with dst == src), so it is not __restrict__; each thread reads and writes only its own element.
-__global__ void __launch_bounds__(256) k_axpy_rows(const double* x, double alpha,
+__global__ void __launch_bounds__(256) k_axpy_rows(const double* x, double alpha, const double* __restrict__ alpha_dev,
                                                    const uint8_t* __restrict__ fixed, int64_t nv, double* y) {
   const int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= 3 * nv) return;
+  if (alpha_dev) alpha = *alpha_dev;
   if (fixed && fixed[i / 3]) return;
   y[i] += alpha * x[i];
 }
@@ -2029,9 +2038,9 @@ cudaError_t launch_scatter_rows(const double* src, int width, const int32_t* row
 }
 
 cudaError_t launch_axpy(const double* x, const double* d, double alpha, double* out, int64_t n,
-                        cudaStream_t st) {
+                        cudaStream_t st, const double* alpha_dev) {
   if (n <= 0) return cudaSuccess;
-  k_axpy<<<blocks_for(n, 256), 256, 0, st>>>(x, d, alpha, out, n);
+  k_axpy<<<blocks_for(n, 256), 256, 0, st>>>(x, d, alpha, alpha_dev, out, n);
   return cudaGetLastError();
 }
 
@@ -2552,14 +2561,51 @@ cudaError_t launch_normal_change(const int32_t* tri, int32_t nf, int32_t nv, con
 }
 
 cudaError_t launch_cg_direction(const double* g, const double* pg, const double* pd, const uint8_t* fixed,
-                                int64_t nv, double* d, cudaStream_t st) {
-  if (nv > 0) k_cg_direction<<<blocks_for(nv, 256), 256, 0, st>>>(g, pg, pd, fixed, nv, d);
+                                int64_t nv, double* d, cudaStream_t st, const int32_t* restart_dev) {
+  if (nv > 0) k_cg_direction<<<blocks_for(nv, 256), 256, 0, st>>>(g, pg, pd, fixed, nv, d, restart_dev);
   return cudaGetLastError();
 }
 
 cudaError_t launch_axpy_rows(const double* x, double alpha, const uint8_t* fixed, int64_t nv, double* y,
-                             cudaStream_t st) {
-  if (nv > 0) k_axpy_rows<<<blocks_for(3 * nv, 256), 256, 0, st>>>(x, alpha, fixed, nv, y);
+                             cudaStream_t st, const double* alpha_dev) {
+  if (nv > 0) k_axpy_rows<<<blocks_for(3 * nv, 256), 256, 0, st>>>(x, alpha, alpha_dev, fixed, nv, y);
+  return cudaGetLastError();
+}
+
+namespace {
+// initial words of the line-search reductions: min edge^2 = 1e300, max |d|^2 = 0, guard flag, spare
+__global__ void k_ls_init(unsigned long long* bits) {
+  if (threadIdx.x == 0) {
+    bits[0] = (unsigned long long)__double_as_longlong(1.0e300);
+    bits[1] = (unsigned long long)__double_as_longlong(0.0);
+    bits[2] = bits[3] = 0ull;
+  }
+}
+
+// one thread: advance the loop of ms_ctx_minimize to its next action and open that action's IF node
+__global__ void k_min_control(MinOpts o, MinState* s, const double* scalars, const unsigned long long* ls_bits, int32_t nf,
+                              double* hist, int32_t hist_cap, int32_t proj_grad, int32_t ran_a_grad, MinHandles h) {
+  if (threadIdx.x != 0) return;
+  MinInput in;
+  in.sc = scalars;
+  ms_min_ls_stats(ls_bits, scalars, nf, in.ls);
+  in.ok = reinterpret_cast<const int*>(ls_bits + 2)[0] == 0;
+  const int32_t act = ms_min_step(o, *s, in, hist, hist_cap, proj_grad, ran_a_grad);
+  for (int k = 0; k < MN_ACTIONS; ++k)
+    if (h.present & (1u << k)) cudaGraphSetConditional(h.act[k], act == k ? 1u : 0u);
+  cudaGraphSetConditional(h.run, act == MN_DONE ? 0u : 1u);
+}
+}  // namespace
+
+cudaError_t launch_ls_init(unsigned long long* bits, cudaStream_t st) {
+  k_ls_init<<<1, 32, 0, st>>>(bits);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_min_control(const MinOpts& o, MinState* s, const double* scalars, const unsigned long long* ls_bits,
+                               int32_t nf, double* hist, int32_t hist_cap, int32_t proj_grad, int32_t ran_a_grad,
+                               const MinHandles& h, cudaStream_t st) {
+  k_min_control<<<1, 32, 0, st>>>(o, s, scalars, ls_bits, nf, hist, hist_cap, proj_grad, ran_a_grad, h);
   return cudaGetLastError();
 }
 

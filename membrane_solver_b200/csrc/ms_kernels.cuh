@@ -11,6 +11,7 @@
 #include "ms_math.cuh"
 #include "ms_pack.h"
 #include "ms_equiangulate.cuh"
+#include "ms_minimize.cuh"
 #include "ms_pack_device.cuh"
 #include "ms_refine.cuh"
 #include "ms_vertex_average.cuh"
@@ -188,9 +189,10 @@ cudaError_t launch_gather_rows(const double* src, int width, const int32_t* rows
 // out[rows[i]*width + c] = src[i*width + c]: internal vertex order -> caller's order
 cudaError_t launch_scatter_rows(const double* src, int width, const int32_t* rows, int64_t n,
                                 double* out, cudaStream_t st);
-// x_out = x + alpha * d  (trial positions of the line search, line_search.py:358-382)
+// x_out = x + alpha * d  (trial positions of the line search, line_search.py:358-382); alpha_dev (device, may be
+// null) replaces alpha
 cudaError_t launch_axpy(const double* x, const double* d, double alpha, double* out, int64_t n,
-                        cudaStream_t st);
+                        cudaStream_t st, const double* alpha_dev = nullptr);
 
 // --- generic (any triangle soup) kernels behind the stateless KernelSpec shims ---
 struct SoupArgs {
@@ -230,9 +232,24 @@ cudaError_t launch_normal_change(const int32_t* tri, int32_t nf, int32_t nv, con
                                  const double* new_pos, double cos_limit, int* flag, cudaStream_t st);
 cudaError_t launch_scale(const double* x, double scale, double* out, int64_t n, cudaStream_t st);
 cudaError_t launch_axpy_rows(const double* x, double alpha, const uint8_t* fixed, int64_t nv, double* y,
-                             cudaStream_t st);
+                             cudaStream_t st, const double* alpha_dev = nullptr);
+// restart_dev (device, may be null): when it holds a non-zero value, d = -1 * g (launch_scale) instead
 cudaError_t launch_cg_direction(const double* g, const double* pg, const double* pd, const uint8_t* fixed,
-                                int64_t nv, double* d, cudaStream_t st);
+                                int64_t nv, double* d, cudaStream_t st, const int32_t* restart_dev = nullptr);
+// the initial words of launch_min_edge2 / launch_max_row_norm2 / launch_normal_change (4 words)
+cudaError_t launch_ls_init(unsigned long long* bits, cudaStream_t st);
+
+// --- loop control of ms_ctx_minimize (ms_minimize.cuh): condition handles of the graph's WHILE node and of the IF
+// node of every action present (bit k of `present`) ---
+struct MinHandles {
+  cudaGraphConditionalHandle run;
+  cudaGraphConditionalHandle act[MN_ACTIONS];
+  uint32_t present;
+};
+// one thread: ms_min_step on the device state, then the condition values of the next action
+cudaError_t launch_min_control(const MinOpts& o, MinState* s, const double* scalars, const unsigned long long* ls_bits,
+                               int32_t nf, double* hist, int32_t hist_cap, int32_t proj_grad, int32_t ran_a_grad,
+                               const MinHandles& h, cudaStream_t st);
 
 constexpr int kSumBlocks = 592;  // partial sums of the two-stage fixed-order reductions (4 CTAs per SM)
 // --- bending-tilt coupling on the resident mesh (ms_bt.cuh); corner holds 12*nf doubles, e_out 1 + kSumBlocks ---

@@ -16,6 +16,12 @@ constraints and without tilts --
   backtracking factor ``beta``, growth ``gamma``, the normal-flip guard of
   ``runtime/topology.py:13-48`` for steps larger than 0.3 x the shortest edge.
 
+With ``device_loop=True`` on a ``DeviceMesh`` the loop itself runs under device control (``ms_ctx_minimize``,
+``csrc/ms_minimize.cuh``): one CUDA graph and one host synchronisation per ``minimize`` call, with the decisions of
+the host loop (``minimize_host``) bit for bit.  It is opt-in because it measures slower than the host loop on one
+B200 (DESIGN.md section 1, row f1).  The host loop is the default; it also serves ``PartitionedDevice``
+(cross-rank reductions) and is the reference of the tests.
+
 It is an optional consumer of the hot path, not part of it: the reference's own minimiser keeps
 working on the plugin modules (INTEGRATION.md section 2).
 """
@@ -51,6 +57,7 @@ class DeviceMinimizer:
     edge_fraction: float = 0.0     # global parameter shape_step_edge_fraction
     stepper: str = "gd"            # "gd" | "cg" (per-vertex Polak-Ribiere, conjugate_gradient.py:63-119)
     restart_interval: int = 10
+    device_loop: bool = False      # run minimize() under device control (DeviceMesh.minimize), opt-in: measured slower
     _cg_iter: int = 0
     _cg_have_history: bool = False
     history: list = field(default_factory=list)
@@ -165,7 +172,38 @@ class DeviceMinimizer:
         return False, max(reduced, step_size * self.beta), energy0
 
     # -- the loop (minimizer.py:1189-1535) ------------------------------------------------------------
+    def minimize_options(self):
+        """The options of the device-controlled loop (``ms_minimize_opts``)."""
+        return L.MinimizeOpts(
+            modules=self.modules, flags=self.flags, volume_mode={"lagrange": 0, "penalty": 1}.get(self.volume_mode, -1),
+            enforce_volume=int(bool(self.enforce_volume)), projection_during=int(bool(self.projection_during_minimization)),
+            stepper={"gd": 0, "cg": 1}[self.stepper], max_zero_steps=self.max_zero_steps, max_iter=self.max_iter,
+            restart_interval=self.restart_interval, k_vol=self.k_vol, v_target=self.v_target, tol=self.tol,
+            step_size_floor=self.step_size_floor, beta=self.beta, c=self.c, gamma=self.gamma,
+            alpha_max_factor=self.alpha_max_factor, edge_fraction=self.edge_fraction,
+            volume_tolerance=self.volume_tolerance)
+
     def minimize(self, n_steps: int = 1) -> dict:
+        """``n_steps`` minimiser steps: the host loop (``minimize_host``) or, with ``device_loop``, the whole loop under
+        device control (``DeviceMesh.minimize``: one host synchronisation per call).  Both take the same decisions bit
+        for bit."""
+        if self.device_loop:
+            if not hasattr(self.dm, "minimize"):
+                raise L.B200Error("device_loop needs a single-context DeviceMesh (ms_ctx_minimize)")
+            res, rows = self.dm.minimize(self.minimize_options(), int(n_steps), step_size=self.step_size,
+                                         cg_iter=self._cg_iter, cg_have_history=self._cg_have_history)
+            self.step_size = float(res.step_size)
+            self._cg_iter, self._cg_have_history = int(res.cg_iter), bool(res.cg_have_history)
+            self.history.extend(rows)
+            out = {"energy": float(res.energy), "iterations": int(res.iterations),
+                   "terminated_early": bool(res.terminated_early), "step_success": bool(res.step_success)}
+            if res.has_grad_norm:
+                out["grad_norm"] = float(res.grad_norm)
+            return out
+        return self.minimize_host(n_steps)
+
+    def minimize_host(self, n_steps: int = 1) -> dict:
+        """The host loop: every decision on the host, one scalar read per evaluation and statistic."""
         zero_steps = 0
         success = True
         energy = float("nan")
